@@ -19,6 +19,10 @@ and compared with tests/golden/c4_checksum.json, which the UNMODIFIED reference 
 (tests/golden/make_c4_checksum.py): the scaling runs carry parity, not only invariants.
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--config C4|C2|C3|C5]
+                  [--dump-outputs DIR]
+
+--dump-outputs DIR (one GPU) writes what the timed steps computed as DIR/<name>.npy (float64, ~50 MB; see dump_graph):
+the inputs are generated from fixed seeds, so two builds run with the same arguments can be compared file by file.
 
 `--impl reference` times the reference's own CPU implementation (oracle/_ref/ref_driver: the unmodified reference
 sources driven through ThreadPoolPPPCSR, -pppcsrnuma, all host threads) on the SAME workload, full size.
@@ -81,7 +85,12 @@ def parse_args():
     ap.add_argument("--ref-budget-s", type=float, default=float(os.environ.get("PPCSR_REF_BUDGET_S", "200")),
                     help="--impl reference: full runs are repeated while they fit this wall-clock budget (>= 1 run)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the graph the last timed step left (a seeded sample) and the last PageRank step as "
+                         "DIR/<name>.npy (one GPU)")
     a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     scale, batch, workload = CONFIGS[a.config]
     a.scale = a.scale if a.scale is not None else scale
     a.batch = a.batch if a.batch is not None else batch
@@ -343,6 +352,48 @@ def main_reference(args):
 
 
 # ------------------------------------------------------------------------------------------------
+# --dump-outputs: what the timed path computed, for comparing two builds output for output
+# ------------------------------------------------------------------------------------------------
+DUMP_SAMPLE = 1 << 20  # vertices and edges sampled: the C4 graph itself (16.8 M vertices, 360 M edges) is GBs
+# the outcome of a batch; the window / byte counts are left out: they describe how a build did the work
+BATCH_COUNTS = ("batch_size", "n_unique", "n_inserted", "n_overwritten", "n_deleted", "n_not_found", "slots_before",
+                "slots_after", "resized")
+
+
+def dump_graph(out_dir, shard, stats):
+    """Writes the logical graph the last timed step left on the shard, as float64 arrays (ids < 2^32 are exact):
+      checksum.npy       edges, edge_hash >> 32, edge_hash & 0xffffffff, nn_hash >> 32, nn_hash & 0xffffffff
+      batch.npy          the last step's counts: BATCH_COUNTS, in that order
+      vertices.npy       a seeded sample of vertex ids (sorted, unique), and for them
+      degree.npy         out-degree in the logical graph (rowptr[v + 1] - rowptr[v])
+      num_neighbors.npy  num_neighbors (call-count semantics of the reference)
+      edge_src.npy       a seeded sample of positions of the exported CSR (sorted, unique): source of the edge there
+      edge_dst.npy       and its destination
+    Returns the vertex sample: run_config writes the last timed PageRank push step at those vertices as pagerank.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+
+    def save(name, a):
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
+
+    cks = shard.checksum()
+    save("checksum", [cks["edges"], cks["edge_hash"] >> 32, cks["edge_hash"] & 0xFFFFFFFF, cks["nn_hash"] >> 32,
+                      cks["nn_hash"] & 0xFFFFFFFF])
+    save("batch", [stats[k] for k in BATCH_COUNTS])
+    rowptr, col = shard.export()
+    rowptr = rowptr.astype(np.int64)
+    n, E = rowptr.size - 1, col.size
+    rng = np.random.default_rng(0)
+    verts = np.unique(rng.integers(0, n, DUMP_SAMPLE)) if n else np.zeros(0, dtype=np.int64)
+    save("vertices", verts)
+    save("degree", (rowptr[verts + 1] - rowptr[verts]).astype(np.int64))
+    save("num_neighbors", shard.num_neighbors()[verts])
+    pos = np.unique(rng.integers(0, E, DUMP_SAMPLE)) if E else np.zeros(0, dtype=np.int64)
+    save("edge_src", np.searchsorted(rowptr, pos, side="right") - 1)
+    save("edge_dst", col[pos])
+    return verts
+
+
+# ------------------------------------------------------------------------------------------------
 # B200 arm
 # ------------------------------------------------------------------------------------------------
 def make_updates(synth, torch, workload, scale, lo, hi, total_updates, dev):
@@ -403,9 +454,9 @@ def build_core(synth, torch, router, scale, rank, world, local_rank, dev, dist, 
 
 
 def run_config(args, scale, B, workload, torch, dist, rank, world, local_rank, dev, steps, warmup, e2e_steps,
-               with_clocks=False, with_pagerank=False, golden=None):
+               with_clocks=False, with_pagerank=False, golden=None, dump_dir=None):
     """Builds the graph, times `steps` device-resident steps and `e2e_steps` host-buffer steps.  Returns a dict of
-    results (rank 0 view; times are the max over ranks)."""
+    results (rank 0 view; times are the max over ranks).  dump_dir (one shard): see dump_graph."""
     synth = importlib.import_module("parallel-packed-csr_b200.synth")
     router = importlib.import_module("parallel-packed-csr_b200.router")
     stream = torch.cuda.current_stream()
@@ -490,6 +541,7 @@ def run_config(args, scale, B, workload, torch, dist, rank, world, local_rank, d
                             "match": ok}
         if not ok:
             raise SystemExit(f"bench.py: logical graph differs from the reference's: {parity} vs {golden}")
+    dump_vertices = dump_graph(dump_dir, graph.shard, stats_acc[-1]) if dump_dir else None
 
     # ---- end to end through the public host-buffer call: pinned host inputs, H2D inside the timed region; the state
     # restore between the steps (a device-to-device copy) is inside the timed region as well
@@ -535,9 +587,11 @@ def run_config(args, scale, B, workload, torch, dist, rank, world, local_rank, d
         p0, p1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         p0.record(stream)
         for _ in range(steps):
-            graph.pagerank_step(vals)
+            pr = graph.pagerank_step(vals)
         p1.record(stream)
         barrier()
+        if dump_vertices is not None:  # the last step's push result at the sampled vertices
+            np.save(os.path.join(dump_dir, "pagerank.npy"), pr.cpu().numpy()[dump_vertices])
         geo = graph.shard.geometry
         pr_ms = allmax(p0.elapsed_time(p1) / steps)
         # SURVEY.md §8d: 12 n (node array) + slot bytes * N (every slot, gaps included) + 4 n (contribution) + 8 E
@@ -603,6 +657,8 @@ def main_b200(args):
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     if not torch.cuda.is_available():
         raise SystemExit("bench.py: no CUDA device (the B200 engine has no CPU fallback)")
+    if args.dump_outputs and world > 1:
+        raise SystemExit("bench.py: --dump-outputs supports one GPU")
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
     dist = None
@@ -616,7 +672,8 @@ def main_b200(args):
 
     scale, B = global_shape(args, world)
     res = run_config(args, scale, B, args.workload, torch, dist, rank, world, local_rank, dev, args.steps, args.warmup,
-                     args.e2e_steps, with_clocks=True, with_pagerank=True, golden=golden_checksum(args, world))
+                     args.e2e_steps, with_clocks=True, with_pagerank=True, golden=golden_checksum(args, world),
+                     dump_dir=args.dump_outputs)
     others = {}
     if world == 1 and not args.only_headline and args.is_named:
         for name in ("C2", "C3", "C5"):
