@@ -267,7 +267,9 @@ int ppcsr_restore(ppcsr_shard *h);
 int ppcsr_debug_dump(ppcsr_shard *h, uint32_t *dest, uint32_t *val, uint32_t *leaf_cnt);
 
 /* ---- primitives exposed for unit tests (host buffers, in place) ---- */
-/* Stable LSD radix sort of (key, payload) pairs by key bits [0,lo_bits) and [32,32+hi_bits). */
+/* Stable LSD radix sort of (key, payload) pairs by key bits [0,lo_bits) and [32,32+hi_bits), 1 <= lo_bits, hi_bits
+ * <= 32.  payload == NULL sorts the keys alone (the keys-only passes the batch pipeline runs when the values need no
+ * sorting). */
 int ppcsr_debug_sort_pairs(int device, uint64_t *keys, uint32_t *payload, uint64_t count, int lo_bits, int hi_bits);
 /* out[i] = sum of in[0..i), out[count] = total (out has count+1 entries). */
 int ppcsr_debug_exclusive_scan(int device, const uint32_t *in, uint32_t *out, uint64_t count);

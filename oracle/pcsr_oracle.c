@@ -495,6 +495,18 @@ uint64_t opcsr_export(const opcsr_t *g, uint64_t *rowptr, uint32_t *col, uint32_
   return k;
 }
 
+/* the stored values in the order of opcsr_export's col (val may be NULL to size) */
+uint64_t opcsr_export_values(const opcsr_t *g, uint32_t *val) {
+  uint64_t k = 0;
+  for (uint64_t v = 0; v < g->n; v++)
+    for (uint32_t i = g->nodes[v].beginning + 1; i < g->nodes[v].end; i++)
+      if (g->items[i].value != 0) {
+        if (val) val[k] = g->items[i].value;
+        k++;
+      }
+  return k;
+}
+
 /* batch front end used by tests and the cpu_baseline leg: value 0 = delete */
 void opcsr_apply(opcsr_t *g, const uint32_t *src, const uint32_t *dst, const uint32_t *val, uint64_t count) {
   for (uint64_t i = 0; i < count; i++) {

@@ -378,10 +378,12 @@ class Shard:
         return dest, val, cnt
 
 
-def debug_sort_pairs(keys, payload, lo_bits, hi_bits, device=0):
+def debug_sort_pairs(keys, payload=None, lo_bits=32, hi_bits=32, device=0):
+    """ppcsr_debug_sort_pairs on copies; payload None sorts the keys alone (and returns None for it)."""
     L = load_library()
     keys = np.ascontiguousarray(keys, dtype=np.uint64).copy()
-    payload = np.ascontiguousarray(payload, dtype=np.uint32).copy()
+    if payload is not None:
+        payload = np.ascontiguousarray(payload, dtype=np.uint32).copy()
     _check(L.ppcsr_debug_sort_pairs(device, _np_ptr(keys), _np_ptr(payload), keys.shape[0], lo_bits, hi_bits))
     return keys, payload
 

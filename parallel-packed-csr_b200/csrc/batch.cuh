@@ -229,6 +229,7 @@ struct SegmentTable {
   uint64_t cap;
   const uint64_t *counts;  // DEVICE array: valid records of every region (deposited by the senders)
   unsigned long long *prefix_out;  // DEVICE array of n_seg + 1 entries (nullable): exclusive prefix of the counts
+  uint64_t bound;  // keys the key array holds: a larger deposited total is reported (seg_total), not written
 };
 __global__ void __launch_bounds__(BT) k_build_keys_segments(const uint64_t *__restrict__ packed,
                                                             const uint32_t *__restrict__ val, uint32_t default_val,
@@ -257,7 +258,7 @@ __global__ void __launch_bounds__(BT) k_build_keys_segments(const uint64_t *__re
   }
   __syncthreads();
   uint32_t my_or = 0, my_bad = 0, my_vmax = 0, my_vinv = 0;
-  const size_t count = (size_t)s_prefix[T.n_seg];
+  const size_t count = min((size_t)s_prefix[T.n_seg], (size_t)T.bound);
   for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < count; i += (size_t)gridDim.x * blockDim.x) {
     uint32_t lo = 0, hi = T.n_seg;  // last region with prefix <= i
     while (hi - lo > 1) {

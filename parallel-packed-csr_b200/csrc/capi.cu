@@ -1171,6 +1171,7 @@ int ppcsr_apply_batch_segments_device(ppcsr_shard *s, const uint64_t *d_packed, 
   uint64_t bound = max_total ? std::min<uint64_t>(max_total, (uint64_t)n_segments * region_cap)
                              : (uint64_t)n_segments * region_cap;
   bound = std::min<uint64_t>(bound, (1ull << 31) - 1);  // one batch holds < 2^31 updates
+  T.bound = bound;  // the keys are sized for `bound`: k_build_keys_segments writes no more than that
   return apply_device_common(s, nullptr, nullptr, d_packed, d_val, bound, default_val, stats, &T);
 }
 
@@ -1927,6 +1928,8 @@ int ppcsr_debug_dump(ppcsr_shard *s, uint32_t *dest, uint32_t *val, uint32_t *le
 
 int ppcsr_debug_sort_pairs(int device, uint64_t *keys, uint32_t *payload, uint64_t count, int lo_bits, int hi_bits) {
   if (ppcsr_device_count() <= device) return PPCSR_ERR_NO_DEVICE;
+  if (count && !keys) return PPCSR_ERR_ARG;
+  if (lo_bits < 1 || lo_bits > 32 || hi_bits < 1 || hi_bits > 32) return PPCSR_ERR_ARG;
   if (count == 0) return PPCSR_OK;
   CUDA_TRY(cudaSetDevice(device));
   ppcsr_shard tmp;
@@ -1935,14 +1938,14 @@ int ppcsr_debug_sort_pairs(int device, uint64_t *keys, uint32_t *payload, uint64
   int rc = reserve_batch_arrays(&tmp, count);
   if (rc != PPCSR_OK) return rc;
   CUDA_TRY(cudaMemcpy(tmp.key_a.p, keys, count * 8, cudaMemcpyHostToDevice));
-  CUDA_TRY(cudaMemcpy(tmp.pay_a.p, payload, count * 4, cudaMemcpyHostToDevice));
+  if (payload) CUDA_TRY(cudaMemcpy(tmp.pay_a.p, payload, count * 4, cudaMemcpyHostToDevice));
   uint64_t *rk;
   uint32_t *rp;
-  rc = prim::radix_sort_pairs(&tmp, tmp.key_a.p, tmp.pay_a.p, tmp.key_b.p, tmp.pay_b.p, count, lo_bits, hi_bits, &rk,
-                              &rp);
+  rc = prim::radix_sort_pairs(&tmp, tmp.key_a.p, payload ? tmp.pay_a.p : nullptr, tmp.key_b.p, tmp.pay_b.p, count,
+                              lo_bits, hi_bits, &rk, &rp);
   if (rc == PPCSR_OK) {
     CUDA_TRY(cudaMemcpy(keys, rk, count * 8, cudaMemcpyDeviceToHost));
-    CUDA_TRY(cudaMemcpy(payload, rp, count * 4, cudaMemcpyDeviceToHost));
+    if (payload) CUDA_TRY(cudaMemcpy(payload, rp, count * 4, cudaMemcpyDeviceToHost));
   }
   dev_free(tmp.key_a); dev_free(tmp.key_b); dev_free(tmp.pay_a); dev_free(tmp.pay_b);
   dev_free(tmp.ukey); dev_free(tmp.uval); dev_free(tmp.uloc); dev_free(tmp.ucls); dev_free(tmp.ufirst);

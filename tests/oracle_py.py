@@ -59,6 +59,8 @@ def lib() -> C.CDLL:
         L.opcsr_neighbourhood.restype = u64
         L.opcsr_export.argtypes = [vp, vp, vp, vp]
         L.opcsr_export.restype = u64
+        L.opcsr_export_values.argtypes = [vp, vp]
+        L.opcsr_export_values.restype = u64
         L.opcsr_apply.argtypes = [vp, vp, vp, vp, u64]
         L.opcsr_pagerank_f64.argtypes = [vp, vp, vp]
         L.opcsr_pagerank_f32.argtypes = [vp, vp, vp]
@@ -136,6 +138,12 @@ class OraclePCSR:
         col = np.zeros(E, dtype=np.uint32)
         self.L.opcsr_export(self.h, _ptr(rowptr), _ptr(col), _ptr(nn))
         return rowptr, col, nn
+
+    def export_values(self):
+        """The stored values, aligned with export()'s col."""
+        val = np.zeros(self.L.opcsr_export_values(self.h, None), dtype=np.uint32)
+        self.L.opcsr_export_values(self.h, _ptr(val))
+        return val
 
     def pagerank(self, values, dtype=np.float64):
         values = np.ascontiguousarray(values, dtype=dtype)

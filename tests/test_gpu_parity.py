@@ -65,6 +65,37 @@ def test_primitives_scan_and_sort():
         order = np.argsort(keys, kind="stable")
         assert np.array_equal(k2, keys[order]), (n, sb, db)
         assert np.array_equal(p2, pay[order]), (n, sb, db)  # stability: ties keep submission order
+    # keys only (payload None) and with payload, against a stable argsort of the compacted field (dst bits [0, lo),
+    # src bits above): random bits outside the field make equal fields of different keys, so instability shows even
+    # without a payload.  Sizes around 2^25, where the keys-only passes publish their tile counts late, and ~40 M;
+    # lo_bits = 32 (no compaction); 64 live bits (8 passes); one field value for all; every key at the field maximum,
+    # where the padding keys of the partial last tile land too.
+    for n, lo, hi, kind in (((1 << 25) - 1, 20, 20, "rand"), (1 << 25, 20, 20, "rand"), ((1 << 25) + 1, 18, 21, "rand"),
+                            (40_000_003, 22, 22, "rand"), (200_001, 32, 12, "rand"), (9000, 32, 7, "rand"),
+                            (300_001, 32, 32, "rand"), (5000, 32, 32, "rand"), (200_003, 16, 16, "equal"),
+                            (3000, 16, 16, "equal"), (100_001, 18, 14, "max"), (16_383, 18, 14, "max")):
+        if kind == "rand" and lo + hi == 64:  # no bits outside the field: repeats from a small pool make the ties
+            pool = rng.integers(0, 1 << 63, n // 4 + 1, dtype=np.uint64) * np.uint64(2) + rng.integers(0, 2, n // 4 + 1).astype(np.uint64)
+            keys = pool[rng.integers(0, pool.size, n)]
+        else:
+            dst = rng.integers(0, 1 << 32, n, dtype=np.uint64) & np.uint64((1 << lo) - 1)
+            src = rng.integers(0, 1 << hi, n, dtype=np.uint64) if kind == "rand" else np.full(n, (1 << hi) - 1, np.uint64)
+            if kind == "equal":
+                src[:], dst[:] = 5, 3
+            elif kind == "max":
+                dst[:] = (1 << lo) - 1
+            junk = rng.integers(0, 1 << 32, n, dtype=np.uint64) >> np.uint64(hi) << np.uint64(hi)  # src bits >= hi
+            keys = ((src | junk) << np.uint64(32)) | dst
+        with np.errstate(over="ignore"):
+            field = keys if lo == 32 else ((keys >> np.uint64(32)) << np.uint64(lo)) | (keys & np.uint64(0xFFFFFFFF))
+        if lo + hi < 64:
+            field = field & np.uint64((1 << (lo + hi)) - 1)
+        order = np.argsort(field, kind="stable")
+        k1, none = pp.debug_sort_pairs(keys, None, lo, hi)
+        assert none is None and np.array_equal(k1, keys[order]), ("keys only", n, lo, hi, kind)
+        pay = np.arange(n, dtype=np.uint32)
+        k2, p2 = pp.debug_sort_pairs(keys, pay, lo, hi)
+        assert np.array_equal(k2, keys[order]) and np.array_equal(p2, order.astype(np.uint32)), ("pairs", n, lo, hi, kind)
 
 
 def test_create_matches_reference_constructor():
@@ -87,7 +118,8 @@ def test_create_matches_reference_constructor():
 POLICIES = [-1, 0]
 
 
-@pytest.mark.parametrize("policy", POLICIES, ids=["windows", "auto"])
+# the golden fixtures also run with policy 1 (always one root window), which disables the small-batch path
+@pytest.mark.parametrize("policy", POLICIES + [1], ids=["windows", "auto", "whole"])
 @pytest.mark.parametrize("path", GOLDEN, ids=[os.path.basename(p)[:-4] for p in GOLDEN])
 def test_golden_fixture(path, policy):
     fx = np.load(path)
