@@ -215,6 +215,21 @@ uint32_t ppcsr_group_owner(const ppcsr_group *g, uint64_t vertex); /* reference 
  * then every shard applies what it received.  stats (nullable) gets one entry per shard. */
 int ppcsr_group_apply(ppcsr_group *g, const uint32_t *src, const uint32_t *dst, const uint32_t *val, uint64_t count,
                       uint32_t default_val, ppcsr_batch_stats *stats);
+/* Traversals across all shards of the group, on the devices.  n = starts[n_shards-1] + (vertices of the last shard
+ * now): the last shard may have grown through ppcsr_add_nodes (PPPCSR::add_node appends there); if any other shard no
+ * longer holds exactly its range, both calls return PPCSR_ERR_ARG.  All work of shard r runs on shard r's stream, the
+ * shards wait for each other through events: a traversal is ordered after the group's last ppcsr_group_apply and
+ * before the next one.  A traversal modifies no shard.
+ * Device memory the group keeps for traversals (allocated on first use, reallocated when n changes, freed by
+ * ppcsr_group_destroy), per shard r with n_r vertices:
+ *   BFS       n_shards * n_r * 4 B of inbox + n / 8 B of bitmap + 3 * n_r * 4 B of distances and frontier queues
+ *   PageRank  n * 8 B of accumulator + n_r * 8 B of ranks
+ * reference src/utility/bfs.h:15-36 over all shards of the group: dist[n] (host), UINT32_MAX = unreached,
+ * start >= n leaves every vertex unreached.  Same result as ppcsr_bfs on one shard holding the graph. */
+int ppcsr_group_bfs(ppcsr_group *g, uint32_t start, uint32_t *dist);
+/* ppcsr_pagerank's recurrence over all shards of the group (n = n_global, divisor num_neighbors, no dangling
+ * redistribution), out[n] on the host; iterations == 0 gives 1/n everywhere.  No host round trip between iterations. */
+int ppcsr_group_pagerank(ppcsr_group *g, uint32_t iterations, double damping, double *out);
 
 /* ---- reads ---- */
 int ppcsr_geometry_of(ppcsr_shard *h, ppcsr_geometry *out);

@@ -79,6 +79,8 @@ SYMBOLS = {
     "ppcsr_group_destroy": (None, [_vp]),
     "ppcsr_group_owner": (_u32, [_vp, _u64]),
     "ppcsr_group_apply": (_i, [_vp, _vp, _vp, _vp, _u64, _u32, C.POINTER(BatchStats)]),
+    "ppcsr_group_bfs": (_i, [_vp, _u32, _vp]),
+    "ppcsr_group_pagerank": (_i, [_vp, _u32, C.c_double, _vp]),
     "ppcsr_add_edge": (_i, [_vp, _u32, _u32, _u32]),
     "ppcsr_remove_edge": (_i, [_vp, _u32, _u32, C.POINTER(_i)]),
     "ppcsr_add_nodes": (_i, [_vp, _u32]),
@@ -439,6 +441,23 @@ class Group:
 
     def owner(self, v: int) -> int:
         return int(self.L.ppcsr_group_owner(self.g, v))
+
+    @property
+    def n(self) -> int:
+        """Global vertex count: the first vertex of the last shard plus its current size (it may have grown)."""
+        return int(self.starts[-2]) + self.shards[-1].n
+
+    def bfs(self, start) -> np.ndarray:
+        """Hop counts from `start` over all shards (ppcsr_group_bfs), UINT32_MAX = unreached; u32 of length n."""
+        out = np.zeros(self.n, dtype=np.uint32)
+        _check(self.L.ppcsr_group_bfs(self.g, start, _np_ptr(out)))
+        return out
+
+    def pagerank(self, iterations=20, damping=0.85) -> np.ndarray:
+        """Iterated PageRank over all shards (ppcsr_group_pagerank, the recurrence of Shard.pagerank); f64 of length n."""
+        out = np.zeros(self.n, dtype=np.float64)
+        _check(self.L.ppcsr_group_pagerank(self.g, iterations, float(damping), _np_ptr(out)))
+        return out
 
     def close(self):
         if getattr(self, "g", None):

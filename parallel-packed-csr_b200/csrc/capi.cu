@@ -16,6 +16,7 @@
 #include "rebalance_m.cuh"
 #include "sort.cuh"
 #include "sparse.cuh"
+#include "traverse.cuh"
 #include "windows.cuh"
 
 thread_local std::string g_ppcsr_error;

@@ -179,6 +179,13 @@ std::vector<uint32_t> PCSR::bfs_levels(uint32_t start) const {
   return d;
 }
 
+std::vector<double> PCSR::pagerank(uint32_t iterations, double damping) const {
+  std::lock_guard<std::mutex> g(edges.global_lock->mutex());
+  std::vector<double> r(get_n());
+  if (!r.empty() && ppcsr_pagerank(shard_, iterations, damping, r.data()) != PPCSR_OK) fail("ppcsr_pagerank");
+  return r;
+}
+
 bool PCSR::check_invariants(bool check_lower, ppcsr_invariant_report *report) const {
   std::lock_guard<std::mutex> g(edges.global_lock->mutex());
   ppcsr_invariant_report r{};

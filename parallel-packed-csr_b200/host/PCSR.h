@@ -75,6 +75,9 @@ class PCSR {
   // one pagerank push step (reference src/utility/pagerank.h:16-29) accumulated into out[0..out.size())
   void pagerank_push(const std::vector<double> &in, std::vector<double> &out) const;
   std::vector<uint32_t> bfs_levels(uint32_t start) const;
+  // iterated PageRank with damping on the device (ppcsr_pagerank): r_0 = 1/n,
+  // r_{t+1}[v] = (1 - damping)/n + damping * sum_{(u,v)} r_t[u] / num_neighbors[u]
+  std::vector<double> pagerank(uint32_t iterations, double damping) const;
   bool check_invariants(bool check_lower, ppcsr_invariant_report *report = nullptr) const;
   ppcsr_shard *handle() const { return shard_; }
   int device() const { return device_; }

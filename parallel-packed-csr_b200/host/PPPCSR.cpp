@@ -37,30 +37,33 @@ PPPCSR::~PPPCSR() {
   if (group_) ppcsr_group_destroy(group_);
 }
 
+void PPPCSR::ensure_group(std::size_t cap, bool values) {
+  const std::size_t parts = partitions.size();
+  if (group_ && cap <= group_cap_ && (!values || group_values_)) return;
+  if (group_) ppcsr_group_destroy(group_);  // (re)size the receive buffers
+  group_ = nullptr;
+  std::vector<ppcsr_shard *> handles;
+  std::vector<uint64_t> starts;
+  uint64_t n = 0;
+  for (std::size_t p = 0; p < parts; p++) {
+    handles.push_back(partitions[p].handle());
+    starts.push_back(distribution[p]);
+    n = distribution[p] + partitions[p].get_n();
+  }
+  starts.push_back(n);
+  group_cap_ = std::max<std::size_t>(cap + cap / 8, 1024);
+  group_values_ = group_values_ || values;
+  if (ppcsr_group_create(handles.data(), (uint32_t)parts, starts.data(), group_cap_, group_values_ ? 1 : 0,
+                         &group_) != PPCSR_OK) {
+    std::cout << "ppcsr_group_create failed: " << ppcsr_last_error() << ". Abort\n";
+    std::exit(EXIT_FAILURE);
+  }
+}
+
 void PPPCSR::apply_batch(const uint32_t *src, const uint32_t *dst, const uint32_t *value, size_t count,
                          std::vector<ppcsr_batch_stats> *stats) {
   const std::size_t parts = partitions.size();
-  const std::size_t slice = (count + parts - 1) / parts;
-  if (!group_ || slice > group_cap_ || (value && !group_values_)) {  // (re)size the receive buffers
-    if (group_) ppcsr_group_destroy(group_);
-    group_ = nullptr;
-    std::vector<ppcsr_shard *> handles;
-    std::vector<uint64_t> starts;
-    uint64_t n = 0;
-    for (std::size_t p = 0; p < parts; p++) {
-      handles.push_back(partitions[p].handle());
-      starts.push_back(distribution[p]);
-      n = distribution[p] + partitions[p].get_n();
-    }
-    starts.push_back(n);
-    group_cap_ = std::max<std::size_t>(slice + slice / 8, 1024);
-    group_values_ = group_values_ || value != nullptr;
-    if (ppcsr_group_create(handles.data(), (uint32_t)parts, starts.data(), group_cap_, group_values_ ? 1 : 0,
-                           &group_) != PPCSR_OK) {
-      std::cout << "ppcsr_group_create failed: " << ppcsr_last_error() << ". Abort\n";
-      std::exit(EXIT_FAILURE);
-    }
-  }
+  ensure_group((count + parts - 1) / parts, value != nullptr);
   std::vector<ppcsr_batch_stats> st(parts);
   if (ppcsr_group_apply(group_, src, dst, value, count, 1, st.data()) != PPCSR_OK) {
     std::cout << "ppcsr_group_apply failed: " << ppcsr_last_error() << ". Abort\n";
@@ -129,4 +132,24 @@ void PPPCSR::pagerank_push(const std::vector<double> &in, std::vector<double> &o
     std::vector<double> slice(in.begin() + lo, in.begin() + lo + n_local);
     partitions[p].pagerank_push(slice, out);
   }
+}
+
+std::vector<uint32_t> PPPCSR::bfs_levels(uint32_t start) {
+  ensure_group(0, false);
+  std::vector<uint32_t> d(get_n());
+  if (ppcsr_group_bfs(group_, start, d.data()) != PPCSR_OK) {
+    std::cout << "ppcsr_group_bfs failed: " << ppcsr_last_error() << ". Abort\n";
+    std::exit(EXIT_FAILURE);
+  }
+  return d;
+}
+
+std::vector<double> PPPCSR::pagerank(uint32_t iterations, double damping) {
+  ensure_group(0, false);
+  std::vector<double> r(get_n());
+  if (ppcsr_group_pagerank(group_, iterations, damping, r.data()) != PPCSR_OK) {
+    std::cout << "ppcsr_group_pagerank failed: " << ppcsr_last_error() << ". Abort\n";
+    std::exit(EXIT_FAILURE);
+  }
+  return r;
 }

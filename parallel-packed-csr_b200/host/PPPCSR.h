@@ -47,6 +47,13 @@ class PPPCSR {
   // per-op hand-over of reference ThreadPoolPPPCSR::submit_* (thread_pool_pppcsr.cpp:96-118).  stats: one per partition.
   void apply_batch(const uint32_t *src, const uint32_t *dst, const uint32_t *value, size_t count,
                    std::vector<ppcsr_batch_stats> *stats = nullptr);
+  // Creates the device-side group over the partitions, or recreates it when `cap` records per (sender, receiver)
+  // region or per-update values exceed what it was created for.  A traversal before any batch needs it too.
+  void ensure_group(std::size_t cap, bool values);
+  // Traversals over all partitions on the devices (ppcsr_group_bfs / ppcsr_group_pagerank): hop counts from `start`
+  // (UINT32_MAX = unreached), and `iterations` damped PageRank iterations with the recurrence of PCSR::pagerank.
+  std::vector<uint32_t> bfs_levels(uint32_t start);
+  std::vector<double> pagerank(uint32_t iterations, double damping);
 
  private:
   void build(uint32_t init_n, bool lock_search, bool use_numa);

@@ -1,35 +1,22 @@
 // Breadth-first search with the reference's signature (reference src/utility/bfs.h:15-36): hop counts
-// from start_node, UINT32_MAX for unreached vertices.  A single-shard graph runs the level-synchronous
-// GPU kernel; any other graph type falls back to the generic queue over get_neighbourhood().
+// from start_node, UINT32_MAX for unreached vertices.  Both graph types run level-synchronous GPU kernels:
+// a PCSR on its one shard (ppcsr_bfs), a PPPCSR across all of its partitions (ppcsr_group_bfs).
 #pragma once
 #include <cstdint>
-#include <queue>
 #include <vector>
 
 #include "PCSR.h"
+#include "PPPCSR.h"
 
 template <typename T>
-std::vector<uint32_t> bfs(T &graph, uint32_t start_node) {
-  const uint64_t n = graph.get_n();
-  std::vector<uint32_t> hops(n, UINT32_MAX);
-  if (start_node >= n) return hops;
-  std::queue<uint32_t> frontier;
-  hops[start_node] = 0;
-  frontier.push(start_node);
-  while (!frontier.empty()) {
-    const uint32_t v = frontier.front();
-    frontier.pop();
-    for (const int w : graph.get_neighbourhood((int)v)) {
-      if ((uint64_t)w < n && hops[w] == UINT32_MAX) {
-        hops[w] = hops[v] + 1;
-        frontier.push((uint32_t)w);
-      }
-    }
-  }
-  return hops;
-}
+std::vector<uint32_t> bfs(T &graph, uint32_t start_node);
 
 template <>
 inline std::vector<uint32_t> bfs<PCSR>(PCSR &graph, uint32_t start_node) {
+  return graph.bfs_levels(start_node);
+}
+
+template <>
+inline std::vector<uint32_t> bfs<PPPCSR>(PPPCSR &graph, uint32_t start_node) {
   return graph.bfs_levels(start_node);
 }
