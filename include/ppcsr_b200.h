@@ -231,6 +231,36 @@ int ppcsr_group_bfs(ppcsr_group *g, uint32_t start, uint32_t *dist);
  * redistribution), out[n] on the host; iterations == 0 gives 1/n everywhere.  No host round trip between iterations. */
 int ppcsr_group_pagerank(ppcsr_group *g, uint32_t iterations, double damping, double *out);
 
+/* What one ppcsr_group_repartition did. */
+typedef struct {
+  uint64_t vertices_moved;  /* vertices whose owner changed                                 */
+  uint64_t edges_moved;     /* their out-edges                                              */
+  uint64_t bytes_copied;    /* bytes copied from one shard's buffers to another's (peer or
+                               same device): col + val + num_neighbors + rowptr of the moved
+                               vertices                                                     */
+  uint32_t shards_rebuilt;  /* shards whose vertex range changed                            */
+  float ms_total;           /* host clock around the call, ending after a device synchronise */
+} ppcsr_repartition_stats;
+/* Moves vertex ranges between the shards of the group: afterwards shard r owns the global vertices
+ * [new_starts[r], new_starts[r+1]).  Every vertex whose owner changes goes to its new shard with all its out-edges
+ * (dst >= n included), their values and its num_neighbors; the logical graph is unchanged.  The data moves device to
+ * device (peer memory across GPUs), never through the host.  new_starts has n_shards + 1 entries: new_starts[0] = 0,
+ * new_starts[n_shards] = n (the first vertex of the last shard + its current vertex count: the vertices the last shard
+ * gained through ppcsr_add_nodes can be spread out this way), each entry strictly larger than the one before.  Every
+ * shard whose range changes is rebuilt whole from a CSR of its new range (a root-window layout, DESIGN.md §5b): its
+ * ppcsr_last_stats then describes that rebuild (whole_array = 1, rebalance_bytes / ms_rebalance_kernel = the layout
+ * pass) and its snapshot is invalidated.  Shards whose range stays the same are not touched; identical boundaries
+ * rebuild nothing.  PPCSR_ERR_ARG, with nothing changed: bad boundaries, a shard other than the last that no longer
+ * holds exactly its range, a poisoned shard, a submitted batch not yet waited for.  Every allocation happens before any
+ * shard is modified, so PPCSR_ERR_CAPACITY (a shard would pass 2^31 slots, or device memory ran out) also means
+ * "nothing moved".  PPCSR_ERR_CUDA (fatal, as everywhere) during the build phase leaves the rebuilt shards POISONED:
+ * they then hold neither their old nor their new ranges.  Transient device memory per rebuilt shard of E edges, n vertices and N slots after the call: the
+ * export of its old range and the CSR of its new one, about 2 * (8 E + 12 n) bytes, plus the out-of-place slot
+ * arrays at N (8 N bytes, kept by the shard as it keeps them after a resize).  The traversal buffers of the group
+ * are freed (their sizes depend on the ranges).  Ordered after the group's last apply or traversal, before the next;
+ * stats nullable. */
+int ppcsr_group_repartition(ppcsr_group *g, const uint64_t *new_starts, ppcsr_repartition_stats *stats);
+
 /* ---- reads ---- */
 int ppcsr_geometry_of(ppcsr_shard *h, ppcsr_geometry *out);
 /* reference PCSR::edge_exists (src/pcsr/PCSR.cpp:860-869); `out_value` (nullable) gets the stored value. */
@@ -249,6 +279,15 @@ int ppcsr_node_ranges(ppcsr_shard *h, uint32_t *beginning, uint32_t *end);
 /* Compacted adjacency (the logical graph): rowptr[n+1], then col/val with *edges entries.  Call with
  * col == NULL to size.  Doubles as the snapshot/export of SURVEY.md §5. */
 int ppcsr_export_csr(ppcsr_shard *h, uint64_t *rowptr, uint32_t *col, uint32_t *val, uint64_t *edges);
+/* The inverse: replaces the shard's whole content with the CSR of n vertices (host buffers): rowptr[n+1], col / val
+ * [rowptr[n]] (val NULL: every value 1), nn[n] the num_neighbors (NULL: the row lengths).  The shard is laid out
+ * afresh, as a root-window rebuild would leave it, at the slot count the density bounds give from its current N.  The
+ * input is validated on the device -- rowptr[0] = 0 and non-decreasing, col strictly ascending within a row and never
+ * 0xFFFFFFFF, no value 0 -- and PPCSR_ERR_ARG leaves the shard untouched (as it does for a poisoned shard or a
+ * submitted batch not yet waited for).  Needs no sort: an exported graph loads in one streaming pass.
+ * ppcsr_last_stats describes the layout pass. */
+int ppcsr_load_csr(ppcsr_shard *h, uint32_t n, const uint64_t *rowptr, const uint32_t *col, const uint32_t *val,
+                   const uint32_t *nn);
 /* One PageRank push step, reference src/utility/pagerank.h:16-29: out[dst] += in[v] / num_neighbors[v].
  * `out_len` entries of out are zeroed then accumulated (dst >= out_len is skipped; the reference would
  * write out of bounds).  Accumulation is fp64 on device.  Host buffers. */

@@ -37,6 +37,14 @@ class BatchStats(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_}
 
 
+class RepartitionStats(C.Structure):
+    _fields_ = [("vertices_moved", C.c_uint64), ("edges_moved", C.c_uint64), ("bytes_copied", C.c_uint64),
+                ("shards_rebuilt", C.c_uint32), ("ms_total", C.c_float)]
+
+    def as_dict(self):
+        return {n: getattr(self, n) for n, _ in self._fields_}
+
+
 class Geometry(C.Structure):
     _fields_ = [("N", C.c_uint64), ("logN", C.c_uint32), ("H", C.c_uint32), ("n", C.c_uint64), ("items", C.c_uint64)]
 
@@ -81,6 +89,7 @@ SYMBOLS = {
     "ppcsr_group_apply": (_i, [_vp, _vp, _vp, _vp, _u64, _u32, C.POINTER(BatchStats)]),
     "ppcsr_group_bfs": (_i, [_vp, _u32, _vp]),
     "ppcsr_group_pagerank": (_i, [_vp, _u32, C.c_double, _vp]),
+    "ppcsr_group_repartition": (_i, [_vp, _vp, C.POINTER(RepartitionStats)]),
     "ppcsr_add_edge": (_i, [_vp, _u32, _u32, _u32]),
     "ppcsr_remove_edge": (_i, [_vp, _u32, _u32, C.POINTER(_i)]),
     "ppcsr_add_nodes": (_i, [_vp, _u32]),
@@ -98,6 +107,7 @@ SYMBOLS = {
     "ppcsr_num_neighbors": (_i, [_vp, _vp]),
     "ppcsr_node_ranges": (_i, [_vp, _vp, _vp]),
     "ppcsr_export_csr": (_i, [_vp, _vp, _vp, _vp, C.POINTER(_u64)]),
+    "ppcsr_load_csr": (_i, [_vp, _u32, _vp, _vp, _vp, _vp]),
     "ppcsr_pagerank_step_f64": (_i, [_vp, _vp, _vp, _u64]),
     "ppcsr_pagerank_step_f32": (_i, [_vp, _vp, _vp, _u64]),
     "ppcsr_pagerank_push_device": (_i, [_vp, _vp, _vp, _u64]),
@@ -337,6 +347,24 @@ class Shard:
         _check(self.L.ppcsr_export_csr(self.h, None, _np_ptr(col), _np_ptr(val), C.byref(E)))
         return (rowptr, col, val) if with_values else (rowptr, col)
 
+    def load_csr(self, rowptr, col, val=None, nn=None) -> dict:
+        """Replaces the whole content with a CSR (ppcsr_load_csr): rowptr[n+1], col / val [rowptr[n]] (val None: all
+        1), nn[n] the num_neighbors (None: the row lengths).  Invalid input raises and leaves the shard untouched.
+        Returns the stats of the layout pass."""
+        rowptr = np.ascontiguousarray(rowptr, dtype=np.uint64)
+        n = rowptr.shape[0] - 1
+        col = _u32_array(col)
+        val = _u32_array(val) if val is not None else None
+        nn = _u32_array(nn) if nn is not None else None
+        if (val is not None and val.shape != col.shape) or (nn is not None and nn.shape != (n,)):
+            raise ValueError("val must have one entry per col, nn one per vertex")
+        if n < 0 or int(rowptr[n]) > col.shape[0]:
+            raise ValueError("rowptr[n] exceeds the length of col")
+        _check(self.L.ppcsr_load_csr(self.h, n, _np_ptr(rowptr), _np_ptr(col), _np_ptr(val), _np_ptr(nn)))
+        st = BatchStats()
+        _check(self.L.ppcsr_last_stats(self.h, C.byref(st)))
+        return st.as_dict()
+
     def pagerank_step(self, values, dtype=np.float64, out_len=None):
         values = np.ascontiguousarray(values, dtype=dtype)
         out_len = self.n if out_len is None else out_len
@@ -458,6 +486,17 @@ class Group:
         out = np.zeros(self.n, dtype=np.float64)
         _check(self.L.ppcsr_group_pagerank(self.g, iterations, float(damping), _np_ptr(out)))
         return out
+
+    def repartition(self, new_starts) -> dict:
+        """Moves vertex ranges between the shards (ppcsr_group_repartition): shard r then owns
+        [new_starts[r], new_starts[r+1]).  new_starts runs from 0 to self.n.  Returns the stats."""
+        new_starts = np.ascontiguousarray(new_starts, dtype=np.uint64)
+        if new_starts.shape != (len(self.shards) + 1,):
+            raise ValueError("new_starts needs one entry per shard plus the end")
+        st = RepartitionStats()
+        _check(self.L.ppcsr_group_repartition(self.g, _np_ptr(new_starts), C.byref(st)))
+        self.starts = new_starts.copy()
+        return st.as_dict()
 
     def close(self):
         if getattr(self, "g", None):

@@ -1,6 +1,7 @@
 // capi.cu -- C-ABI (include/ppcsr_b200.h) and host orchestration of the batch pipeline.
 // Unity build: all kernels are included here and compiled for sm_100a only.
 #include <algorithm>
+#include <chrono>
 #include <cmath>
 #include <mutex>
 #include <string>
@@ -9,6 +10,7 @@
 
 #include "batch.cuh"
 #include "common.cuh"
+#include "migrate.cuh"
 #include "parse.cuh"
 #include "primitives.cuh"
 #include "queries.cuh"
@@ -711,6 +713,122 @@ static int snap_copy(ppcsr_shard *s, DevBuf<T> &dst, const DevBuf<T> &src, size_
   if (elems) CUDA_TRY(cudaMemcpyAsync(dst.p, src.p, elems * sizeof(T), cudaMemcpyDeviceToDevice, s->stream));
   return PPCSR_OK;
 }
+
+// ---- a shard's content as a device-resident CSR, and a shard laid out afresh from one (migrate.cuh) ------------
+struct DevCsr {
+  DevBuf<uint64_t> rowptr;        // [n + 1]
+  DevBuf<uint32_t> col, val, nn;  // [E], [E], [n]
+};
+void csr_free(int device, DevCsr &c) {
+  cudaSetDevice(device);
+  dev_free(c.rowptr);
+  dev_free(c.col);
+  dev_free(c.val);
+  dev_free(c.nn);
+}
+
+// The compacted adjacency of the shard into device buffers (each nullable): rowptr[n + 1], col / val [E], enqueued on
+// the shard's stream.  The body of ppcsr_export_csr.
+int export_device(ppcsr_shard *s, DevBuf<uint64_t> *rowptr, DevBuf<uint32_t> *col, DevBuf<uint32_t> *val) {
+  const uint64_t E = s->items - s->n;
+  const Geometry g = s->geo;
+  if (rowptr) {
+    PPCSR_TRY(refresh_rank_off(s));
+    PPCSR_TRY(dev_reserve(*rowptr, (size_t)s->n + 1, s->stream));
+    qry::k_rowptr<<<div_up((uint64_t)s->n + 1, qry::QT), qry::QT, 0, s->stream>>>(s->beg.p, s->rank_off.p, g.leaf_shift,
+                                                                                s->n, rowptr->p);
+    CUDA_TRY(cudaGetLastError());
+  }
+  if (col && E) {
+    PPCSR_TRY(dev_reserve(*col, E, s->stream));
+    if (val) PPCSR_TRY(dev_reserve(*val, E, s->stream));
+    PPCSR_TRY(prim::device_scan(s, qry::InIsEdge{s->dest.p, s->leaf_cnt.p, g.leaf_shift},
+                                qry::OutEdge{s->dest.p, s->val.p, col->p, val ? val->p : nullptr}, g.N, nullptr,
+                                nullptr));
+  }
+  return PPCSR_OK;
+}
+
+// Slots of a shard laid out afresh with `items` live slots, starting from its current N: grown while the root would be
+// above its upper bound, otherwise shrunk while it is below its lower bound (the rules of a batch that reaches the
+// root).  0: more than 2^31 slots.
+uint64_t layout_slots(uint64_t N, uint64_t items) {
+  const Geometry g = make_geometry(N);
+  if (!window_ok_upper(items, N, g.logN, 0, (int)g.H)) return grown_slots(N, items);
+  return shrunk_slots(N, items);
+}
+
+// Every array a layout of n vertices at N slots writes, allocated before the shard is modified: the out-of-place
+// target at N, and tree / leaf counts / beg / nn with their contents kept, so that a failure leaves the shard intact.
+int reserve_layout(ppcsr_shard *s, uint64_t N, uint32_t n) {
+  const Geometry g2 = make_geometry(N);
+  PPCSR_TRY(dev_reserve(s->dest_alt, g2.N, s->stream));
+  PPCSR_TRY(dev_reserve(s->val_alt, g2.N, s->stream));
+  PPCSR_TRY(dev_reserve(s->tree, (size_t)2 * g2.n_leaves, s->stream, true));
+  PPCSR_TRY(dev_reserve(s->leaf_cnt, g2.n_leaves, s->stream, true));
+  PPCSR_TRY(dev_reserve(s->beg, (size_t)n + 1, s->stream, true));
+  PPCSR_TRY(dev_reserve(s->nn, (size_t)n + 1, s->stream, true));
+  PPCSR_TRY(reserve_leaf_arrays(s, g2));
+  return PPCSR_OK;
+}
+
+// Replaces the shard's content with the device CSR (n vertices, E edges; d_val NULL: every value 1, d_nn NULL:
+// num_neighbors = row lengths), laid out at N slots (reserve_layout first).  Enqueued only: layout_stats reads the
+// timings.  Leaves the state a whole-array rebuild leaves: per-leaf counters clear, every leaf rewritten.
+int commit_layout(ppcsr_shard *s, uint64_t N, uint32_t n, const uint64_t *d_rowptr, const uint32_t *d_col,
+                  const uint32_t *d_val, const uint32_t *d_nn, uint64_t E, ppcsr_batch_stats *st) {
+  const Geometry g = s->geo, g2 = make_geometry(N);
+  *st = ppcsr_batch_stats{};
+  st->slots_before = g.N;
+  st->slots_after = g2.N;
+  st->resized = g2.N > g.N ? 1 : g2.N < g.N ? 2 : 0;
+  st->whole_array = 1;
+  st->n_windows = 1;
+  st->window_slots = g2.N;
+  // CSR reads (col + val per edge, rowptr per vertex) + slot writes (dest + val) + beg
+  st->rebalance_bytes = 8ull * E + 8ull * n + 8ull * g2.N + 4ull * n;
+  s->launches = 0;
+  CUDA_TRY(cudaEventRecord(s->ev[0], s->stream));
+  if (n) {
+    if (d_nn) CUDA_TRY(cudaMemcpyAsync(s->nn.p, d_nn, (size_t)n * 4, cudaMemcpyDeviceToDevice, s->stream));
+    else mig::k_row_lengths<<<div_up(n, mig::MT), mig::MT, 0, s->stream>>>(d_rowptr, n, s->nn.p);
+  }
+  CUDA_TRY(cudaEventRecord(s->ev[5], s->stream));
+  s->launches++;
+  mig::k_layout_from_csr<<<div_up((uint64_t)g2.n_leaves * 32, mig::MT), mig::MT, 0, s->stream>>>(
+      d_rowptr, d_col, d_val, 1u, n, E + n, g2.H, g2.leaf_shift, s->dest_alt.p, s->val_alt.p, s->beg.p, s->leaf_cnt.p,
+      s->tree.p + g2.n_leaves);
+  CUDA_TRY(cudaEventRecord(s->ev[6], s->stream));
+  CUDA_TRY(cudaGetLastError());
+  PPCSR_TRY(win::tree_rebuild(s, s->tree.p, g2.H));
+  reb::k_set_u32<<<1, 1, 0, s->stream>>>(s->beg.p + n, (uint32_t)g2.N);
+  CUDA_TRY(cudaMemsetAsync(s->ins_cnt.p, 0, (size_t)g2.n_leaves * sizeof(uint32_t), s->stream));
+  CUDA_TRY(cudaMemsetAsync(s->del_cnt.p, 0, (size_t)g2.n_leaves * sizeof(uint32_t), s->stream));
+  CUDA_TRY(cudaGetLastError());
+  std::swap(s->dest, s->dest_alt);
+  std::swap(s->val, s->val_alt);
+  s->geo = g2;
+  s->n = n;
+  s->items = E + n;
+  s->cnt_clean = true;
+  s->last_sparse = false;
+  s->all_touched = 4u | 1u;
+  CUDA_TRY(cudaEventRecord(s->ev[4], s->stream));
+  return PPCSR_OK;
+}
+
+// waits for a commit_layout and fills in its timings; the stats become the shard's ppcsr_last_stats
+int layout_stats(ppcsr_shard *s, ppcsr_batch_stats *st) {
+  CUDA_TRY(cudaEventSynchronize(s->ev[4]));
+  CUDA_TRY(cudaEventElapsedTime(&st->ms_total, s->ev[0], s->ev[4]));
+  CUDA_TRY(cudaEventElapsedTime(&st->ms_rebalance, s->ev[5], s->ev[4]));
+  CUDA_TRY(cudaEventElapsedTime(&st->ms_rebalance_kernel, s->ev[5], s->ev[6]));
+  st->kernel_launches = s->launches;
+  s->last = *st;
+  return PPCSR_OK;
+}
+
+bool submit_pending(const ppcsr_shard *s) { return s->pending[0].busy || s->pending[1].busy; }
 
 }  // namespace
 
@@ -1699,32 +1817,77 @@ int ppcsr_export_csr(ppcsr_shard *s, uint64_t *rowptr, uint32_t *col, uint32_t *
   PPCSR_TRY(set_device(s));
   const uint64_t E = s->items - s->n;
   if (edges) *edges = E;
-  const Geometry g = s->geo;
-  if (rowptr) {
-    PPCSR_TRY(refresh_rank_off(s));
-    DevBuf<uint64_t> d_row;
-    PPCSR_TRY(dev_reserve(d_row, (size_t)s->n + 1, s->stream));
-    qry::k_rowptr<<<div_up((uint64_t)s->n + 1, qry::QT), qry::QT, 0, s->stream>>>(s->beg.p, s->rank_off.p, g.leaf_shift,
-                                                                                s->n, d_row.p);
+  DevCsr d;
+  const int rc = [&]() -> int {
+    PPCSR_TRY(export_device(s, rowptr ? &d.rowptr : nullptr, col ? &d.col : nullptr, col && val ? &d.val : nullptr));
+    if (rowptr)
+      CUDA_TRY(cudaMemcpyAsync(rowptr, d.rowptr.p, ((size_t)s->n + 1) * 8, cudaMemcpyDeviceToHost, s->stream));
+    if (col && E) {
+      CUDA_TRY(cudaMemcpyAsync(col, d.col.p, E * 4, cudaMemcpyDeviceToHost, s->stream));
+      if (val) CUDA_TRY(cudaMemcpyAsync(val, d.val.p, E * 4, cudaMemcpyDeviceToHost, s->stream));
+    }
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    return PPCSR_OK;
+  }();
+  csr_free(s->device, d);
+  return rc;
+}
+
+int ppcsr_load_csr(ppcsr_shard *s, uint32_t n, const uint64_t *rowptr, const uint32_t *col, const uint32_t *val,
+                   const uint32_t *nn) {
+  if (!s || !rowptr) return PPCSR_ERR_ARG;
+  PPCSR_TRY(set_device(s));
+  if (s->poisoned) {
+    g_ppcsr_error = "ppcsr_load_csr: the shard is poisoned by a failed batch; ppcsr_restore it first";
+    return PPCSR_ERR_ARG;
+  }
+  if (submit_pending(s)) {
+    g_ppcsr_error = "ppcsr_load_csr: a submitted batch is still pending; ppcsr_wait for it first";
+    return PPCSR_ERR_ARG;
+  }
+  if ((uint64_t)n >= 0xFFFFFFFEull || rowptr[0] != 0 || (rowptr[n] && !col)) {
+    g_ppcsr_error = "ppcsr_load_csr: rowptr[0] must be 0, n below 2^32 - 2, and col given when there are edges";
+    return PPCSR_ERR_ARG;
+  }
+  const uint64_t E = rowptr[n];
+  const uint64_t N2 = E < PPCSR_MAX_SLOTS ? layout_slots(s->geo.N, E + n) : 0;
+  if (N2 == 0) {
+    g_ppcsr_error = "ppcsr_load_csr: edge array would exceed 2^31 slots";
+    return PPCSR_ERR_CAPACITY;
+  }
+  DevCsr d;
+  const int rc = [&]() -> int {
+    // the input, then its validation on the device: nothing of the shard is modified before it passes
+    PPCSR_TRY(dev_reserve(d.rowptr, (size_t)n + 1, s->stream));
+    PPCSR_TRY(dev_reserve(d.col, E, s->stream));
+    if (val) PPCSR_TRY(dev_reserve(d.val, E, s->stream));
+    if (nn) PPCSR_TRY(dev_reserve(d.nn, n, s->stream));
+    PPCSR_TRY(dev_reserve(s->misc, 16, s->stream));
+    CUDA_TRY(cudaMemcpyAsync(d.rowptr.p, rowptr, ((size_t)n + 1) * 8, cudaMemcpyHostToDevice, s->stream));
+    if (E) CUDA_TRY(cudaMemcpyAsync(d.col.p, col, E * 4, cudaMemcpyHostToDevice, s->stream));
+    if (E && val) CUDA_TRY(cudaMemcpyAsync(d.val.p, val, E * 4, cudaMemcpyHostToDevice, s->stream));
+    if (n && nn) CUDA_TRY(cudaMemcpyAsync(d.nn.p, nn, (size_t)n * 4, cudaMemcpyHostToDevice, s->stream));
+    CUDA_TRY(cudaMemsetAsync(s->misc.p, 0, 4, s->stream));
+    mig::k_validate_csr<<<div_up(std::max<uint64_t>((uint64_t)n + 1, E), mig::MT), mig::MT, 0, s->stream>>>(
+        d.rowptr.p, d.col.p, val ? d.val.p : nullptr, n, E, s->misc.p);
     CUDA_TRY(cudaGetLastError());
-    CUDA_TRY(cudaMemcpyAsync(rowptr, d_row.p, ((size_t)s->n + 1) * 8, cudaMemcpyDeviceToHost, s->stream));
+    uint32_t *hp = reinterpret_cast<uint32_t *>(s->h_pinned);
+    CUDA_TRY(cudaMemcpyAsync(hp, s->misc.p, 4, cudaMemcpyDeviceToHost, s->stream));
     CUDA_TRY(cudaStreamSynchronize(s->stream));
-    dev_free(d_row);
-  }
-  if (col && E) {
-    DevBuf<uint32_t> d_col, d_w;
-    PPCSR_TRY(dev_reserve(d_col, E, s->stream));
-    if (val) PPCSR_TRY(dev_reserve(d_w, E, s->stream));
-    PPCSR_TRY(prim::device_scan(s, qry::InIsEdge{s->dest.p, s->leaf_cnt.p, g.leaf_shift},
-                                qry::OutEdge{s->dest.p, s->val.p, d_col.p, val ? d_w.p : nullptr}, g.N, nullptr,
-                                nullptr));
-    CUDA_TRY(cudaMemcpyAsync(col, d_col.p, E * 4, cudaMemcpyDeviceToHost, s->stream));
-    if (val) CUDA_TRY(cudaMemcpyAsync(val, d_w.p, E * 4, cudaMemcpyDeviceToHost, s->stream));
-    CUDA_TRY(cudaStreamSynchronize(s->stream));
-    dev_free(d_col);
-    dev_free(d_w);
-  }
-  return PPCSR_OK;
+    if (hp[0]) {
+      g_ppcsr_error = std::string("ppcsr_load_csr: invalid CSR:") + ((hp[0] & 1u) ? " rowptr not 0 .. E non-decreasing;" : "") +
+                      ((hp[0] & 2u) ? " col holds 0xFFFFFFFF;" : "") + ((hp[0] & 4u) ? " a value is 0;" : "") +
+                      ((hp[0] & 8u) ? " a row is not strictly ascending;" : "");
+      return PPCSR_ERR_ARG;
+    }
+    PPCSR_TRY(reserve_layout(s, N2, n));
+    ppcsr_batch_stats st;
+    PPCSR_TRY(commit_layout(s, N2, n, d.rowptr.p, d.col.p, val ? d.val.p : nullptr, nn ? d.nn.p : nullptr, E, &st));
+    PPCSR_TRY(layout_stats(s, &st));
+    return PPCSR_OK;
+  }();
+  csr_free(s->device, d);
+  return rc;
 }
 
 int ppcsr_pagerank_push_device(ppcsr_shard *s, const double *d_in, double *d_out, uint64_t out_len) {

@@ -153,3 +153,17 @@ std::vector<double> PPPCSR::pagerank(uint32_t iterations, double damping) {
   }
   return r;
 }
+
+ppcsr_repartition_stats PPPCSR::repartition(const std::vector<size_t> &boundaries) {
+  ensure_group(0, false);
+  std::vector<uint64_t> starts(boundaries.begin(), boundaries.end());
+  starts.push_back(get_n());
+  ppcsr_repartition_stats st{};
+  if (starts.size() != partitions.size() + 1 || ppcsr_group_repartition(group_, starts.data(), &st) != PPCSR_OK) {
+    std::cout << "ppcsr_group_repartition failed: " << ppcsr_last_error() << ". Abort\n";
+    std::exit(EXIT_FAILURE);
+  }
+  distribution = boundaries;
+  for (auto &part : partitions) part.batch_applied();
+  return st;
+}

@@ -54,6 +54,10 @@ class PPPCSR {
   // (UINT32_MAX = unreached), and `iterations` damped PageRank iterations with the recurrence of PCSR::pagerank.
   std::vector<uint32_t> bfs_levels(uint32_t start);
   std::vector<double> pagerank(uint32_t iterations, double damping);
+  // Moves vertex ranges between the partitions on the devices (ppcsr_group_repartition): partition p then starts at
+  // boundaries[p] (boundaries[0] == 0, strictly ascending, one entry per partition; the last partition ends at
+  // get_n()).  The logical graph is unchanged.
+  ppcsr_repartition_stats repartition(const std::vector<size_t> &boundaries);
 
  private:
   void build(uint32_t init_n, bool lock_search, bool use_numa);
