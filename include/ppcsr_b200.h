@@ -215,6 +215,31 @@ uint32_t ppcsr_group_owner(const ppcsr_group *g, uint64_t vertex); /* reference 
  * then every shard applies what it received.  stats (nullable) gets one entry per shard. */
 int ppcsr_group_apply(ppcsr_group *g, const uint32_t *src, const uint32_t *dst, const uint32_t *val, uint64_t count,
                       uint32_t default_val, ppcsr_batch_stats *stats);
+/* Pipelined form of ppcsr_group_apply for a stream of batches (replaces a sequence of ThreadPoolPPPCSR start()/stop()
+ * regions): ppcsr_group_submit starts the host->device copy of every slice (cut as ppcsr_group_apply cuts it) and
+ * enqueues its binning and peer stores on the sending shard's copy stream, then returns at once with a ticket -- no
+ * host synchronisation; ppcsr_group_wait(ticket) makes every shard apply what it received
+ * (ppcsr_apply_batch_segments_device, one host thread per shard) and returns the per-shard stats (n_shards entries,
+ * nullable).  With
+ *     submit(b0); for i: { submit(b[i+1]); wait(b[i]); }
+ * the copy and routing of batch i+1 run on the devices while the shards apply batch i, and the graph, num_neighbors
+ * and per-shard counters are exactly those of ppcsr_group_apply(b0); ppcsr_group_apply(b1); ...  Global ids, values,
+ * default_val and the with_values rule are those of ppcsr_group_apply.  At most two batches in flight, applied in
+ * submission order: a third submit, a wait for the newer ticket first or for an unknown ticket return PPCSR_ERR_ARG.
+ * The host buffers must stay valid until the matching wait returns; they should be page-locked.  A slice above
+ * region_cap or a failed allocation returns PPCSR_ERR_CAPACITY with nothing in flight: everything the routing needs
+ * is allocated in submit.  A failing wait reports the first failing shard, as ppcsr_group_apply does; the other batch
+ * in flight stays valid and is applied by its own wait.  While a batch is in flight, ppcsr_group_apply,
+ * ppcsr_group_bfs, ppcsr_group_pagerank and ppcsr_group_repartition return PPCSR_ERR_ARG and change nothing, and the
+ * group's shards must not be modified through shard-level calls; ppcsr_group_destroy synchronises and frees the
+ * batches in flight without applying them.  Ordering: a streamed batch is ordered after the group's last apply,
+ * traversal or repartition and before the next, also when the shards run on external streams (ppcsr_set_stream).
+ * Device memory, allocated on the first submit and kept until ppcsr_group_destroy: per receiver a second receive set,
+ * n_shards * region_cap * (8 [+ 4 with values]) B plus n_shards * 8 B of counts; per sender two staging slots of its
+ * slice, 2 * slice * (8 [+ 4 with values]) B.  A group that only uses ppcsr_group_apply allocates none of it. */
+int ppcsr_group_submit(ppcsr_group *g, const uint32_t *src, const uint32_t *dst, const uint32_t *val, uint64_t count,
+                       uint32_t default_val, uint64_t *ticket);
+int ppcsr_group_wait(ppcsr_group *g, uint64_t ticket, ppcsr_batch_stats *stats);
 /* Traversals across all shards of the group, on the devices.  n = starts[n_shards-1] + (vertices of the last shard
  * now): the last shard may have grown through ppcsr_add_nodes (PPPCSR::add_node appends there); if any other shard no
  * longer holds exactly its range, both calls return PPCSR_ERR_ARG.  All work of shard r runs on shard r's stream, the

@@ -87,6 +87,8 @@ SYMBOLS = {
     "ppcsr_group_destroy": (None, [_vp]),
     "ppcsr_group_owner": (_u32, [_vp, _u64]),
     "ppcsr_group_apply": (_i, [_vp, _vp, _vp, _vp, _u64, _u32, C.POINTER(BatchStats)]),
+    "ppcsr_group_submit": (_i, [_vp, _vp, _vp, _vp, _u64, _u32, C.POINTER(_u64)]),
+    "ppcsr_group_wait": (_i, [_vp, _u64, C.POINTER(BatchStats)]),
     "ppcsr_group_bfs": (_i, [_vp, _u32, _vp]),
     "ppcsr_group_pagerank": (_i, [_vp, _u32, C.c_double, _vp]),
     "ppcsr_group_repartition": (_i, [_vp, _vp, C.POINTER(RepartitionStats)]),
@@ -467,6 +469,28 @@ class Group:
         _check(self.L.ppcsr_group_apply(self.g, _np_ptr(src), _np_ptr(dst), _np_ptr(val), src.shape[0], default_val, st))
         return [x.as_dict() for x in st]
 
+    def submit(self, src, dst, val=None, default_val: int = 1) -> int:
+        """Pipelined submit (ppcsr_group_submit): starts the copy and the routing of the batch, returns a ticket for
+        wait().  The arrays must stay alive (and should be pinned) until wait() returns; they are kept referenced
+        here.  At most two batches in flight, waited for in submission order."""
+        src = _u32_array(src)
+        dst = _u32_array(dst, src.shape[0])
+        val = _u32_array(val, src.shape[0]) if val is not None else None
+        t = C.c_uint64()
+        _check(self.L.ppcsr_group_submit(self.g, _np_ptr(src), _np_ptr(dst), _np_ptr(val), src.shape[0], default_val,
+                                         C.byref(t)))
+        if not hasattr(self, "_inflight"):
+            self._inflight = {}
+        self._inflight[t.value] = (src, dst, val)
+        return t.value
+
+    def wait(self, ticket: int) -> list[dict]:
+        """Applies the submitted batch on every shard (ppcsr_group_wait); one stats dict per shard."""
+        st = (BatchStats * len(self.shards))()
+        _check(self.L.ppcsr_group_wait(self.g, ticket, st))
+        self._inflight.pop(ticket, None)
+        return [x.as_dict() for x in st]
+
     def owner(self, v: int) -> int:
         return int(self.L.ppcsr_group_owner(self.g, v))
 
@@ -502,6 +526,7 @@ class Group:
         if getattr(self, "g", None):
             self.L.ppcsr_group_destroy(self.g)
             self.g = None
+            self._inflight = {}  # the destroy synchronised: no copy reads them any more
             for s in self.shards:
                 s.close()
 

@@ -40,6 +40,10 @@ PPPCSR::~PPPCSR() {
 void PPPCSR::ensure_group(std::size_t cap, bool values) {
   const std::size_t parts = partitions.size();
   if (group_ && cap <= group_cap_ && (!values || group_values_)) return;
+  if (in_flight_) {  // destroying the group would drop the batches in flight
+    std::cout << "PPPCSR: a batch needs a larger group while submitted batches are in flight. Abort\n";
+    std::exit(EXIT_FAILURE);
+  }
   if (group_) ppcsr_group_destroy(group_);  // (re)size the receive buffers
   group_ = nullptr;
   std::vector<ppcsr_shard *> handles;
@@ -69,6 +73,29 @@ void PPPCSR::apply_batch(const uint32_t *src, const uint32_t *dst, const uint32_
     std::cout << "ppcsr_group_apply failed: " << ppcsr_last_error() << ". Abort\n";
     std::exit(EXIT_FAILURE);
   }
+  for (auto &part : partitions) part.batch_applied();
+  if (stats) *stats = st;
+}
+
+uint64_t PPPCSR::submit_batch(const uint32_t *src, const uint32_t *dst, const uint32_t *value, size_t count) {
+  const std::size_t parts = partitions.size();
+  ensure_group((count + parts - 1) / parts, value != nullptr);
+  uint64_t ticket = 0;
+  if (ppcsr_group_submit(group_, src, dst, value, count, 1, &ticket) != PPCSR_OK) {
+    std::cout << "ppcsr_group_submit failed: " << ppcsr_last_error() << ". Abort\n";
+    std::exit(EXIT_FAILURE);
+  }
+  in_flight_++;
+  return ticket;
+}
+
+void PPPCSR::wait_batch(uint64_t ticket, std::vector<ppcsr_batch_stats> *stats) {
+  std::vector<ppcsr_batch_stats> st(partitions.size());
+  if (ppcsr_group_wait(group_, ticket, st.data()) != PPCSR_OK) {
+    std::cout << "ppcsr_group_wait failed: " << ppcsr_last_error() << ". Abort\n";
+    std::exit(EXIT_FAILURE);
+  }
+  in_flight_--;
   for (auto &part : partitions) part.batch_applied();
   if (stats) *stats = st;
 }

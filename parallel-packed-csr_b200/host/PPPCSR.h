@@ -47,8 +47,16 @@ class PPPCSR {
   // per-op hand-over of reference ThreadPoolPPPCSR::submit_* (thread_pool_pppcsr.cpp:96-118).  stats: one per partition.
   void apply_batch(const uint32_t *src, const uint32_t *dst, const uint32_t *value, size_t count,
                    std::vector<ppcsr_batch_stats> *stats = nullptr);
+  // The same batch as a stream (C-ABI ppcsr_group_submit / ppcsr_group_wait): submit_batch starts the copy and the
+  // routing and returns a ticket, wait_batch applies that batch on every partition.  With
+  //     submit(b0); for i: { submit(b[i+1]); wait(b[i]); }
+  // batch i+1 is routed while the partitions apply batch i, with the result of apply_batch(b0); apply_batch(b1); ...
+  // At most two batches in flight, waited for in submission order; the arrays must stay valid until the wait.
+  uint64_t submit_batch(const uint32_t *src, const uint32_t *dst, const uint32_t *value, size_t count);
+  void wait_batch(uint64_t ticket, std::vector<ppcsr_batch_stats> *stats = nullptr);
   // Creates the device-side group over the partitions, or recreates it when `cap` records per (sender, receiver)
-  // region or per-update values exceed what it was created for.  A traversal before any batch needs it too.
+  // region or per-update values exceed what it was created for (never while a submitted batch is in flight).  A
+  // traversal before any batch needs it too.
   void ensure_group(std::size_t cap, bool values);
   // Traversals over all partitions on the devices (ppcsr_group_bfs / ppcsr_group_pagerank): hop counts from `start`
   // (UINT32_MAX = unreached), and `iterations` damped PageRank iterations with the recurrence of PCSR::pagerank.
@@ -67,4 +75,5 @@ class PPPCSR {
   ppcsr_group *group_ = nullptr;     // device-side router over the partitions, (re)created for the largest batch seen
   size_t group_cap_ = 0;
   bool group_values_ = false;
+  int in_flight_ = 0;                // batches submitted and not yet waited for
 };

@@ -18,6 +18,10 @@
 // "Repartition: moved <V> vertices <E> edges, <S> partitions rebuilt, <ms> ms" -- -check, -checksum and the traversals
 // then run on the new layout; -checksum prints an order-independent checksum of the logical graph
 // ("Graph checksum: edges <E> edge_hash <016x>").
+// -batches=<k> cuts the update phase (the first `size` updates) into k consecutive batches of ceil(size / k) and streams
+// them two ahead (-ppcsr: ppcsr_submit_batch / ppcsr_wait; partitioned modes: PPPCSR::submit_batch / wait_batch), so the
+// copy (and, partitioned, the routing) of the next batch runs while the current one is applied; the second "Elapsed
+// wall clock time" line covers the whole stream, "not found" sums over its batches.  Default 1: one batch.
 // Traversals after the updates, on the devices (-ppcsr: one shard; partitioned modes: across all partitions):
 //   -bfs=<start>         prints "BFS from <start>: reached <k> levels <L> hash <016x>": k reached vertices, L = 1 + the
 //                        largest hop count (0 if nothing is reached), hash = sum mod 2^64 of
@@ -188,9 +192,10 @@ static void run_phase(const EdgeArrays &e, Pool *pool, int threads, size_t count
 }
 
 template <typename Pool>
-static void execute(int threads, int size, const EdgeArrays &core, const EdgeArrays &updates,
+static void execute(int threads, int size, int batches, const EdgeArrays &core, const EdgeArrays &updates,
                     std::unique_ptr<Pool> &pool) {
   run_phase(core, pool.get(), threads, core.size());
+  pool->set_batches(batches);
   run_phase(updates, pool.get(), threads, (size_t)size);
 }
 
@@ -277,7 +282,7 @@ static void run_traversals(G &graph, long bfs_start, long pr_iterations) {
 }
 
 int main(int argc, char *argv[]) {
-  int threads = 8, size = 1000000, num_nodes = 0, partitions_per_domain = 1;
+  int threads = 8, size = 1000000, num_nodes = 0, partitions_per_domain = 1, batches = 1;
   bool lock_search = true, insert = true, check = false, host_parse = false, balanced = false, checksum = false,
        repartition = false;
   long bfs_start = -1, pr_iterations = -1;  // -bfs= / -pagerank= (negative: not requested)
@@ -305,6 +310,14 @@ int main(int argc, char *argv[]) {
       partitions_per_domain = std::stoi(s.substr(23));
     } else if (starts_with(s, "-gpus=")) {
       setenv("PPCSR_GPUS", s.substr(6).c_str(), 1);
+    } else if (starts_with(s, "-batches=")) {
+      char *end = nullptr;
+      const long k = std::strtol(s.c_str() + 9, &end, 10);
+      if (end == s.c_str() + 9 || *end != '\0' || k < 1 || k > 0x7FFFFFFF) {
+        std::cout << "Invalid -batches value (a number >= 1 expected): " << s.substr(9) << std::endl;
+        return EXIT_FAILURE;
+      }
+      batches = (int)k;
     } else if (starts_with(s, "-bfs=")) {
       bfs_start = std::stol(s.substr(5));
     } else if (starts_with(s, "-pagerank=")) {
@@ -343,7 +356,7 @@ int main(int argc, char *argv[]) {
   uint64_t sum[3] = {0, 0, 0};  // -checksum: edges, edge hash, num_neighbors hash of the logical graph
   if (v == Version::PPCSR) {
     auto pool = std::make_unique<ThreadPool>(threads, lock_search, num_nodes + 1, partitions_per_domain);
-    execute(threads, size, core_graph, updates, pool);
+    execute(threads, size, batches, core_graph, updates, pool);
     const ppcsr_batch_stats &st = pool->last_stats();
     std::cout << "{\"updates\": " << st.batch_size << ", \"device_ms\": " << st.ms_total
               << ", \"rebalance_bytes_per_update\": " << (st.batch_size ? (double)st.rebalance_bytes / st.batch_size : 0)
@@ -365,7 +378,7 @@ int main(int argc, char *argv[]) {
       pool = std::make_unique<ThreadPoolPPPCSR>(threads, lock_search, num_nodes + 1, partitions_per_domain,
                                                 v == Version::PPPCSRNUMA);
     }
-    execute(threads, size, core_graph, updates, pool);
+    execute(threads, size, batches, core_graph, updates, pool);
     const auto &sts = pool->last_stats();
     uint64_t upd = 0, bytes = 0, windows = 0;
     float device_ms = 0;

@@ -1,7 +1,10 @@
 // ThreadPool over one GPU shard: see thread_pool.h.
 #include "thread_pool.h"
 
+#include <cstdlib>
 #include <iostream>
+
+#include "stream.h"
 
 ThreadPool::ThreadPool(const int NUM_OF_THREADS, bool lock_search, uint32_t init_num_nodes, int partitions_per_domain)
     : finished_(false), threads_(NUM_OF_THREADS) {
@@ -46,7 +49,31 @@ void ThreadPool::start(int threads) {
   finished_ = false;
   std::cout << "Thread 0 has " << src_.size() + reads_.size() << " tasks" << std::endl;
   pcsr->edges.global_lock->registerThread();
-  if (!src_.empty()) pcsr->apply_batch(src_, dst_, val_, &stats_);
+  if (batches_ > 1 && !src_.empty()) {
+    stats_ = ppcsr_batch_stats{};
+    ppcsr_shard *h = pcsr->handle();
+    stream_batches(
+        src_.size(), (size_t)batches_,
+        [&](size_t lo, size_t len) {
+          uint64_t ticket = 0;
+          if (ppcsr_submit_batch(h, src_.data() + lo, dst_.data() + lo, val_.data() + lo, len, 1, &ticket) != PPCSR_OK) {
+            std::cout << "ppcsr_submit_batch failed: " << ppcsr_last_error() << ". Abort\n";
+            std::exit(EXIT_FAILURE);
+          }
+          return ticket;
+        },
+        [&](uint64_t ticket) {
+          ppcsr_batch_stats st{};
+          if (ppcsr_wait(h, ticket, &st) != PPCSR_OK) {
+            std::cout << "ppcsr_wait failed: " << ppcsr_last_error() << ". Abort\n";
+            std::exit(EXIT_FAILURE);
+          }
+          add_batch_stats(stats_, st);
+        });
+    pcsr->batch_applied();
+  } else if (!src_.empty()) {
+    pcsr->apply_batch(src_, dst_, val_, &stats_);
+  }
   for (int v : reads_) pcsr->read_neighbourhood(v);
   pcsr->edges.global_lock->unregisterThread();
 }

@@ -26,6 +26,9 @@ class ThreadPool {
   void submit_bulk(const uint32_t *src, const uint32_t *dst, const uint32_t *value, size_t count);
   void start(int threads);
   void stop();
+  // start() applies the staged updates as `k` consecutive batches of ceil(count / k), streamed two ahead through
+  // ppcsr_submit_batch / ppcsr_wait (k = 1: one batch); last_stats() then sums the counters over the batches
+  void set_batches(int k) { batches_ = k; }
 
   const ppcsr_batch_stats &last_stats() const { return stats_; }
 
@@ -36,4 +39,5 @@ class ThreadPool {
   std::atomic_bool finished_;
   ppcsr_batch_stats stats_{};
   int threads_;
+  int batches_ = 1;
 };

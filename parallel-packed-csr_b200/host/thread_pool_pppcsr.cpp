@@ -6,6 +6,8 @@
 #include <iostream>
 #include <thread>
 
+#include "stream.h"
+
 static int usable_gpus(int threads) {
   int gpus = ppcsr_device_count();
   if (const char *e = std::getenv("PPCSR_GPUS")) gpus = std::min(gpus, std::max(1, std::atoi(e)));
@@ -87,7 +89,19 @@ void ThreadPoolPPPCSR::start(int threads) {
   std::cout << "Thread 0 has " << src_.size() << " tasks for " << pcsr->partition_count()
             << " partitions, routed on the device" << std::endl;
   for (std::size_t p = 0; p < pcsr->partition_count(); p++) pcsr->registerThread((int)p);
-  if (!src_.empty()) pcsr->apply_batch(src_.data(), dst_.data(), val_.data(), src_.size(), &stats_);
+  if (batches_ > 1 && !src_.empty()) {
+    stats_.assign(pcsr->partition_count(), ppcsr_batch_stats{});
+    std::vector<ppcsr_batch_stats> st;
+    stream_batches(
+        src_.size(), (size_t)batches_,
+        [&](size_t lo, size_t len) { return pcsr->submit_batch(src_.data() + lo, dst_.data() + lo, val_.data() + lo, len); },
+        [&](uint64_t ticket) {
+          pcsr->wait_batch(ticket, &st);
+          for (std::size_t p = 0; p < st.size(); p++) add_batch_stats(stats_[p], st[p]);
+        });
+  } else if (!src_.empty()) {
+    pcsr->apply_batch(src_.data(), dst_.data(), val_.data(), src_.size(), &stats_);
+  }
   for (std::size_t p = 0; p < pcsr->partition_count(); p++) pcsr->unregisterThread((int)p);
   for (auto &st : stats_) not_found_ += st.n_not_found;
   for (int v : reads_) pcsr->read_neighbourhood(v);

@@ -30,6 +30,9 @@ class ThreadPoolPPPCSR {
   void submit_bulk(const uint32_t *src, const uint32_t *dst, const uint32_t *value, size_t count);
   void start(int threads);
   void stop();
+  // start() applies the staged updates as `k` consecutive batches of ceil(count / k), streamed two ahead through
+  // PPPCSR::submit_batch / wait_batch (k = 1: one batch); last_stats() then sums the counters over the batches
+  void set_batches(int k) { batches_ = k; }
 
   // thread -> domain table of the reference (thread_pool_pppcsr.cpp:32-47), kept for the CPU-side reads
   const std::vector<int> &thread_to_domain() const { return threadToDomain; }
@@ -47,6 +50,7 @@ class ThreadPoolPPPCSR {
   std::atomic_bool finished_;
   uint64_t not_found_ = 0;
   std::vector<ppcsr_batch_stats> stats_;
+  int batches_ = 1;
 
   const int available_nodes;  // GPUs used as "domains"
   int partitions_per_domain = 1;
