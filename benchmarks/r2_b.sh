@@ -20,7 +20,7 @@ timeout 900 ncu --metrics gpu__time_duration.sum --clock-control none -k 'regex:
     > gpurun_out/${tag}_c4_launches.log 2>&1; echo "ncu launches exit $?"
 # full capture of the hot kernels of the warm-up batch (the core load launches 6 passes + locate + rebalance first)
 timeout 1200 ncu --set full --clock-control none --import-source on \
-    -k 'regex:^(k_rebalance_p|k_os_pass|k_locate)$' --launch-skip 8 -c 8 \
+    -k 'regex:^(k_rebalance_m|k_os_pass|k_locate)$' --launch-skip 8 -c 8 \
     -f -o gpurun_out/${tag}_c4_full python bench.py --only-headline --steps 1 --warmup 1 --e2e-steps 1 \
     > gpurun_out/${tag}_c4_full.log 2>&1; echo "ncu full exit $?"
 ls -la gpurun_out/${tag}_*

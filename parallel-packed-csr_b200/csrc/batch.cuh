@@ -27,74 +27,6 @@ __device__ __forceinline__ uint64_t emit_key(bool ok, uint64_t key, uint32_t v, 
   return (op_bit && v == 0u) ? (key | KEY_OP_BIT) : key;
 }
 
-// ---- raw key sources: the sort's first pass (prim::k_os_pass / k_os_hist / k_sort_small) builds the key word of
-// update i straight from the caller's arrays, guards included, so the unsorted batch is never written as a key array.
-// Same arithmetic as the builders below (which then only take the scalars and the histograms).
-__device__ __forceinline__ bool update_ok(uint32_t s, uint32_t d, uint32_t v, uint32_t n) {
-  return s < n && !(v != 0 && d == PPCSR_SENT);
-}
-struct RawArrays {
-  const uint32_t *src, *dst, *val;  // val nullable: every update carries default_val
-  uint32_t default_val, n, op_bit;
-  __device__ __forceinline__ uint64_t key(size_t i) const {
-    const uint32_t s = src[i], d = dst[i], v = val ? val[i] : default_val;
-    return emit_key(update_ok(s, d, v, n), ((uint64_t)s << 32) | d, v, n, op_bit);
-  }
-  __device__ __forceinline__ uint32_t payload(size_t i) const {
-    const uint32_t v = val[i];
-    return update_ok(src[i], dst[i], v, n) ? v : 0u;
-  }
-};
-struct RawPacked {
-  const uint64_t *packed;
-  const uint32_t *val;
-  uint32_t default_val, n, op_bit, swap_halves;
-  __device__ __forceinline__ uint64_t word(size_t i) const {
-    const uint64_t k = packed[i];
-    return swap_halves ? (k << 32) | (k >> 32) : k;
-  }
-  __device__ __forceinline__ uint64_t key(size_t i) const {
-    const uint64_t k = word(i);
-    const uint32_t v = val ? val[i] : default_val;
-    return emit_key(update_ok((uint32_t)(k >> 32), (uint32_t)k, v, n), k, v, n, op_bit);
-  }
-  __device__ __forceinline__ uint32_t payload(size_t i) const {
-    const uint64_t k = word(i);
-    const uint32_t v = val[i];
-    return update_ok((uint32_t)(k >> 32), (uint32_t)k, v, n) ? v : 0u;
-  }
-};
-// records deposited by the peers: n_seg regions of `cap` records, region r holding prefix[r + 1] - prefix[r] of them
-// (prefix: a DEVICE array written by k_build_keys_segments)
-struct RawSegments {
-  const uint64_t *packed;
-  const uint32_t *val;
-  const unsigned long long *prefix;
-  unsigned long long cap;
-  uint32_t n_seg, default_val, n, op_bit;
-  __device__ __forceinline__ size_t at(size_t i) const {
-    uint32_t lo = 0, hi = n_seg;  // last region with prefix <= i
-    while (hi - lo > 1) {
-      const uint32_t mid = (lo + hi) >> 1;
-      if (prefix[mid] <= i) lo = mid;
-      else hi = mid;
-    }
-    return (size_t)lo * cap + (i - (size_t)prefix[lo]);
-  }
-  __device__ __forceinline__ uint64_t key(size_t i) const {
-    const size_t a = at(i);
-    const uint64_t k = packed[a];
-    const uint32_t v = val ? val[a] : default_val;
-    return emit_key(update_ok((uint32_t)(k >> 32), (uint32_t)k, v, n), k, v, n, op_bit);
-  }
-  __device__ __forceinline__ uint32_t payload(size_t i) const {
-    const size_t a = at(i);
-    const uint64_t k = packed[a];
-    const uint32_t v = val[a];
-    return update_ok((uint32_t)(k >> 32), (uint32_t)k, v, n) ? v : 0u;
-  }
-};
-
 // The key builders can also take the sort's digit histograms (all passes, prim::k_os_hist's job) while the keys pass
 // through their registers: the host SPECULATES the sort layout from the widest dst seen so far and the vertex count,
 // and falls back to prim::k_os_hist when the batch turns out wider (capi.cu).  Saves one read of the batch.
@@ -143,9 +75,9 @@ __global__ void __launch_bounds__(BT) k_build_keys(const uint32_t *__restrict__ 
     const uint32_t v = val ? val[i] : default_val;
     const bool ok = s < n && !(v != 0 && d == PPCSR_SENT);
     const uint64_t kq = emit_key(ok, ((uint64_t)s << 32) | d, v, n, op_bit);
-    if (keys) keys[i] = kq;  // nullptr: the sort reads the raw arrays itself (RawArrays)
+    keys[i] = kq;
     hist_add(s_h, H, kq);
-    if (pay && keys) pay[i] = ok ? v : 0u;
+    if (pay) pay[i] = ok ? v : 0u;
     if (ok) my_or |= d;
     else my_bad++;
     if (pay && ok && v) my_vmax = max(my_vmax, v), my_vinv = max(my_vinv, ~v);
@@ -195,9 +127,9 @@ __global__ void __launch_bounds__(BT) k_build_keys_packed(const uint64_t *__rest
     const uint32_t v = val ? val[i] : default_val;
     const bool ok = s < n && !(v != 0 && d == PPCSR_SENT);
     const uint64_t kq = emit_key(ok, k, v, n, op_bit);
-    if (keys) keys[i] = kq;  // nullptr: the sort reads the raw records itself (RawPacked / RawSegments)
+    keys[i] = kq;
     hist_add(s_h, H, kq);
-    if (pay && keys) pay[i] = ok ? v : 0u;
+    if (pay) pay[i] = ok ? v : 0u;
     if (ok) my_or |= d;
     else my_bad++;
     if (pay && ok && v) my_vmax = max(my_vmax, v), my_vinv = max(my_vinv, ~v);
@@ -228,7 +160,6 @@ struct SegmentTable {
   uint32_t n_seg;
   uint64_t cap;
   const uint64_t *counts;  // DEVICE array: valid records of every region (deposited by the senders)
-  unsigned long long *prefix_out;  // DEVICE array of n_seg + 1 entries (nullable): exclusive prefix of the counts
   uint64_t bound;  // keys the key array holds: a larger deposited total is reported (seg_total), not written
 };
 __global__ void __launch_bounds__(BT) k_build_keys_segments(const uint64_t *__restrict__ packed,
@@ -250,11 +181,7 @@ __global__ void __launch_bounds__(BT) k_build_keys_segments(const uint64_t *__re
       run += min(T.counts[r], T.cap);
     }
     s_prefix[T.n_seg] = run;
-    if (blockIdx.x == 0) {
-      sc->seg_total = run;  // the host learns the batch size with the sort width
-      if (T.prefix_out)
-        for (uint32_t r = 0; r <= T.n_seg; r++) T.prefix_out[r] = s_prefix[r];  // for RawSegments
-    }
+    if (blockIdx.x == 0) sc->seg_total = run;  // the host learns the batch size with the sort width
   }
   __syncthreads();
   uint32_t my_or = 0, my_bad = 0, my_vmax = 0, my_vinv = 0;
@@ -272,9 +199,9 @@ __global__ void __launch_bounds__(BT) k_build_keys_segments(const uint64_t *__re
     const uint32_t v = val ? val[at] : default_val;
     const bool ok = s < n && !(v != 0 && d == PPCSR_SENT);
     const uint64_t kq = emit_key(ok, k, v, n, op_bit);
-    if (keys) keys[i] = kq;  // nullptr: the sort reads the raw records itself (RawPacked / RawSegments)
+    keys[i] = kq;
     hist_add(s_h, H, kq);
-    if (pay && keys) pay[i] = ok ? v : 0u;
+    if (pay) pay[i] = ok ? v : 0u;
     if (ok) my_or |= d;
     else my_bad++;
     if (pay && ok && v) my_vmax = max(my_vmax, v), my_vinv = max(my_vinv, ~v);
@@ -456,13 +383,7 @@ constexpr int LCAP_LEAVES = LCAP / 8;  // leaves are >= 8 slots
 // memory and only the in-leaf half (one 128-byte line per update, shared by neighbouring keys) goes to global memory.
 // At C4's update density (one update per ~5 slots) a tile of 512 sorted updates spans ~2.7 K slots: too long to stage,
 // ~90 table entries.
-#ifndef PPCSR_LOC_TAB
-#define PPCSR_LOC_TAB 1
-#endif
-#ifndef PPCSR_LOC_FAST1  // find_fast for whole-staged windows too
-#define PPCSR_LOC_FAST1 0
-#endif
-constexpr int LTAB = PPCSR_LOC_TAB ? 1536 : 0;  // leaves a tile can stage as a table (in the place of dest[])
+constexpr int LTAB = 1536;  // leaves a tile can stage as a table (in the place of dest[])
 struct LocTable {
   uint32_t first[LTAB + 1];
   uint8_t cnt8[LTAB + 1];
@@ -483,17 +404,15 @@ struct LocSmem {
 };
 static_assert(sizeof(LocSmem) <= 48 * 1024, "k_locate is launched without a shared-memory opt-in");
 
-// The search of a staged tile without empty leaves, with UNIFORM trip counts: a warp's lanes search vertex ranges of
-// different lengths, so the data-dependent loops of find_in / find_tab run for the longest range in the warp at ~12
-// instructions per step, diverged (ncu: 47 % of k_locate's instructions, which is issue-bound).  Here the leaf level
-// takes `steps` = ceil(log2(leaves of the window)) branch-free halvings and the in-leaf lower_bound five (a leaf has
-// <= 32 slots).  TAB: the window is staged as a leaf table (the in-leaf half reads global memory), else whole.
-// Same result as find_in / find_tab when no leaf of the window is empty.
-template <bool TAB>
+// The search of a tile staged as a leaf table without empty leaves, with UNIFORM trip counts: a warp's lanes search
+// vertex ranges of different lengths, so the data-dependent loops of find_tab run for the longest range in the warp at
+// ~12 instructions per step, diverged (ncu: 47 % of k_locate's instructions, which is issue-bound).  Here the leaf level
+// takes `steps` = ceil(log2(leaves of the window)) branch-free halvings in the table and the in-leaf lower_bound five in
+// global memory (a leaf has <= 32 slots).  Same result as find_tab when no leaf of the window is empty.
 __device__ __forceinline__ bool find_fast(const LocSmem &S, const uint32_t *__restrict__ dest, uint32_t wa,
                                           uint32_t steps, uint32_t b, uint32_t e, uint32_t ls, uint32_t d,
                                           uint32_t *slot) {
-  const uint32_t l0 = wa >> ls, fs = TAB ? 0u : ls;
+  const uint32_t l0 = wa >> ls;
   const uint32_t Lb = b >> ls, Le = (e - 1) >> ls;
   uint32_t lo = Lb - l0, n = Le - Lb + 1u;  // candidates: the window's leaves [lo, lo + n)
   // as many halvings as the longest range among the lanes searching right now needs (most vertices span one or two
@@ -501,16 +420,16 @@ __device__ __forceinline__ bool find_fast(const LocSmem &S, const uint32_t *__re
   steps = min(steps, 32u - (uint32_t)__clz(__reduce_max_sync(__activemask(), n)));
   for (uint32_t st = 0; st < steps; st++) {
     const uint32_t half = n >> 1;
-    // unconditional probe (branch-free): half == 0 re-reads [lo] and adds nothing.  S.tab.first aliases S.dest
-    lo += S.dest[(lo + half) << fs] <= d ? half : 0u;
+    // unconditional probe (branch-free): half == 0 re-reads [lo] and adds nothing
+    lo += S.tab.first[lo + half] <= d ? half : 0u;
     n -= half;
   }
   const uint32_t leaf = lo + l0, base = leaf << ls;
-  const uint32_t cnt = TAB ? (uint32_t)S.tab.cnt8[lo] : S.cnt[lo];
+  const uint32_t cnt = S.tab.cnt8[lo];
   const uint32_t f_lo = (leaf == Lb) ? (b - base) + 1u : 0u;
   uint32_t f_hi = cnt;
   if (leaf == (e >> ls) && (e - base) < f_hi) f_hi = e - base;
-  const uint32_t *L = TAB ? dest + base : S.dest + (base - wa);
+  const uint32_t *L = dest + base;
   uint32_t x = f_lo, m = f_hi > f_lo ? f_hi - f_lo : 0u;  // lower_bound of d in [f_lo, f_hi): the answer lies in [x, x + m]
 #pragma unroll
   for (int st = 0; st < 5; st++) {
@@ -670,16 +589,9 @@ __global__ void __launch_bounds__(LT, 8) k_locate(const uint64_t *__restrict__ k
           const uint32_t d = (uint32_t)k;
           uint32_t slot;
           bool hit;
-#if PPCSR_LOC_FAST1
-          if (fast) {
-            hit = mode == 3u ? find_fast<true>(S, dest, wa, steps, vb[r], ve[r], ls, d, &slot)
-                             : find_fast<false>(S, dest, wa, steps, vb[r], ve[r], ls, d, &slot);
-          } else {
-#else
           if (fast && mode == 3u) {  // (whole-staged windows: measured 4 % slower than find_in's short loops, C2)
-            hit = find_fast<true>(S, dest, wa, steps, vb[r], ve[r], ls, d, &slot);
+            hit = find_fast(S, dest, wa, steps, vb[r], ve[r], ls, d, &slot);
           } else {
-#endif
             hit = mode == 3u ? find_tab(S.tab.first, S.tab.cnt8, wa >> ls, dest, vb[r], ve[r], ls, d, &slot)
                              : find_in(D, doff, C, coff, vb[r], ve[r], true, ls, d, &slot);
           }

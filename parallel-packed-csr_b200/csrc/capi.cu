@@ -117,52 +117,11 @@ int alloc_geometry(ppcsr_shard *s, const Geometry &g) {
   return PPCSR_OK;
 }
 
-// development knob: PPCSR_REB_PAD_SMEM=<bytes> of unused dynamic shared memory caps the resident CTAs per SM of
-// k_rebalance (occupancy experiments); unset in production
-// the knobs below are read once; function-local statics with an initialiser are thread-safe (PPPCSR drives its shards
-// from several host threads)
-uint32_t reb_prefetch_dist() {  // development knob: PPCSR_REB_PREFETCH=<chunks>, default one wave of resident CTAs
-  static const long d = [] {
-    const char *e = getenv("PPCSR_REB_PREFETCH");
-    return e ? atol(e) : 148L * 4;
-  }();
-  return (uint32_t)d;
-}
-size_t reb_pad_smem() {
-  static const long pad = [] {
-    const char *e = getenv("PPCSR_REB_PAD_SMEM");
-    const long p = e ? atol(e) : 0;
-#if PPCSR_HAVE_V6
-    if (p > 0) cudaFuncSetAttribute(reb::k_rebalance, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)p);
-#endif
-    return p;
-  }();
-  return (size_t)pad;
-}
-
-// The default is the rank-dense persistent kernel (k_rebalance_m, rebalance_m.cuh).  PPCSR_REB_KERNEL=9 selects the
-// slot-dealt persistent kernel of round 1 (k_rebalance_p), =6 the one-chunk-per-CTA kernel (k_rebalance), for A/B runs.
-int reb_kernel() {
-  static const int k = [] {
-    const char *e = getenv("PPCSR_REB_KERNEL");
-    return e ? atoi(e) : 10;
-  }();
-  return k;
-}
-bool reb_kernel_m() { return reb_kernel() != 6 && reb_kernel() != 9; }
-// plan entries are 32 bytes (ChunkPlan) or 64 (ChunkPlanM): the buffer is kept in units of ChunkPlan
-int reserve_plan(ppcsr_shard *s, size_t n_chunks) {
-  return dev_reserve(s->plan, reb_kernel_m() ? 2 * n_chunks : n_chunks, s->stream);
-}
+int reserve_plan(ppcsr_shard *s, size_t n_chunks) { return dev_reserve(s->plan, n_chunks, s->stream); }
 void launch_plan(ppcsr_shard *s, const WindowDesc *windows, uint32_t n_windows, uint32_t ls_src, uint32_t ls_dst,
                  uint32_t m_dst_override, uint32_t n_chunks, uint32_t CL) {
-  if (reb_kernel_m())
-    reb::k_plan_chunks_m<<<div_up(n_chunks, reb::RT), reb::RT, 0, s->stream>>>(
-        windows, n_windows, s->rank_off.p, s->ins_off.p, ls_src, ls_dst, m_dst_override, n_chunks, CL,
-        reinterpret_cast<reb::ChunkPlanM *>(s->plan.p));
-  else
-    reb::k_plan_chunks<<<div_up(n_chunks, reb::RT), reb::RT, 0, s->stream>>>(
-        windows, n_windows, s->rank_off.p, s->ins_off.p, ls_src, ls_dst, m_dst_override, n_chunks, CL, s->plan.p);
+  reb::k_plan_chunks_m<<<div_up(n_chunks, reb::RT), reb::RT, 0, s->stream>>>(
+      windows, n_windows, s->rank_off.p, s->ins_off.p, ls_src, ls_dst, m_dst_override, n_chunks, CL, s->plan.p);
 }
 template <bool TOMB, bool UNIV>
 int launch_rebalance_m(ppcsr_shard *s, unsigned n_chunks, const reb::Args &A) {
@@ -182,8 +141,8 @@ int launch_rebalance_m(ppcsr_shard *s, unsigned n_chunks, const reb::Args &A) {
     return e ? atol(e) : (long)PPCSR_M_CTAS;
   }();
   const unsigned grid = std::min<unsigned>(n_chunks, (unsigned)(sms[dv] * ctas));
-  reb::k_rebalance_m<TOMB, UNIV><<<grid, reb::MTT, sizeof(reb::MSmem<TOMB, UNIV>), s->stream>>>(
-      A, reinterpret_cast<const reb::ChunkPlanM *>(s->plan.p), n_chunks);
+  reb::k_rebalance_m<TOMB, UNIV><<<grid, reb::MTT, sizeof(reb::MSmem<TOMB, UNIV>), s->stream>>>(A, s->plan.p,
+                                                                                                 n_chunks);
 #ifdef PPCSR_M_TRACE
   if (const char *path = getenv("PPCSR_TRACE_OUT")) {  // development build: clock stamps of the launch just made
     static uint32_t host_trace[4 * 64 * 9 * 8];
@@ -199,40 +158,9 @@ int launch_rebalance_m(ppcsr_shard *s, unsigned n_chunks, const reb::Args &A) {
 }
 // tomb: the batch wrote tombstones (it deleted edges); without, the leaves are still left-packed
 int launch_rebalance(ppcsr_shard *s, unsigned n_chunks, const reb::Args &A, bool tomb) {
-  if (reb_kernel_m()) {
-    if (A.ins_val == nullptr)
-      return tomb ? launch_rebalance_m<true, true>(s, n_chunks, A) : launch_rebalance_m<false, true>(s, n_chunks, A);
-    return tomb ? launch_rebalance_m<true, false>(s, n_chunks, A) : launch_rebalance_m<false, false>(s, n_chunks, A);
-  }
-  if (reb_kernel() == 6) {
-#if PPCSR_HAVE_V6
-    reb::k_rebalance<<<n_chunks, reb::KT, reb_pad_smem(), s->stream>>>(A);
-    return PPCSR_OK;
-#else
-    g_ppcsr_error = "this build has no one-chunk-per-CTA kernel";
-    return PPCSR_ERR_ARG;
-#endif
-  }
-  // per device, once, and thread-safe: PPPCSR drives its shards from several host threads
-  static std::once_flag once[64];
-  static int sms[64] = {0};
-  static cudaError_t once_err[64];
-  const int dv = s->device & 63;
-  std::call_once(once[dv], [&] {
-    once_err[dv] = cudaDeviceGetAttribute(&sms[dv], cudaDevAttrMultiProcessorCount, s->device);
-    if (once_err[dv] == cudaSuccess)
-      once_err[dv] = cudaFuncSetAttribute(reb::k_rebalance_p, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          (int)sizeof(reb::PSmem));
-  });
-  CUDA_TRY(once_err[dv]);
-  const int n_sm = sms[dv];
-  static const long ctas = [] {  // development knob: resident CTAs per SM the grid is sized for
-    const char *e = getenv("PPCSR_REB_GRID_CTAS");
-    return e ? atol(e) : (long)PPCSR_REB_CTAS;
-  }();
-  const unsigned grid = std::min<unsigned>(n_chunks, (unsigned)(n_sm * ctas));
-  reb::k_rebalance_p<<<grid, reb::KT, sizeof(reb::PSmem), s->stream>>>(A, n_chunks);
-  return PPCSR_OK;
+  if (A.ins_val == nullptr)
+    return tomb ? launch_rebalance_m<true, true>(s, n_chunks, A) : launch_rebalance_m<false, true>(s, n_chunks, A);
+  return tomb ? launch_rebalance_m<true, false>(s, n_chunks, A) : launch_rebalance_m<false, false>(s, n_chunks, A);
 }
 
 // Output leaves per chunk of a whole-array rebuild.  A chunk's source range is its share of the source leaves plus
@@ -355,7 +283,6 @@ int rebuild_whole_array(ppcsr_shard *s, uint64_t new_N, uint64_t items_new, cons
   reb::Args A{};
   A.src_dest = s->dest.p;
   A.src_val = s->val.p;
-  A.leaf_cnt = s->leaf_cnt.p;
   A.rank_off = s->rank_off.p;
   A.ins_off = s->ins_off.p;
   A.ins_dst = s->ins_dst.p;
@@ -365,22 +292,18 @@ int rebuild_whole_array(ppcsr_shard *s, uint64_t new_N, uint64_t items_new, cons
   A.out_dest_single = A.out_dest_multi = s->dest_alt.p;
   A.out_val_single = A.out_val_multi = s->val_alt.p;
   A.tree_leaf_out = s->tree.p + g2.n_leaves;
-  // the persistent kernel reads no leaf counts (kept flags come from val[]), so the new counts can go straight into
-  // leaf_cnt[]; sized for the new geometry before the launch (old contents are not needed any more)
+  // the kernel reads no leaf counts (kept flags come from val[]), so the new counts can go straight into leaf_cnt[];
+  // sized for the new geometry before the launch (old contents are not needed any more)
   PPCSR_TRY(dev_reserve(s->leaf_cnt, g2.n_leaves, s->stream));
-  A.leaf_cnt = s->leaf_cnt.p;
-  A.leaf_cnt_out = reb_kernel() == 6 ? nullptr : s->leaf_cnt.p;
+  A.leaf_cnt = A.leaf_cnt_out = s->leaf_cnt.p;
   A.beg = s->beg.p;
   A.windows = s->windows.p;
   A.n_windows = 1;
   A.ls_src = g.leaf_shift;
   A.ls_dst = g2.leaf_shift;
   A.m_dst_override = g2.n_leaves;
-  A.prefetch_dist = reb_prefetch_dist();
-  A.chunk_leaves = CL2;
   A.ins_sentinels = s->ins_sentinels ? 1u : 0u;
   PPCSR_TRY(reserve_plan(s, (size_t)hw->n_chunks));
-  A.plan = s->plan.p;
   launch_plan(s, s->windows.p, 1u, g.leaf_shift, g2.leaf_shift, g2.n_leaves, hw->n_chunks, CL2);
   s->launches += 4;
   CUDA_TRY(cudaEventRecord(s->ev[5], s->stream));
@@ -392,9 +315,6 @@ int rebuild_whole_array(ppcsr_shard *s, uint64_t new_N, uint64_t items_new, cons
   s->geo = g2;
   s->cnt_clean = false;
   PPCSR_TRY(reserve_leaf_arrays(s, g2));
-  if (!A.leaf_cnt_out)  // the one-chunk-per-CTA kernel leaves the counts in the tree only
-    reb::k_copy_u32<<<div_up(g2.n_leaves, 256), 256, 0, s->stream>>>(s->leaf_cnt.p, s->tree.p + g2.n_leaves,
-                                                                    g2.n_leaves);
   PPCSR_TRY(win::tree_rebuild(s, s->tree.p, g2.H));
   reb::k_set_u32<<<1, 1, 0, s->stream>>>(s->beg.p + s->n, (uint32_t)g2.N);
   // every leaf was rewritten: for the invariant checker all of them count as touched by this batch (a flag, not two
@@ -461,7 +381,7 @@ int finish_batch_impl(ppcsr_shard *s, size_t list_cap, ppcsr_batch_stats *st) {
   // window selection + rebalance stages together): the window path costs ~150 us of launches and host round trip,
   // ~0.012 us per 1000 leaves (its O(leaves) passes: post-batch counts, tree, touched list, the two offset scans)
   // and ~1.05 us per 1000 touched leaves (path walks, window list, one warp per window): 0.19 / 0.23 / 0.40 ms at
-  // 10 K / 72 K / 224 K windows.  Streaming the whole array through k_rebalance_p costs ~105 us (scans, plan, tree
+  // 10 K / 72 K / 224 K windows.  Streaming the whole array through the rebalance costs ~105 us (scans, plan, tree
   // of the new array) + 16 bytes per slot at ~3.8 TB/s: 0.25 ms at 2^25 slots.  So at scale 20 the root window wins
   // from ~80 K touched leaves on (8 % of them), at scale 24 from ~1.9 M (11 %); the earlier fixed rule (a quarter
   // of the leaves) left a 1 M-update batch on the window path (0.61 ms instead of 0.47 ms).
@@ -560,8 +480,6 @@ int finish_batch_impl(ppcsr_shard *s, size_t list_cap, ppcsr_batch_stats *st) {
     A.n_windows = (uint32_t)h.n_windows;
     A.ls_src = A.ls_dst = g.leaf_shift;
     A.m_dst_override = 0;
-    A.prefetch_dist = reb_prefetch_dist();
-    A.chunk_leaves = CL;
     A.ins_sentinels = s->ins_sentinels ? 1u : 0u;
     CUDA_TRY(cudaEventRecord(s->ev[5], s->stream));
     if (h.n_small) {
@@ -586,21 +504,14 @@ int finish_batch_impl(ppcsr_shard *s, size_t list_cap, ppcsr_batch_stats *st) {
     }
     if (h.n_chunks) {
       PPCSR_TRY(reserve_plan(s, (size_t)h.n_chunks));
-      A.plan = s->plan.p;
       launch_plan(s, s->windows.p, (uint32_t)h.n_windows, g.leaf_shift, g.leaf_shift, 0, (uint32_t)h.n_chunks, CL);
       s->launches += 2 + (h.multi_slots ? 1 : 0);
       PPCSR_TRY(launch_rebalance(s, (unsigned)h.n_chunks, A, h.n_deleted != 0));
     }
     CUDA_TRY(cudaEventRecord(s->ev[6], s->stream));
-    if (h.multi_slots) {
-      if (reb_kernel_m())
-        reb::k_copy_back_m<<<(unsigned)h.n_chunks, reb::RT, 0, s->stream>>>(
-            reinterpret_cast<const reb::ChunkPlanM *>(s->plan.p), g.leaf_shift, s->dest_alt.p, s->val_alt.p, s->dest.p,
-            s->val.p);
-      else
-        reb::k_copy_back<<<(unsigned)h.n_chunks, reb::RT, 0, s->stream>>>(s->plan.p, g.leaf_shift, s->dest_alt.p,
+    if (h.multi_slots)
+      reb::k_copy_back_m<<<(unsigned)h.n_chunks, reb::RT, 0, s->stream>>>(s->plan.p, g.leaf_shift, s->dest_alt.p,
                                                                           s->val_alt.p, s->dest.p, s->val.p);
-    }
     s->launches += 1;
     reb::k_copy_u32<<<div_up(L, 256), 256, 0, s->stream>>>(s->leaf_cnt.p, s->tree.p + L, L);
     PPCSR_TRY(win::tree_rebuild(s, s->tree.p, g.H));
@@ -668,21 +579,14 @@ __global__ void k_fill_new_nodes(uint32_t *ins_dst, uint32_t *ins_val, uint32_t 
   }
 }
 
-// One PageRank push step over the whole shard.  Default: the leaf walk (k_pagerank_push_leaves, a coalesced stream
-// over the packed array); PPCSR_PR_KERNEL=vertex selects the warp-per-vertex kernel (A/B).
+// One PageRank push step over the whole shard: the leaf walk (k_pagerank_push_leaves, a coalesced stream over the
+// packed array).
 template <typename W>
 static void launch_pagerank_push(ppcsr_shard *s, const W *d_in, double *d_acc, uint64_t out_len) {
-  static const bool per_vertex = getenv("PPCSR_PR_KERNEL") && std::string(getenv("PPCSR_PR_KERNEL")) == "vertex";
-  if (per_vertex) {
-    const unsigned blocks = std::min<unsigned>(div_up((uint64_t)s->n * 32, qry::QT), 148 * 16);
-    qry::k_pagerank_push<W><<<blocks, qry::QT, 0, s->stream>>>(s->dest.p, s->leaf_cnt.p, s->beg.p, s->nn.p,
-                                                              s->geo.leaf_shift, s->n, d_in, d_acc, out_len);
-  } else {
-    const unsigned blocks = std::min<unsigned>(div_up(s->geo.N, (uint64_t)qry::QT * qry::PRL_BATCH), 148 * 16);
-    qry::k_pagerank_push_leaves<W><<<blocks, qry::QT, 0, s->stream>>>(s->dest.p, s->val.p, s->leaf_cnt.p, s->beg.p,
-                                                                     s->nn.p, s->geo.leaf_shift, s->n, s->geo.N, d_in,
-                                                                     d_acc, out_len);
-  }
+  const unsigned blocks = std::min<unsigned>(div_up(s->geo.N, (uint64_t)qry::QT * qry::PRL_BATCH), 148 * 16);
+  qry::k_pagerank_push_leaves<W><<<blocks, qry::QT, 0, s->stream>>>(s->dest.p, s->val.p, s->leaf_cnt.p, s->beg.p,
+                                                                   s->nn.p, s->geo.leaf_shift, s->n, s->geo.N, d_in,
+                                                                   d_acc, out_len);
 }
 
 template <typename W>
@@ -901,7 +805,7 @@ void ppcsr_destroy(ppcsr_shard *s) {
   dev_free(s->uloc); dev_free(s->ucls); dev_free(s->ufirst); dev_free(s->ins_dst); dev_free(s->ins_val); dev_free(s->ins_pred);
   dev_free(s->block_tmp); dev_free(s->hist); dev_free(s->pr_acc); dev_free(s->misc);
   dev_free(s->scan_state); dev_free(s->scan_ticket); dev_free(s->tile_cnt);
-  dev_free(s->touch_stamp); dev_free(s->touched_flags); dev_free(s->seg_prefix);
+  dev_free(s->touch_stamp); dev_free(s->touched_flags);
   dev_free(s->snap.dest); dev_free(s->snap.val); dev_free(s->snap.leaf_cnt); dev_free(s->snap.tree);
   dev_free(s->snap.beg); dev_free(s->snap.nn);
   for (auto &P : s->pending) {
@@ -1031,22 +935,15 @@ static int apply_device_common(ppcsr_shard *s, const uint32_t *d_src, const uint
   H.ghist = nullptr;
   const bool fused_hist = count > prim::SS_MAX;  // (smaller batches are sorted by one CTA: no global histograms)
   if (fused_hist) PPCSR_TRY(prim::radix_sort_prepare(s, count, H.P, &H.ghist));
-  // The builder writes the batch out as an array of key words.  PPCSR_RAW_FIRST_PASS=1 (development knob) skips that:
-  // the first pass of the sort then builds the key words from the caller's arrays itself (batch::RawArrays / RawPacked /
-  // RawSegments).  Measured on B200: one write and one read of the batch less, but two 4-byte streams and the guards
-  // inside the instruction-bound sort pass cost more than they save -- sort stage 3.35 -> 3.69 ms on C4, 0.364 -> 0.403 ms
-  // on C2 -- so it is off by default.
-  static const bool raw_first_pass = getenv("PPCSR_RAW_FIRST_PASS") != nullptr;
-  const bool materialize = !raw_first_pass || (!segments && count <= prim::SS_MAX);
-  uint64_t *key_out = materialize ? s->key_a.p : nullptr;
-  const uint32_t src_default = default_val;  // (default_val may be replaced below when the values are all equal)
+  // The builder writes the batch out as an array of key words.  (Building the key words inside the sort's first pass
+  // instead, from the caller's arrays, saves one write and one read of the batch but measured slower on B200: two
+  // 4-byte streams and the guards inside the instruction-bound sort pass cost more than they save -- sort stage
+  // 3.35 -> 3.69 ms on C4, 0.364 -> 0.403 ms on C2.)
+  uint64_t *key_out = s->key_a.p;
   const unsigned kb = std::min<unsigned>(div_up(count, batch::BT * 8), 148 * (fused_hist ? 8 : 16));
   if (segments) {
-    PPCSR_TRY(dev_reserve(s->seg_prefix, (size_t)segments->n_seg + 2, s->stream));
-    batch::SegmentTable T = *segments;
-    T.prefix_out = s->seg_prefix.p;
-    batch::k_build_keys_segments<<<kb, batch::BT, 0, s->stream>>>(d_packed, d_val, default_val, T, s->n, op_bit, key_out,
-                                                                 has_pay ? s->pay_a.p : nullptr, sc, H);
+    batch::k_build_keys_segments<<<kb, batch::BT, 0, s->stream>>>(d_packed, d_val, default_val, *segments, s->n, op_bit,
+                                                                 key_out, has_pay ? s->pay_a.p : nullptr, sc, H);
   } else if (d_packed) {
     batch::k_build_keys_packed<<<kb, batch::BT, 0, s->stream>>>(d_packed, d_val, default_val, count, s->n, op_bit, key_out,
                                                                has_pay ? s->pay_a.p : nullptr, sc, pairs ? 1u : 0u, H);
@@ -1112,22 +1009,8 @@ static int apply_device_common(ppcsr_shard *s, const uint32_t *d_src, const uint
   // 2. stable radix sort by (src,dst)
   uint64_t *keys;
   uint32_t *pay;
-  if (materialize) {
-    PPCSR_TRY(prim::radix_sort_pairs(s, s->key_a.p, sort_pay ? s->pay_a.p : nullptr, s->key_b.p, s->pay_b.p, count,
-                                     lo_bits, hi_bits, &keys, &pay, hist_done));
-  } else if (segments) {
-    const batch::RawSegments R{d_packed, d_val, s->seg_prefix.p, segments->cap, segments->n_seg, src_default, s->n, op_bit};
-    PPCSR_TRY(prim::radix_sort_from(s, R, sort_pay, s->key_a.p, s->pay_a.p, s->key_b.p, s->pay_b.p, count, lo_bits,
-                                    hi_bits, &keys, &pay, hist_done));
-  } else if (d_packed) {
-    const batch::RawPacked R{d_packed, d_val, src_default, s->n, op_bit, pairs ? 1u : 0u};
-    PPCSR_TRY(prim::radix_sort_from(s, R, sort_pay, s->key_a.p, s->pay_a.p, s->key_b.p, s->pay_b.p, count, lo_bits,
-                                    hi_bits, &keys, &pay, hist_done));
-  } else {
-    const batch::RawArrays R{d_src, d_dst, d_val, src_default, s->n, op_bit};
-    PPCSR_TRY(prim::radix_sort_from(s, R, sort_pay, s->key_a.p, s->pay_a.p, s->key_b.p, s->pay_b.p, count, lo_bits,
-                                    hi_bits, &keys, &pay, hist_done));
-  }
+  PPCSR_TRY(prim::radix_sort_pairs(s, s->key_a.p, sort_pay ? s->pay_a.p : nullptr, s->key_b.p, s->pay_b.p, count,
+                                   lo_bits, hi_bits, &keys, &pay, hist_done));
   if (stage_ev) CUDA_TRY(cudaEventRecord(s->ev[1], s->stream));
   // 3+4. call counts, last-op-wins, locate, per-leaf counts -- one kernel over the sorted batch
   const uint64_t invalid_key = (uint64_t)s->n << 32;
@@ -1159,9 +1042,8 @@ static int apply_device_common(ppcsr_shard *s, const uint32_t *d_src, const uint
   PPCSR_TRY(dev_reserve(s->tile_cnt, (size_t)lblocks + 1, s->stream));
   // a batch of ONE tile needs no scan and no gather: the tile's run is the insert list
   // With no payload every insert of the batch carries default_val: the general path then neither writes nor reads a
-  // value list (k_rebalance_m / k_rebalance_small take the one value; the small-batch path and the round-1 kernels
-  // keep the list)
-  s->ins_uniform_val = (!pay && !sparse && reb_kernel_m()) ? default_val : 0u;
+  // value list (k_rebalance_m / k_rebalance_small take the one value; the small-batch path keeps the list)
+  s->ins_uniform_val = (!pay && !sparse) ? default_val : 0u;
   if (s->ins_uniform_val) tile_val = nullptr;
   uint32_t *t_dst = lblocks == 1 ? s->ins_dst.p : tile_dst;
   uint32_t *t_val = s->ins_uniform_val ? nullptr : lblocks == 1 ? s->ins_val.p : tile_val;
@@ -1626,9 +1508,8 @@ int ppcsr_bin_to_peers(int device, void *cuda_stream, const uint64_t *d_starts, 
   PPCSR_TRY(dev_reserve(tmp.hist, std::max<size_t>(hn + 1, batch::BIN_MAX_PARTS), st));
   // Without per-update values every update of the batch is the same operation and their order inside a destination's
   // region does not matter: the tiles then claim their places with one atomicAdd per destination (tmp.hist[0 .. parts) is
-  // the cursor) and the count pass + scan in front of the scatter go away (PPCSR_ROUTE_ORDERED=1 keeps them).
-  static const bool force_ordered = getenv("PPCSR_ROUTE_ORDERED") != nullptr;
-  const bool ordered = d_val != nullptr || force_ordered;
+  // the cursor) and the count pass + scan in front of the scatter go away.
+  const bool ordered = d_val != nullptr;
   if (ordered) {
     batch::k_bin_count<<<nblocks, batch::BT, 0, st>>>(d_src, count, d_starts, n_parts, tmp.hist.p, nblocks);
     PPCSR_TRY(prim::device_scan(&tmp, prim::InArray{tmp.hist.p}, prim::OutPrefixWithTotal{tmp.hist.p, hn}, hn, nullptr,

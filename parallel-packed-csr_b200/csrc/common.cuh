@@ -160,19 +160,9 @@ struct WindowDesc {
   uint32_t n_chunks;
 };
 
-// Where one rebalance CTA (one chunk of CHUNK_SLOTS output slots) finds its work: precomputed by
-// k_plan_chunks so that no CTA runs a serial binary search while 255 threads wait at a barrier.
-struct ChunkPlan {
-  uint32_t leaf0;    // first leaf of the chunk's window
-  uint32_t m_multi;  // source leaves in the window | bit 31: the window spans several chunks (written out of place)
-  uint32_t items;    // live items of the window after the batch
-  uint32_t o_lo;     // first output leaf of the chunk (relative to the window)
-  uint32_t i_lo;     // first source leaf (relative to the window) feeding the chunk's rank range
-  uint32_t i_hi;     // last source leaf; i_lo > i_hi means the chunk receives no items
-  uint32_t q_lo;     // inserts of the source leaves i_lo..i_hi that can rank inside the chunk: [q_lo, q_hi)
-  uint32_t q_hi;
-};
-static_assert(sizeof(ChunkPlan) == 32, "a rebalance CTA starts from one 32-byte plan entry");
+namespace reb {
+struct ChunkPlanM;  // one entry per chunk of the chunked rebalance (rebalance_m.cuh)
+}
 
 struct ppcsr_shard {
   int device = 0;
@@ -200,7 +190,7 @@ struct ppcsr_shard {
   DevBuf<uint32_t> touched_win;        // [n_leaves] window node of each touched leaf
   DevBuf<WindowDesc> windows;          // [n_leaves]
   DevBuf<uint32_t> win_chunk_off;      // [n_leaves+1]
-  DevBuf<ChunkPlan> plan;              // [n_chunks]
+  DevBuf<reb::ChunkPlanM> plan;        // [n_chunks]
   bool ins_sentinels = false;          // the pending insert list holds sentinels (ppcsr_add_nodes)
   uint32_t ins_uniform_val = 0;        // != 0: the pending insert list has no value array, every insert carries this
   uint32_t all_touched = 0;            // invariant checker: bit 2 = the last batch rewrote every leaf (bit 0 inserts, bit 1 deletes)
@@ -235,7 +225,6 @@ struct ppcsr_shard {
   DevBuf<uint32_t> uval;               // [batch]
   DevBuf<uint32_t> uloc;               // [batch, whole tiles] predecessor slots of the locate tiles' inserts
   DevBuf<uint32_t> tile_cnt;           // [tiles + 1] inserts per locate tile -> exclusive scan
-  DevBuf<unsigned long long> seg_prefix;  // [segments + 1] prefix of the peers' record counts (batch::RawSegments)
   DevBuf<uint8_t> ucls;                // [batch] class
   DevBuf<uint8_t> ufirst;              // [batch] first op of the key in this batch is a remove
   DevBuf<uint32_t> ins_dst, ins_val, ins_pred;  // [batch] compacted pure inserts, key order
@@ -253,14 +242,14 @@ struct ppcsr_shard {
   void *h_pinned = nullptr;            // pinned staging for small D2H/H2D
   size_t h_pinned_bytes = 0;
 
-  cudaEvent_t ev[8] = {};  // 0 start, 1 sorted, 2 located, 3 selected, 4 done, 5/6 around k_rebalance
+  cudaEvent_t ev[8] = {};  // 0 start, 1 sorted, 2 located, 3 selected, 4 done, 5/6 around the rebalance kernels
   ppcsr_batch_stats last{};
   Snapshot snap;
 };
 
 // Every device array comes from dev_reserve and ends with at least DEV_PAD_ELEMS elements beyond the requested count.
-// The bulk (TMA) loads of reb::k_rebalance_p round their length up to 16 bytes and may READ up to 3 elements past the
-// logical end of rank_off / ins_off / ins_pred / ins_dst / ins_val (rebalance.cuh: issue_round): the pad is what makes
+// The bulk (TMA) loads of reb::k_rebalance_m round their length up to 16 bytes and may READ up to 3 elements past the
+// logical end of rank_off / ins_off / ins_pred / ins_dst / ins_val (rebalance_m.cuh: issue_round): the pad is what makes
 // that legal, whatever size the caller asked for.
 constexpr size_t DEV_PAD_ELEMS = 64;
 static_assert(DEV_PAD_ELEMS >= 4, "the rebalance kernel's 16-byte bulk loads over-read by up to 3 elements");

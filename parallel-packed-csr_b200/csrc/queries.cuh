@@ -91,39 +91,16 @@ __global__ void __launch_bounds__(QT) k_touch(const uint32_t *__restrict__ dest,
   if (lane_id() == 0 && acc) atomicAdd(sum, acc);
 }
 
-// ---- PageRank push step: warp per vertex, fp64 accumulation -----------------------------------------
-// out[dst] += in[v] / num_neighbors[v] for every edge (v,dst)  (reference pagerank.h:19-26; the divisor
-// is the call-count num_neighbors, not the degree).  A vertex without live edges contributes nothing,
-// whatever its divisor.
-template <typename W>
-__global__ void __launch_bounds__(QT) k_pagerank_push(const uint32_t *__restrict__ dest,
-                                                      const uint32_t *__restrict__ leaf_cnt,
-                                                      const uint32_t *__restrict__ beg, const uint32_t *__restrict__ nn,
-                                                      uint32_t ls, uint32_t n, const W *__restrict__ in,
-                                                      double *__restrict__ acc, uint64_t out_len) {
-  const uint32_t warps = (gridDim.x * blockDim.x) >> 5;
-  const uint32_t lane = lane_id();
-  for (uint32_t v = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; v < n; v += warps) {
-    const uint32_t b = beg[v], e = beg[v + 1];
-    if (e - b <= 1) continue;
-    const W contrib = in[v] / (W)nn[v];
-    for (uint32_t slot = b + 1 + lane; slot < e; slot += 32) {
-      const uint32_t f = slot & ((1u << ls) - 1u);
-      if (f < leaf_cnt[slot >> ls]) {
-        const uint32_t d = dest[slot];
-        if (d < out_len) atomicAdd(&acc[d], (double)contrib);
-      }
-    }
-  }
-}
 // ---- PageRank push step, leaf walk: a warp streams a run of consecutive 32-slot groups ----------------------
-// The warp-per-vertex form above pays a dependent chain (beg[v], beg[v+1], in[v], nn[v]) per vertex and leaves most
-// lanes idle on an R-MAT graph (half of the vertices own at most a couple of edges).  The packed array itself
+// out[dst] += in[v] / num_neighbors[v] for every edge (v,dst)  (reference pagerank.h:19-26; the divisor is the
+// call-count num_neighbors, not the degree).  A vertex without live edges contributes nothing, whatever its divisor.
+// A warp per vertex would pay a dependent chain (beg[v], beg[v+1], in[v], nn[v]) per vertex and leave most lanes idle
+// on an R-MAT graph (half of the vertices own at most a couple of edges).  The packed array itself
 // carries everything a full scan needs, in order: a sentinel (dest == SENT, val == v + 1) opens vertex v's run, every
 // live slot after it is one of v's edges.  So: one coalesced 128-byte read of dest[] per group, the sentinels of the
 // group fetch their vertex's contribution, a ballot + shuffle hands every edge the contribution of the nearest
 // sentinel below it (or the one carried in from the previous group), and the warp finds the vertex of its first
-// slot with ONE binary search over beg[].  Same arithmetic as k_pagerank_push (contribution in W, accumulation fp64).
+// slot with ONE binary search over beg[].  The contribution is computed in W, the accumulation is fp64.
 constexpr int PRL_BATCH = 4;  // groups whose loads are issued together
 template <typename W>
 __global__ void __launch_bounds__(QT) k_pagerank_push_leaves(const uint32_t *__restrict__ dest,

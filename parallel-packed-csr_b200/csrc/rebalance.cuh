@@ -1,25 +1,20 @@
-// rebalance.cuh -- the rebalance kernel: merge the kept items of a window with the batch's inserts,
-// drop the tombstones, and spread the result evenly over the window's leaves, fixing the vertex
-// sentinels' back pointers in the same pass.
+// rebalance.cuh -- what the rebalance kernels share, and the small-window kernel.
+// A rebalance merges the kept items of a window with the batch's inserts, drops the tombstones, and spreads the result
+// evenly over the window's leaves, fixing the vertex sentinels' back pointers in the same pass.
 // Replaces reference PCSR::redistribute + fix_sentinel + slide_right/slide_left + double_list/half_list
 // (src/pcsr/PCSR.cpp:222-249, 168-183, 326-390, 251-320).
 //
-// Formulation (gather, output-driven).  For a window of m source leaves the merged sequence is the
-// concatenation over source leaves i of merge(kept(i), inserts(i)); its ranks are
+// Rank arithmetic.  For a window of m source leaves the merged sequence is the concatenation over source leaves i of
+// merge(kept(i), inserts(i)); its ranks are
 //     rank(kept item at offset f of leaf i) = R[i] + #kept before f + #inserts of i whose predecessor < f
 //     rank(q-th insert of leaf i)           = R[i] + q + #kept items of i at offsets <= offset(pred)
 // with R = exclusive scan of the post-batch leaf counts.  Output leaf o of m_out (a power of two: windows are
 // nodes of the implicit tree) receives the ranks [(o*j) >> lg(m_out), ((o+1)*j) >> lg(m_out)) left-packed,
 // the rest of the leaf is nulled.
 //
-// Work decomposition: a CTA owns CHUNK_SLOTS consecutive output slots (its source-leaf range comes from
-// k_plan_chunks), and inside it every WARP owns SUB_SLOTS = 256 of them and runs on its own -- no block
-// barrier on the data path, so the resident warps of an SM each keep a tile of 16 independent 128-B
-// loads in flight.  A warp locates its source leaves in the CTA's slice of R (shared memory), computes the
-// rank of every kept item and insert with ballots / popcounts, scatters them into its 2 KB staging buffer
-// ALREADY IN THE FINAL LAYOUT (leaf-packed, null tails), and hands the buffer to the TMA engine: two 1-KB
-// bulk stores (cp.async.bulk shared -> global) write dest[] and val[].
-// Algorithmic traffic: every window slot is read once and written once.
+// Here: the arguments of the chunked kernel (k_rebalance_m, rebalance_m.cuh) and the searches, bulk-copy (TMA) and
+// mbarrier helpers it uses; k_rebalance_small, which takes the windows of <= SMALL_MAX_LEAVES leaves one warp each; and
+// the kernels that lay out a fresh array.
 #pragma once
 #include "common.cuh"
 #include "primitives.cuh"
@@ -31,15 +26,16 @@ constexpr int RWARPS = RT / 32;
 #ifndef PPCSR_CHUNK_SLOTS
 #define PPCSR_CHUNK_SLOTS 2048
 #endif
-#ifndef PPCSR_REB_THREADS
-#define PPCSR_REB_THREADS 256
-#endif
 #ifndef PPCSR_SEG_SLOTS
 #define PPCSR_SEG_SLOTS 2048
 #endif
-constexpr int KT = PPCSR_REB_THREADS;  // threads of a k_rebalance CTA
-constexpr int CHUNK_SLOTS = PPCSR_CHUNK_SLOTS;               // output slots per CTA
+constexpr int CHUNK_SLOTS = PPCSR_CHUNK_SLOTS;     // output slots per chunk
+constexpr int SEG_LEAVES_SLOTS = PPCSR_SEG_SLOTS;  // source slots examined per segment (64 leaves of 32 slots): 2 quads per thread
+// leaves per segment: 64 of 32 slots; arrays with smaller leaves are tiny, their segments are capped at 128 leaves
+constexpr int SEG_MAX_LEAVES = SEG_LEAVES_SLOTS / 32 > 128 ? SEG_LEAVES_SLOTS / 32 : 128;
 
+// k_rebalance_m reads neither leaf_cnt, windows, n_windows nor ins_sentinels.  They stay for now: without them the other
+// parameters move, and ptxas allocates the kernel's registers differently.
 struct Args {
   const uint32_t *src_dest, *src_val;  // source slots
   const uint32_t *leaf_cnt;            // source physical leaf counts (tombstones included)
@@ -49,19 +45,15 @@ struct Args {
   uint32_t *out_dest_single, *out_val_single;  // target of single-CTA windows (in place)
   uint32_t *out_dest_multi, *out_val_multi;    // target of multi-CTA windows (out of place)
   uint32_t *tree_leaf_out;                     // post-rebalance leaf counts (leaf level of the tree)
-  uint32_t *leaf_cnt_out;                      // nullable: the same counts, straight into the new leaf_cnt[] (k_rebalance_p)
+  uint32_t *leaf_cnt_out;                      // nullable: the same counts, straight into the new leaf_cnt[]
   uint32_t *beg;
   const WindowDesc *windows;
   uint32_t n_windows;
   uint32_t ls_src, ls_dst;
   uint32_t m_dst_override;  // != 0: resize, the single window maps onto this many output leaves from leaf 0
-  const ChunkPlan *plan;    // one entry per CTA
-  uint32_t prefetch_dist;   // L2 prefetch distance in chunks (0 = off)
-  uint32_t chunk_leaves;    // output leaves per chunk (<= CHUNK_SLOTS >> ls_dst; not necessarily a power of two)
   uint32_t ins_sentinels;   // != 0: the insert list itself holds sentinels (add_nodes)
-  uint32_t ins_uniform;     // k_rebalance_m, ins_val == nullptr: the value every insert of the batch carries
+  uint32_t ins_uniform;     // ins_val == nullptr: the value every insert of the batch carries
 };
-
 
 __device__ __forceinline__ uint32_t upper_bound_u32(const uint32_t *a, uint32_t n, uint32_t key) {
   uint32_t lo = 0, hi = n;  // first index with a[idx] > key
@@ -87,55 +79,6 @@ __device__ __forceinline__ uint32_t leaf_rank0(uint32_t o, uint32_t j, uint32_t 
   return (uint32_t)(((uint64_t)o * j) >> lg);
 }
 
-// One thread per chunk: the window the chunk belongs to, copied into the plan entry so that the rebalance CTA
-// starts from ONE 32-byte load; the source leaves that feed the chunk's rank range [a, b); and the part of their
-// insert run that can rank inside it.  An insert q of leaf i ranks at R[i] + (q - ins_off[i]) + (kept items up to
-// its predecessor, <= one leaf), so the inserts of the FIRST leaf before ins_off + (a - R - leaf) rank below a and
-// those of the LAST leaf from ins_off + (b - R) on rank at or above b: a hub run spanning thousands of chunks is
-// clipped to <= span + leaf inserts per chunk without any search.
-__global__ void __launch_bounds__(RT) k_plan_chunks(const WindowDesc *__restrict__ windows, uint32_t n_windows,
-                                                    const uint32_t *__restrict__ rank_off,
-                                                    const uint32_t *__restrict__ ins_off, uint32_t ls_src,
-                                                    uint32_t ls_dst, uint32_t m_dst_override, uint32_t n_chunks,
-                                                    uint32_t CL, ChunkPlan *__restrict__ plan) {
-  const uint32_t chunk = blockIdx.x * blockDim.x + threadIdx.x;
-  if (chunk >= n_chunks) return;
-  uint32_t lo = 0, hi = n_windows;  // last window with chunk0 <= chunk
-  while (hi - lo > 1) {
-    const uint32_t mid = (lo + hi) >> 1;
-    if (windows[mid].chunk0 <= chunk) lo = mid;
-    else hi = mid;
-  }
-  const WindowDesc w = windows[lo];
-  const uint32_t m_dst = m_dst_override ? m_dst_override : w.m;
-  const uint32_t lg = 31u - (uint32_t)__clz(m_dst);
-  const uint32_t o_lo = (chunk - w.chunk0) * CL;  // CL output leaves per chunk
-  const uint32_t o_hi = min(o_lo + CL, m_dst);
-  const uint32_t a = leaf_rank0(o_lo, w.items, lg);
-  const uint32_t b = leaf_rank0(o_hi, w.items, lg);
-  const uint32_t *R = rank_off + w.leaf0;
-  const uint32_t *IO = ins_off + w.leaf0;
-  const uint32_t R0 = R[0];
-  ChunkPlan p;
-  p.leaf0 = w.leaf0;
-  p.m_multi = w.m | (w.n_chunks > 1 ? 0x80000000u : 0u);
-  p.items = w.items;
-  p.o_lo = o_lo;
-  if (b > a) {
-    p.i_lo = upper_bound_u32(R, w.m, R0 + a) - 1;      // source leaf holding rank a
-    p.i_hi = upper_bound_u32(R, w.m, R0 + b - 1) - 1;  // source leaf holding rank b-1
-    const uint32_t below = a - (R[p.i_lo] - R0);        // ranks of the first leaf below the chunk
-    const uint32_t leaf = 1u << ls_src;
-    p.q_lo = min(IO[p.i_lo] + (below > leaf ? below - leaf : 0u), IO[p.i_lo + 1]);
-    p.q_hi = max(p.q_lo, min(IO[p.i_hi] + (b - (R[p.i_hi] - R0)), IO[p.i_hi + 1]));
-  } else {
-    p.i_lo = 1;
-    p.i_hi = 0;
-    p.q_lo = p.q_hi = 0;
-  }
-  plan[chunk] = p;
-}
-
 // ---- TMA (bulk async copy) helpers: sm_90+/sm_100a PTX -----------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
 // generic-proxy writes to shared memory become visible to the async proxy (the TMA engine)
@@ -153,16 +96,6 @@ __device__ __forceinline__ void bulk_prefetch_l2(const void *src_gmem, uint32_t 
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 
-#ifndef PPCSR_REB_CTAS
-#define PPCSR_REB_CTAS 4
-#endif
-#ifndef PPCSR_TMA_STORE
-#define PPCSR_TMA_STORE 1
-#endif
-constexpr int SEG_LEAVES_SLOTS = PPCSR_SEG_SLOTS;  // source slots examined per segment (64 leaves of 32 slots): 2 quads per thread
-constexpr int QPT = SEG_LEAVES_SLOTS / 4 / KT;  // 16-byte quads per thread and segment
-constexpr int INS_PREFETCH = 2;                 // inserts per thread whose loads are issued together with the quads
-
 // inclusive scan of x over runs of `lpl` consecutive lanes (lpl = 2, 4 or 8: the lanes holding one source leaf)
 __device__ __forceinline__ uint32_t leaf_incl_scan(uint32_t x, unsigned lane, uint32_t lpl) {
   const uint32_t in_leaf = lane & (lpl - 1u);
@@ -173,267 +106,6 @@ __device__ __forceinline__ uint32_t leaf_incl_scan(uint32_t x, unsigned lane, ui
   }
   return x;
 }
-
-// One CTA per chunk of CHUNK_SLOTS output slots.  Per segment of <= 2048 source slots:
-//   P1  every thread loads its 16-byte quads of dest[]/val[] (and, in flight with them, its first inserts),
-//       counts the kept items of each leaf with a segmented warp scan            -> s_kupto
-//   P2  the segment's inserts, spread evenly over the CTA: rank, hang marker, placed -> s_last, staging
-//   P3  the kept items (still in registers): rank from s_last's running maximum, placed -> staging
-// then ONE bulk store (TMA) per array writes the chunk.
-#define PPCSR_HAVE_V6 (PPCSR_CHUNK_SLOTS <= 2048 && PPCSR_SEG_SLOTS <= 2048)
-#if PPCSR_HAVE_V6
-__global__ void __launch_bounds__(KT, PPCSR_REB_CTAS) k_rebalance(Args A) {
-  __shared__ __align__(128) uint32_t s_dest[CHUNK_SLOTS];  // the chunk's output slots in their final layout
-  __shared__ __align__(128) uint32_t s_val[CHUNK_SLOTS];
-  __shared__ uint16_t s_pos[CHUNK_SLOTS];                   // chunk-relative rank -> output slot
-  __shared__ uint32_t s_a[CHUNK_SLOTS / 8 + 8];             // first rank of every output leaf of the chunk (+ end)
-  __shared__ uint32_t s_R[SEG_LEAVES_SLOTS / 8 + 1], s_ioff[SEG_LEAVES_SLOTS / 8 + 1];
-  __shared__ __align__(16) uint32_t s_last[SEG_LEAVES_SLOTS];  // 1 + index of the last insert hanging on a slot
-  __shared__ __align__(16) uint8_t s_kupto[SEG_LEAVES_SLOTS];  // kept items of the leaf up to and including a slot
-
-  const ChunkPlan plan = A.plan[blockIdx.x];
-  // CTAs start in grid order, so the chunk `prefetch_dist` places ahead is picked up about one wave of resident
-  // CTAs from now: pull its source leaves and insert run into L2 so that its loads do not pay DRAM latency.
-  if (threadIdx.x == 0 && A.prefetch_dist && blockIdx.x + A.prefetch_dist < gridDim.x) {
-    const ChunkPlan nx = A.plan[blockIdx.x + A.prefetch_dist];
-    if (nx.i_lo <= nx.i_hi) {
-      const size_t slot0 = (size_t)(nx.leaf0 + nx.i_lo) << A.ls_src;
-      const uint32_t bytes = min(((nx.i_hi - nx.i_lo + 1u) << A.ls_src) * 4u, 16384u);
-      bulk_prefetch_l2(A.src_dest + slot0, bytes);
-      bulk_prefetch_l2(A.src_val + slot0, bytes);
-      if (nx.q_hi > nx.q_lo) {
-        const uint32_t qa = nx.q_lo & ~3u;
-        const uint32_t ib = min((((nx.q_hi - qa) + 3u) & ~3u) * 4u, 8192u);
-        bulk_prefetch_l2(A.ins_pred + qa, ib);
-        bulk_prefetch_l2(A.ins_dst + qa, ib);
-        bulk_prefetch_l2(A.ins_val + qa, ib);
-      }
-    }
-  }
-  const unsigned lane = lane_id(), lt = lanemask_lt();
-  const uint32_t ls_src = A.ls_src, ls_dst = A.ls_dst;
-  const uint32_t m_src = plan.m_multi & 0x7FFFFFFFu;
-  const bool multi = (plan.m_multi >> 31) != 0;
-  const uint32_t m_dst = A.m_dst_override ? A.m_dst_override : m_src;
-  const uint32_t lg = 31u - (uint32_t)__clz(m_dst);
-  const uint32_t dst_leaf0 = A.m_dst_override ? 0u : plan.leaf0;
-  const uint32_t j = plan.items;
-  const uint32_t n_out = min(A.chunk_leaves, m_dst - plan.o_lo);  // output leaves of the chunk
-  const uint32_t out_slot0 = (dst_leaf0 + plan.o_lo) << ls_dst;          // N <= 2^31 slots
-  const uint32_t a = leaf_rank0(plan.o_lo, j, lg);
-  const uint32_t span = leaf_rank0(plan.o_lo + n_out, j, lg) - a;  // items the chunk receives
-  const uint32_t nl = span ? plan.i_hi - plan.i_lo + 1u : 0u;       // source leaves feeding the chunk
-  const uint32_t gl0 = plan.leaf0 + plan.i_lo;                      // the chunk's first source leaf
-  const uint32_t seg_leaves = SEG_LEAVES_SLOTS >> ls_src;
-  const uint32_t lpl = 1u << (ls_src - 2u);                          // lanes per source leaf
-  const unsigned gm = ((1u << lpl) - 1u) << (lane & ~(lpl - 1u));    // the lanes of my leaf
-  const uint32_t R0 = nl ? A.rank_off[plan.leaf0] : 0u;
-
-  // item of window rank r, written straight into its final slot
-  auto place = [&](uint32_t r, uint32_t d, uint32_t v) {
-    const uint32_t t = r - a;
-    if (t < span) {
-      const uint32_t pos = s_pos[t];
-      s_dest[pos] = d;
-      s_val[pos] = v;
-      // fix_sentinel (reference PCSR.cpp:168-183): a sentinel that lands here refreshes its vertex's back pointer
-      if (d == PPCSR_SENT) A.beg[v - 1u] = out_slot0 + pos;
-    }
-  };
-
-  for (uint32_t seg = 0; seg < nl || seg == 0; seg += seg_leaves) {
-    const uint32_t seg_nl = min(seg_leaves, nl - seg);
-    const uint32_t seg_slot0 = (gl0 + seg) << ls_src;  // first source slot of the segment
-    const uint32_t seg_slots = seg_nl << ls_src;
-    if (seg) __syncthreads();  // everybody is done with the previous segment's tables
-    // ---- P1: loads.  Nothing below depends on anything but the plan entry.
-    uint4 D[QPT], V[QPT];
-#pragma unroll
-    for (int u = 0; u < QPT; u++) {
-      const uint32_t rel = (u * KT + threadIdx.x) * 4u;
-      D[u] = make_uint4(0u, 0u, 0u, 0u);
-      V[u] = make_uint4(0u, 0u, 0u, 0u);
-      if (rel < seg_slots) {
-        D[u] = *reinterpret_cast<const uint4 *>(A.src_dest + seg_slot0 + rel);
-        V[u] = *reinterpret_cast<const uint4 *>(A.src_val + seg_slot0 + rel);
-      }
-    }
-    uint32_t ip[INS_PREFETCH], id[INS_PREFETCH], iv[INS_PREFETCH];
-    if (seg == 0) {
-#pragma unroll
-      for (int u = 0; u < INS_PREFETCH; u++) {
-        const uint32_t q = plan.q_lo + u * KT + threadIdx.x;
-        if (q < plan.q_hi) {
-          ip[u] = A.ins_pred[q];
-          id[u] = A.ins_dst[q];
-          iv[u] = A.ins_val[q];
-        }
-      }
-    }
-    for (uint32_t x = threadIdx.x; x <= seg_nl && nl; x += KT) {
-      s_R[x] = A.rank_off[gl0 + seg + x] - R0;
-      s_ioff[x] = A.ins_off[gl0 + seg + x];
-    }
-    {
-      const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
-#pragma unroll
-      for (int u = 0; u < QPT; u++) reinterpret_cast<uint4 *>(s_last)[u * KT + threadIdx.x] = zero;
-    }
-    if (seg == 0) {  // null the staging buffers; first rank of every output leaf
-      const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
-      uint4 *zd = reinterpret_cast<uint4 *>(s_dest), *zv = reinterpret_cast<uint4 *>(s_val);
-#pragma unroll
-      for (int x = 0; x < CHUNK_SLOTS / 4 / KT; x++) {
-        zd[x * KT + threadIdx.x] = zero;
-        zv[x * KT + threadIdx.x] = zero;
-      }
-      for (uint32_t k = threadIdx.x; k <= n_out; k += KT) s_a[k] = leaf_rank0(plan.o_lo + k, j, lg) - a;
-      __syncthreads();
-      // rank -> slot table, built per output leaf by (KT / max leaves) threads each
-      constexpr uint32_t TPL8 = KT / (CHUNK_SLOTS / 8);  // threads per 8-slot leaf (a power of two; 0 = several leaves per thread)
-      static_assert(TPL8 >= 1, "at least one thread per smallest leaf");
-      const uint32_t tpl_shift = (ls_dst - 3u) + (31u - (uint32_t)__clz(TPL8));
-      const uint32_t k = threadIdx.x >> tpl_shift, sub = threadIdx.x & ((1u << tpl_shift) - 1u);
-      if (k < n_out) {
-        const uint32_t a_k = s_a[k], cnt = s_a[k + 1] - a_k;
-        for (uint32_t i = sub; i < cnt; i += 1u << tpl_shift) s_pos[a_k + i] = (uint16_t)((k << ls_dst) + i);
-      }
-    }
-    // kept items (tombstones have val 0 and drop out here) and their running count inside the leaf
-    uint32_t pre[QPT];
-#pragma unroll
-    for (int u = 0; u < QPT; u++) {
-      const uint32_t k0 = V[u].x != 0u, k1 = V[u].y != 0u, k2 = V[u].z != 0u, k3 = V[u].w != 0u;
-      const uint32_t c = k0 + k1 + k2 + k3;
-      pre[u] = leaf_incl_scan(c, lane, lpl) - c;  // kept items of my leaf in lower lanes
-      const uint32_t p0 = pre[u] + k0, p1 = p0 + k1, p2 = p1 + k2, p3 = p2 + k3;
-      reinterpret_cast<uint32_t *>(s_kupto)[u * KT + threadIdx.x] = p0 | (p1 << 8) | (p2 << 16) | (p3 << 24);
-    }
-    __syncthreads();
-    // ---- P2: the segment's inserts: rank = R[leaf] + index in the leaf's run + kept items up to the predecessor.
-    // plan.q_lo / q_hi already exclude the inserts of the first / last leaf that cannot rank inside the chunk.
-    {
-      const uint32_t q_begin = max(plan.q_lo, s_ioff[0]), q_end = min(plan.q_hi, s_ioff[seg_nl]);
-      auto insert = [&](uint32_t q, uint32_t pred, uint32_t d, uint32_t v) {
-        const uint32_t rel = pred - seg_slot0;
-        const uint32_t li = rel >> ls_src;
-        const uint32_t t = q - s_ioff[li];
-        atomicMax(&s_last[rel], t + 1u);
-        place(s_R[li] + t + s_kupto[rel], d, v);
-      };
-      uint32_t q = q_begin + threadIdx.x;
-      if (seg == 0) {
-#pragma unroll
-        for (int u = 0; u < INS_PREFETCH; u++, q += KT)
-          if (q < q_end) insert(q, ip[u], id[u], iv[u]);
-      }
-      for (; q < q_end; q += KT) insert(q, A.ins_pred[q], A.ins_dst[q], A.ins_val[q]);
-    }
-    __syncthreads();
-    // ---- P3: kept items: rank = R[leaf] + kept before + inserts hanging on earlier slots of the leaf.  The inserts
-    // of a leaf are ordered by predecessor, so that count is `last` of the nearest earlier slot that has any (a
-    // running maximum); the inserts of the chunk's first leaf that the plan clipped away all rank below the chunk,
-    // i.e. precede every item that is placed.
-    const uint32_t base_lo = (seg == 0 && nl) ? plan.q_lo - s_ioff[0] : 0u;
-#pragma unroll
-    for (int u = 0; u < QPT; u++) {
-      const uint32_t rel = (u * KT + threadIdx.x) * 4u;
-      const uint4 L = reinterpret_cast<const uint4 *>(s_last)[u * KT + threadIdx.x];
-      const uint32_t lane_max = max(max(L.x, L.y), max(L.z, L.w));
-      const unsigned nz = __ballot_sync(0xFFFFFFFFu, lane_max != 0u) & lt & gm;
-      uint32_t carry = __shfl_sync(0xFFFFFFFFu, lane_max, nz ? 31 - __clz(nz) : 0);
-      if (!nz) carry = 0;
-      const uint32_t my_leaf = rel >> ls_src;
-      if (my_leaf == 0) carry = max(carry, base_lo);
-      const uint32_t k0 = V[u].x != 0u, k1 = V[u].y != 0u, k2 = V[u].z != 0u, k3 = V[u].w != 0u;
-      if (k0 | k1 | k2 | k3) {  // implies rel < seg_slots
-        const uint32_t Rl = s_R[my_leaf] + pre[u];
-        const uint32_t ib1 = max(carry, L.x), ib2 = max(ib1, L.y), ib3 = max(ib2, L.z);
-        if (k0) place(Rl + carry, D[u].x, V[u].x);
-        if (k1) place(Rl + k0 + ib1, D[u].y, V[u].y);
-        if (k2) place(Rl + k0 + k1 + ib2, D[u].z, V[u].z);
-        if (k3) place(Rl + k0 + k1 + k2 + ib3, D[u].w, V[u].w);
-      }
-    }
-  }
-  // every source leaf has been read (a single-CTA window is rebalanced in place) and the staging buffers are
-  // complete: write the chunk
-  {
-    uint32_t *out_dest = (multi ? A.out_dest_multi : A.out_dest_single) + out_slot0;
-    uint32_t *out_val = (multi ? A.out_val_multi : A.out_val_single) + out_slot0;
-    const uint32_t out_slots = n_out << ls_dst;
-#if PPCSR_TMA_STORE
-    fence_proxy_async_smem();
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      bulk_s2g(out_dest, s_dest, out_slots * 4u);
-      bulk_s2g(out_val, s_val, out_slots * 4u);
-      bulk_commit();
-    }
-#else
-    __syncthreads();
-    for (uint32_t x = threadIdx.x * 4u; x < out_slots; x += KT * 4u) {
-      *reinterpret_cast<uint4 *>(out_dest + x) = *reinterpret_cast<const uint4 *>(s_dest + x);
-      *reinterpret_cast<uint4 *>(out_val + x) = *reinterpret_cast<const uint4 *>(s_val + x);
-    }
-#endif
-  }
-  for (uint32_t k = threadIdx.x; k < n_out; k += KT) A.tree_leaf_out[dst_leaf0 + plan.o_lo + k] = s_a[k + 1] - s_a[k];
-#if PPCSR_TMA_STORE
-  if (threadIdx.x == 0) bulk_wait_read0();  // the staging buffers must outlive the copy
-#endif
-}
-
-#endif  // PPCSR_HAVE_V6
-
-// ---------------------------------------------------------------------------------------------------------
-// k_rebalance_p: the same rank arithmetic as k_rebalance, as a PERSISTENT, software-pipelined kernel (the default).
-//
-// ncu on k_rebalance (profiles/r1_v6c_*): 40 % of the warp stall samples sit on the first use of the chunk's plan
-// entry and of its source quads -- every CTA walks plan -> addresses -> DRAM -> compute -> store with nothing to
-// overlap but the three other CTAs of its SM -- and another 25 % at its five block barriers.  Here one CTA per
-// resident slot (grid = SMs x PPCSR_REB_CTAS) loops over the chunks c, c+G, c+2G, ...; a ROUND is one segment of
-// one chunk, and as soon as the operands of a round sit in registers (after P1) lane 0 of four warps issues the bulk
-// copies (cp.async.bulk global -> shared, completing on ONE mbarrier with four arrivals) of the next round:
-//   * source quads of the segment, its R / insert-offset slices, and for the first segment of a chunk its first
-//     PINS inserts, R0 and the plan entry of the chunk after it;
-// so DRAM latency hides behind P2/P3 of the previous round, and the bulk store of a chunk drains while the next
-// one runs P1.  Two block barriers per round instead of five:
-//   BT  all placements of the previous round are done (then: bulk store of a finished chunk, wait for the stage)
-//   P1  stage -> registers; markers of the inserts; tables; kept counts; staging buffers re-zeroed
-//   B2  tables complete, stage consumed (then: bulk loads of the next round)
-//   P2  inserts placed;  P3  kept items placed -- no barrier between them: the marker a kept item needs (how many
-//       inserts hang on earlier slots of its leaf) is written in P1 by the LAST insert of each slot (neighbour
-//       compare on the staged predecessors: 16-bit, no shared-memory atomics) and cleared again by its reader.
-// The warps of a CTA do not carry the same load (see "Division of labour" below); the per-chunk housekeeping -- the
-// rank -> slot table of the CTA's NEXT chunk (double-buffered), leaf counts, tables, the store -- is dealt to the light
-// ones.  Measured (B200, same box as k_rebalance): C2 265 -> 225 us, C4 2.46 -> 2.23 ms, C3 124 -> 121 us.
-// ---------------------------------------------------------------------------------------------------------
-constexpr int PINS = INS_PREFETCH * KT;  // staged inserts per chunk
-// leaves per segment: 64 of 32 slots; arrays with smaller leaves are tiny, their segments are capped at 128 leaves
-constexpr int PSEG_MAX_LEAVES = SEG_LEAVES_SLOTS / 32 > 128 ? SEG_LEAVES_SLOTS / 32 : 128;
-constexpr int TBL = PSEG_MAX_LEAVES + 1;
-
-struct PSmem {  // dynamic shared memory layout of k_rebalance_p
-  uint32_t s_dest[CHUNK_SLOTS];   // the chunk's output slots in their final layout (128-byte aligned: first member)
-  uint32_t s_val[CHUNK_SLOTS];
-  uint32_t st_d[SEG_LEAVES_SLOTS];  // stage: source quads of the next round
-  uint32_t st_v[SEG_LEAVES_SLOTS];
-  uint16_t s_last[SEG_LEAVES_SLOTS];  // 1 + (index - base) of the last insert hanging on a slot
-  uint16_t s_pos[2][CHUNK_SLOTS];     // chunk-relative rank -> output slot; [parity of the CTA's chunk count]
-  uint8_t s_kupto[SEG_LEAVES_SLOTS];  // kept items of the leaf up to and including a slot
-  uint32_t s_R[TBL + 3], s_ioff[TBL + 3];
-  // stage, 16-byte aligned arrays filled by bulk copies that start at the 16-byte boundary below the first element
-  // wanted: entry x of a table sits at [x + (first index & 3)]
-  alignas(16) uint32_t st_R[TBL + 7];     // R slice of the next round's segment
-  alignas(16) uint32_t st_ioff[TBL + 7];  // insert offsets of the same leaves
-  alignas(16) uint32_t st_ip[PINS + 8];   // first inserts of the next chunk (+ one more predecessor)
-  alignas(16) uint32_t st_id[PINS + 8];
-  alignas(16) uint32_t st_iv[PINS + 8];
-  alignas(16) uint32_t st_R0[4];
-  alignas(16) uint4 plan[2][2];           // plan entries: [parity][half]
-  alignas(8) uint64_t mbar;               // completion of the stage's bulk copies
-};
 
 // ---- mbarrier + bulk copy global -> shared (the TMA engine; sm_90+/sm_100a PTX) ------------------------------
 __device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
@@ -463,353 +135,11 @@ __device__ __forceinline__ void bulk_g2s(void *dst_smem, const void *src_gmem, u
                "l"(src_gmem), "r"(bytes), "r"(smem_u32(bar))
                : "memory");
 }
-__device__ __forceinline__ ChunkPlan plan_from(const uint4 lo, const uint4 hi) {
-  ChunkPlan r;
-  r.leaf0 = lo.x; r.m_multi = lo.y; r.items = lo.z; r.o_lo = lo.w;
-  r.i_lo = hi.x; r.i_hi = hi.y; r.q_lo = hi.z; r.q_hi = hi.w;
-  return r;
-}
-
-__global__ void __launch_bounds__(KT, PPCSR_REB_CTAS) k_rebalance_p(Args A, uint32_t n_chunks) {
-  extern __shared__ __align__(128) uint8_t p_smem_raw[];
-  PSmem &S = *reinterpret_cast<PSmem *>(p_smem_raw);
-  const unsigned lane = lane_id(), lt = lanemask_lt();
-  const uint32_t ls_src = A.ls_src, ls_dst = A.ls_dst;
-  const uint32_t seg_leaves = min((uint32_t)SEG_LEAVES_SLOTS >> ls_src, (uint32_t)PSEG_MAX_LEAVES);
-  const uint32_t lpl = 1u << (ls_src - 2u);                        // lanes per source leaf
-  const unsigned gm = ((1u << lpl) - 1u) << (lane & ~(lpl - 1u));  // the lanes of my leaf
-  const uint32_t warp_rel0 = (threadIdx.x & ~31u) * 4u;            // first slot of my warp's quads in round 0
-  const uint32_t G = gridDim.x;
-  constexpr uint32_t NONE = 0xFFFFFFFFu;
-
-  uint32_t c = blockIdx.x;
-  if (c >= n_chunks) return;
-  // Division of labour between the warps of the CTA.  The per-item phases are spread over all warps, but not evenly:
-  // a chunk's source range is its share of the leaves plus one or two straddled at the ends, so warp 0 runs a second
-  // round of quads that the others skip, and the inserts beyond the first KT land on one or two warps (they are
-  // dealt from the last thread down so that these are not warp 0 again).  Everybody waits for the slowest warp at
-  // the round's barrier, so the per-chunk housekeeping goes to the others: warp IO_WARP stores the finished chunk and
-  // re-zeroes the staging buffers, the warps other than 0 and IO_WARP ("hk") build the tables -- the rank -> slot
-  // table of the NEXT chunk after their own P3, while warp 0 is still placing -- and lane 0 of four of them issues
-  // the bulk loads of the next round (quads / tables + R0 / inserts / plan entry: one mbarrier arrival each).
-  const unsigned warp = threadIdx.x >> 5;
-  constexpr unsigned IO_WARP = 3;
-  static_assert(KT >= 128, "k_rebalance_p deals its housekeeping to warps 1, 2 (4, 5) (loads) and 3 (store)");
-  constexpr uint32_t HK = KT - 64;  // housekeeping threads
-  const bool is_io = warp == IO_WARP, is_io_thread = threadIdx.x == IO_WARP * 32;
-  const bool is_hk = warp != 0 && warp != IO_WARP;
-  const uint32_t hk_tid = threadIdx.x - 32u - (warp > IO_WARP ? 32u : 0u);
-  const uint32_t itid = KT - 1u - threadIdx.x;  // my place in the deal of the inserts
-  // issuer threads: lane 0 of warp 1 (role 0: quads), 2 (1: tables, R0), 4 (2: inserts), 5 (3: plan entry)
-  // (a CTA of 128 threads has no warps 4 and 5: lanes 0 and 1 of warps 1 and 2 issue instead)
-  const bool is_issuer = KT >= 256 ? lane == 0 && (warp == 1 || warp == 2 || warp == 4 || warp == 5)
-                                   : lane < 2 && (warp == 1 || warp == 2);
-  const uint32_t role = KT >= 256 ? (warp < 3 ? warp - 1u : warp - 2u) : (warp - 1u) * 2u + lane;
-
-  // The bulk copies of one round, complete on the stage's mbarrier (four arrivals).  gl / snl: first leaf and leaf
-  // count of the segment; first_seg: the round opens chunk p (stage its first inserts and R0 too, and fetch the
-  // plan entry of the CTA's chunk after it into plan slot `slot_after`).
-  auto issue_round = [&](bool first_seg, uint32_t gl, uint32_t snl, const ChunkPlan &p, uint32_t c_after,
-                         uint32_t slot_after) {
-    uint32_t bytes = 0;
-    if (role == 0) {
-      if (snl) {
-        const uint32_t qb = (snl << ls_src) * 4u;
-        bulk_g2s(S.st_d, A.src_dest + ((size_t)gl << ls_src), qb, &S.mbar);
-        bulk_g2s(S.st_v, A.src_val + ((size_t)gl << ls_src), qb, &S.mbar);
-        bytes = 2u * qb;
-      }
-    } else if (role == 1) {
-      if (snl) {
-        const uint32_t sh = gl & 3u;
-        // 16-byte granules: reads up to 3 entries past rank_off / ins_off [n_leaves] (covered by DEV_PAD_ELEMS)
-        const uint32_t tb = ((snl + 1u + sh + 3u) & ~3u) * 4u;
-        bulk_g2s(S.st_R, A.rank_off + (gl - sh), tb, &S.mbar);
-        bulk_g2s(S.st_ioff, A.ins_off + (gl - sh), tb, &S.mbar);
-        bytes = 2u * tb;
-        if (first_seg) {
-          bulk_g2s(S.st_R0, A.rank_off + (p.leaf0 & ~3u), 16u, &S.mbar);
-          bytes += 16u;
-        }
-      }
-    } else if (role == 2) {
-      const uint32_t nq = p.q_hi - p.q_lo;
-      if (first_seg && snl && nq) {
-        const uint32_t sh = p.q_lo & 3u;
-        const uint32_t ib = ((min(nq, (uint32_t)PINS + 1u) + sh + 3u) & ~3u) * 4u;
-        bulk_g2s(S.st_ip, A.ins_pred + (p.q_lo - sh), ib, &S.mbar);
-        bulk_g2s(S.st_id, A.ins_dst + (p.q_lo - sh), ib, &S.mbar);
-        bulk_g2s(S.st_iv, A.ins_val + (p.q_lo - sh), ib, &S.mbar);
-        bytes = 3u * ib;
-        if (nq > (uint32_t)PINS) {  // a run longer than the stage is read straight from global memory: pull it into L2
-          const uint32_t q1 = (p.q_lo + PINS) & ~3u;
-          const uint32_t tb = min(((p.q_hi - q1 + 3u) & ~3u) * 4u, 16384u);
-          bulk_prefetch_l2(A.ins_pred + q1, tb);
-          bulk_prefetch_l2(A.ins_dst + q1, tb);
-          bulk_prefetch_l2(A.ins_val + q1, tb);
-        }
-      }
-    } else {
-      if (first_seg && c_after < n_chunks) {
-        bulk_g2s(&S.plan[slot_after][0], A.plan + c_after, 32u, &S.mbar);
-        bytes = 32u;
-      }
-    }
-    mbar_expect_tx(&S.mbar, bytes);
-  };
-  auto issue_chunk = [&](const ChunkPlan &p, uint32_t c_after, uint32_t slot_after) {
-    const uint32_t nl_n = p.i_lo <= p.i_hi ? p.i_hi - p.i_lo + 1u : 0u;
-    issue_round(true, p.leaf0 + p.i_lo, min(seg_leaves, nl_n), p, c_after, slot_after);
-  };
-  // rank -> slot table of the chunk with plan entry p, by the hk threads: (1 << tpl_shift) threads per output leaf
-  auto build_pos = [&](const ChunkPlan &p, uint32_t buf) {
-    const uint32_t md = A.m_dst_override ? A.m_dst_override : (p.m_multi & 0x7FFFFFFFu);
-    const uint32_t lgn = 31u - (uint32_t)__clz(md);
-    const uint32_t no = min(A.chunk_leaves, md - p.o_lo);
-    const uint32_t an = leaf_rank0(p.o_lo, p.items, lgn);
-    const uint32_t tpl_shift = ls_dst - 3u;
-    uint16_t *tab = S.s_pos[buf];
-    for (uint32_t x = hk_tid; x < (no << tpl_shift); x += HK) {
-      const uint32_t kk = x >> tpl_shift, sub = x & ((1u << tpl_shift) - 1u);
-      const uint32_t a_k = leaf_rank0(p.o_lo + kk, p.items, lgn) - an;
-      const uint32_t cnt = leaf_rank0(p.o_lo + kk + 1u, p.items, lgn) - an - a_k;
-      for (uint32_t i = sub; i < cnt; i += 1u << tpl_shift) tab[a_k + i] = (uint16_t)((kk << ls_dst) + i);
-    }
-  };
-  {
-    const uint4 lo = __ldg(reinterpret_cast<const uint4 *>(A.plan + c));
-    const uint4 hi = __ldg(reinterpret_cast<const uint4 *>(A.plan + c) + 1);
-    if (threadIdx.x == 0) {
-      S.plan[0][0] = lo;
-      S.plan[0][1] = hi;
-      mbar_init(&S.mbar, 4u);
-    }
-    const uint4 zero = make_uint4(0u, 0u, 0u, 0u);  // the markers start out clear; every round clears what it set
-    for (uint32_t x = threadIdx.x; x < (uint32_t)SEG_LEAVES_SLOTS * 2u / 16u; x += KT)
-      reinterpret_cast<uint4 *>(S.s_last)[x] = zero;
-    if (is_hk) build_pos(plan_from(lo, hi), 0u);
-    __syncthreads();  // the mbarrier is initialised before anybody arrives on it or polls it
-    if (is_issuer) issue_chunk(plan_from(lo, hi), c + G, 1u);
-  }
-  uint32_t parity = 0;
-
-  // state of the chunk in progress (set by its first segment)
-  ChunkPlan plan;
-  uint32_t k = 0, seg = 0;
-  uint32_t m_dst = 0, lg = 0, dst_leaf0 = 0, j = 0, n_out = 0, out_slot0 = 0, a = 0, span = 0, nl = 0, gl0 = 0, R0 = 0;
-  bool multi = false, store_pending = false;
-
-  // item of window rank r, written straight into its final slot; returns the slot (or CHUNK_SLOTS)
-  auto place = [&](uint32_t r, uint32_t d, uint32_t v) -> uint32_t {
-    const uint32_t t = r - a;
-    uint32_t pos = CHUNK_SLOTS;
-    if (t < span) {
-      pos = S.s_pos[k & 1u][t];
-      S.s_dest[pos] = d;
-      S.s_val[pos] = v;
-    }
-    return pos;
-  };
-  // fix_sentinel (reference PCSR.cpp:168-183): a sentinel that lands in slot pos refreshes its vertex's back pointer
-  auto fix_sentinel = [&](uint32_t d, uint32_t v, uint32_t pos) {
-    if (d == PPCSR_SENT && pos < CHUNK_SLOTS) A.beg[v - 1u] = out_slot0 + pos;
-  };
-
-  for (;;) {  // one round per (chunk, segment of <= SEG_LEAVES_SLOTS source slots)
-    if (store_pending) fence_proxy_async_smem();  // my placements are visible to the bulk-copy engine
-    __syncthreads();                              // BT: previous round's tables free, the chunk's placements done
-    if (store_pending) {
-      if (is_io_thread) {  // the finished chunk leaves: one bulk store per array
-        const uint32_t bytes = (n_out << ls_dst) * 4u;
-        bulk_s2g((multi ? A.out_dest_multi : A.out_dest_single) + out_slot0, S.s_dest, bytes);
-        bulk_s2g((multi ? A.out_val_multi : A.out_val_single) + out_slot0, S.s_val, bytes);
-        bulk_commit();
-      }
-      store_pending = false;
-      if (c >= n_chunks) break;
-    }
-    mbar_wait(&S.mbar, parity);  // this round's operands (and plan entry) have landed in the stage
-    parity ^= 1u;
-    if (seg == 0) {
-      plan = plan_from(S.plan[k & 1u][0], S.plan[k & 1u][1]);
-      const uint32_t m_src = plan.m_multi & 0x7FFFFFFFu;
-      multi = (plan.m_multi >> 31) != 0;
-      m_dst = A.m_dst_override ? A.m_dst_override : m_src;
-      lg = 31u - (uint32_t)__clz(m_dst);
-      dst_leaf0 = A.m_dst_override ? 0u : plan.leaf0;
-      j = plan.items;
-      n_out = min(A.chunk_leaves, m_dst - plan.o_lo);  // output leaves of the chunk
-      out_slot0 = (dst_leaf0 + plan.o_lo) << ls_dst;          // N <= 2^31 slots
-      a = leaf_rank0(plan.o_lo, j, lg);
-      span = leaf_rank0(plan.o_lo + n_out, j, lg) - a;        // items the chunk receives
-      nl = plan.i_lo <= plan.i_hi ? plan.i_hi - plan.i_lo + 1u : 0u;  // source leaves feeding the chunk
-      gl0 = plan.leaf0 + plan.i_lo;                           // the chunk's first source leaf
-      R0 = nl ? S.st_R0[plan.leaf0 & 3u] : 0u;
-    }
-    const uint32_t seg_nl = min(seg_leaves, nl - seg);
-    const uint32_t seg_slot0 = (gl0 + seg) << ls_src;  // first source slot of the segment
-    const uint32_t seg_slots = seg_nl << ls_src;
-    const uint32_t *t_R = S.st_R + ((gl0 + seg) & 3u), *t_ioff = S.st_ioff + ((gl0 + seg) & 3u);  // staged tables
-    // ---- P1: operands from the stage into registers
-    uint4 D[QPT], V[QPT];
-#pragma unroll
-    for (int u = 0; u < QPT; u++) {
-      const uint32_t rel = (u * KT + threadIdx.x) * 4u;
-      D[u] = make_uint4(0u, 0u, 0u, 0u);
-      V[u] = make_uint4(0u, 0u, 0u, 0u);
-      if (rel < seg_slots) {
-        D[u] = *reinterpret_cast<const uint4 *>(S.st_d + rel);
-        V[u] = *reinterpret_cast<const uint4 *>(S.st_v + rel);
-      }
-    }
-    // the segment's inserts: plan.q_lo / q_hi already exclude those of the chunk's first / last leaf that cannot rank
-    // inside the chunk.  First segment: from the stage; later segments: straight from global memory.  The LAST
-    // insert hanging on a slot (its successor has another predecessor) leaves 1 + its index in the leaf's run there
-    // (relative to the clipped start in the chunk's first leaf): P3 needs no more than that, and it costs no barrier.
-    const uint32_t q_begin = nl ? max(plan.q_lo, t_ioff[0]) : 0u;
-    const uint32_t q_end = nl ? min(plan.q_hi, t_ioff[seg_nl]) : 0u;
-    const uint32_t base_lo = (seg == 0 && nl) ? plan.q_lo - t_ioff[0] : 0u;
-    const uint32_t ish = plan.q_lo & 3u;  // staged insert i sits at [i + ish]
-    auto mark = [&](uint32_t q, uint32_t pred, uint32_t nx) {
-      if (nx != pred) {
-        const uint32_t rel = pred - seg_slot0;
-        const uint32_t li = rel >> ls_src;
-        S.s_last[rel] = (uint16_t)(q - t_ioff[li] + 1u - (li == 0u ? base_lo : 0u));
-      }
-    };
-    uint32_t ip[INS_PREFETCH], id[INS_PREFETCH], iv[INS_PREFETCH];
-#pragma unroll
-    for (int u = 0; u < INS_PREFETCH; u++) {
-      const uint32_t i = u * KT + itid;
-      const uint32_t q = q_begin + i;
-      ip[u] = id[u] = iv[u] = 0u;
-      if (q < q_end) {
-        uint32_t nx = NONE;
-        if (seg == 0) {
-          ip[u] = S.st_ip[i + ish];
-          id[u] = S.st_id[i + ish];
-          iv[u] = S.st_iv[i + ish];
-          if (q + 1u < q_end) nx = S.st_ip[i + ish + 1u];
-        } else {
-          ip[u] = A.ins_pred[q];
-          id[u] = A.ins_dst[q];
-          iv[u] = A.ins_val[q];
-          if (q + 1u < q_end) nx = A.ins_pred[q + 1u];
-        }
-        mark(q, ip[u], nx);
-      }
-    }
-    for (uint32_t q = q_begin + PINS + itid; q < q_end; q += KT)  // a long run (hub vertex): beyond the stage
-      mark(q, A.ins_pred[q], q + 1u < q_end ? A.ins_pred[q + 1u] : NONE);
-    if (is_hk) {  // housekeeping: the segment's tables
-      for (uint32_t x = hk_tid; x <= seg_nl && nl; x += HK) {
-        S.s_R[x] = t_R[x] - R0;
-        S.s_ioff[x] = t_ioff[x];
-      }
-    }
-    // kept items (tombstones have val 0 and drop out here) and their running count inside the leaf
-    uint32_t pre[QPT];
-#pragma unroll
-    for (int u = 0; u < QPT; u++) {
-      pre[u] = 0;
-      if (u * KT * 4u + warp_rel0 >= seg_slots) continue;  // warp-uniform: nothing of this round lies in the segment
-      const uint32_t k0 = V[u].x != 0u, k1 = V[u].y != 0u, k2 = V[u].z != 0u, k3 = V[u].w != 0u;
-      const uint32_t cc = k0 + k1 + k2 + k3;
-      pre[u] = leaf_incl_scan(cc, lane, lpl) - cc;  // kept items of my leaf in lower lanes
-      const uint32_t p0 = pre[u] + k0, p1 = p0 + k1, p2 = p1 + k2, p3 = p2 + k3;
-      reinterpret_cast<uint32_t *>(S.s_kupto)[u * KT + threadIdx.x] = p0 | (p1 << 8) | (p2 << 16) | (p3 << 24);
-    }
-    if (seg == 0 && is_io) {  // null the staging buffers once the copy engine has read the previous chunk out of them
-      if (lane == 0) bulk_wait_read0();
-      __syncwarp();
-      const uint4 zero = make_uint4(0u, 0u, 0u, 0u);
-      uint4 *z = reinterpret_cast<uint4 *>(S.s_dest);  // s_dest and s_val are adjacent
-#pragma unroll 8
-      for (int x = 0; x < 2 * CHUNK_SLOTS / 4 / 32; x++) z[x * 32 + lane] = zero;
-    }
-    __syncthreads();  // B2: tables, markers, kept counts and nulled staging are complete; the stage has been consumed
-    // ---- the next round's operands: the chunk's next segment, or the first segment of this CTA's next chunk
-    const bool more_seg = seg + seg_leaves < nl;
-    if (is_issuer) {
-      if (more_seg) {
-        issue_round(false, gl0 + seg + seg_leaves, min(seg_leaves, nl - seg - seg_leaves), plan, 0u, 0u);
-      } else if (c + G < n_chunks) {
-        issue_chunk(plan_from(S.plan[(k + 1u) & 1u][0], S.plan[(k + 1u) & 1u][1]), c + 2u * G, k & 1u);
-      }
-    }
-    // ---- P2: inserts: rank = R[leaf] + index in the leaf's run + kept items up to the predecessor
-    {
-      auto insert = [&](uint32_t q, uint32_t pred, uint32_t d, uint32_t v) {
-        const uint32_t rel = pred - seg_slot0;
-        const uint32_t li = rel >> ls_src;
-        const uint32_t pos = place(S.s_R[li] + (q - S.s_ioff[li]) + S.s_kupto[rel], d, v);
-        if (A.ins_sentinels) fix_sentinel(d, v, pos);
-      };
-      uint32_t q = q_begin + itid;
-#pragma unroll
-      for (int u = 0; u < INS_PREFETCH; u++, q += KT)
-        if (q < q_end) insert(q, ip[u], id[u], iv[u]);
-      for (; q < q_end; q += KT) insert(q, A.ins_pred[q], A.ins_dst[q], A.ins_val[q]);
-    }
-    // ---- P3: kept items: rank = R[leaf] + kept before + inserts hanging on earlier slots of the leaf.  The inserts
-    // of a leaf are ordered by predecessor, so that count is the marker of the nearest earlier slot that has one (a
-    // running maximum); the inserts of the chunk's first leaf that the plan clipped away all rank below the chunk,
-    // i.e. precede every item that is placed (base_lo).
-#pragma unroll
-    for (int u = 0; u < QPT; u++) {
-      if (u * KT * 4u + warp_rel0 >= seg_slots) continue;  // warp-uniform
-      const uint32_t rel = (u * KT + threadIdx.x) * 4u;
-      const uint2 Lw = reinterpret_cast<const uint2 *>(S.s_last)[u * KT + threadIdx.x];
-      if (Lw.x | Lw.y) reinterpret_cast<uint2 *>(S.s_last)[u * KT + threadIdx.x] = make_uint2(0u, 0u);  // clear what was set
-      const uint32_t L0 = Lw.x & 0xFFFFu, L1 = Lw.x >> 16, L2 = Lw.y & 0xFFFFu, L3 = Lw.y >> 16;
-      const uint32_t lane_max = max(max(L0, L1), max(L2, L3));
-      const unsigned nz = __ballot_sync(0xFFFFFFFFu, lane_max != 0u) & lt & gm;
-      uint32_t carry = __shfl_sync(0xFFFFFFFFu, lane_max, nz ? 31 - __clz(nz) : 0);
-      if (!nz) carry = 0;
-      const uint32_t my_leaf = rel >> ls_src;
-      const uint32_t k0 = V[u].x != 0u, k1 = V[u].y != 0u, k2 = V[u].z != 0u, k3 = V[u].w != 0u;
-      if (k0 | k1 | k2 | k3) {  // implies rel < seg_slots
-        const uint32_t Rl = S.s_R[my_leaf] + pre[u] + (my_leaf == 0u ? base_lo : 0u);
-        const uint32_t ib1 = max(carry, L0), ib2 = max(ib1, L1), ib3 = max(ib2, L2);
-        uint32_t p0 = CHUNK_SLOTS, p1 = CHUNK_SLOTS, p2 = CHUNK_SLOTS, p3 = CHUNK_SLOTS;
-        if (k0) p0 = place(Rl + carry, D[u].x, V[u].x);
-        if (k1) p1 = place(Rl + k0 + ib1, D[u].y, V[u].y);
-        if (k2) p2 = place(Rl + k0 + k1 + ib2, D[u].z, V[u].z);
-        if (k3) p3 = place(Rl + k0 + k1 + k2 + ib3, D[u].w, V[u].w);
-        if (D[u].x == PPCSR_SENT || D[u].y == PPCSR_SENT || D[u].z == PPCSR_SENT || D[u].w == PPCSR_SENT) {
-          fix_sentinel(D[u].x, V[u].x, p0);
-          fix_sentinel(D[u].y, V[u].y, p1);
-          fix_sentinel(D[u].z, V[u].z, p2);
-          fix_sentinel(D[u].w, V[u].w, p3);
-        }
-      }
-    }
-    if (more_seg) {
-      seg += seg_leaves;
-      continue;
-    }
-    // every source leaf has been read (a single-CTA window is rebalanced in place) and the staging buffers are
-    // complete: the chunk is stored after the next barrier
-    if (is_hk) {  // post-rebalance leaf counts of this chunk; rank -> slot table of the CTA's next chunk
-      for (uint32_t kk = hk_tid; kk < n_out; kk += HK) {
-        const uint32_t c_k = leaf_rank0(plan.o_lo + kk + 1u, j, lg) - leaf_rank0(plan.o_lo + kk, j, lg);
-        A.tree_leaf_out[dst_leaf0 + plan.o_lo + kk] = c_k;
-        if (A.leaf_cnt_out) A.leaf_cnt_out[dst_leaf0 + plan.o_lo + kk] = c_k;
-      }
-      if (c + G < n_chunks) build_pos(plan_from(S.plan[(k + 1u) & 1u][0], S.plan[(k + 1u) & 1u][1]), (k + 1u) & 1u);
-    }
-    store_pending = true;
-    c += G;
-    k++;
-    seg = 0;
-  }
-  if (is_io_thread) bulk_wait_read0();  // the staging buffers must outlive the last copy
-}
 
 // ---------------------------------------------------------------------------------------------------------
 // Small windows (<= SMALL_MAX_LEAVES leaves, the overwhelmingly common case of a steady-state batch: a touched
 // leaf that stays within its bounds is its own window): ONE WARP per window, no block barriers, in place.
-// Same rank arithmetic as k_rebalance; the window's items are staged in the warp's 2 KB slice of shared memory.
+// The rank arithmetic above, window by window; the window's items are staged in the warp's 2 KB slice of shared memory.
 // ---------------------------------------------------------------------------------------------------------
 constexpr int SMALL_MAX_LEAVES = 8;
 constexpr int SMALL_MAX_SLOTS = SMALL_MAX_LEAVES * 32;
@@ -835,7 +165,7 @@ __global__ void __launch_bounds__(RT) k_rebalance_small(SmallArgs A) {
   const uint32_t wid = blockIdx.x * RWARPS + warp;
   if (wid >= A.n_windows) return;  // whole warp exits together
   const WindowDesc w = A.windows[wid];
-  if (w.n_chunks != 0) return;     // a large window: k_rebalance owns it
+  if (w.n_chunks != 0) return;     // a large window: k_rebalance_m owns it
   const uint32_t m = w.m, j = w.items, logN = 1u << A.ls;
   const uint32_t R0 = A.rank_off[w.leaf0];
   uint32_t *sd = s_dest[warp], *sv = s_val[warp];
@@ -923,20 +253,6 @@ __global__ void __launch_bounds__(RT) k_rebalance_small(SmallArgs A) {
 }
 
 // copy the chunks of multi-CTA windows back from the out-of-place target into the live array
-__global__ void __launch_bounds__(RT) k_copy_back(const ChunkPlan *__restrict__ plan, uint32_t ls,
-                                                  const uint32_t *__restrict__ alt_dest,
-                                                  const uint32_t *__restrict__ alt_val, uint32_t *__restrict__ dest,
-                                                  uint32_t *__restrict__ val) {
-  const ChunkPlan p = plan[blockIdx.x];
-  if (!(p.m_multi >> 31)) return;
-  const uint32_t o_hi = min(p.o_lo + (CHUNK_SLOTS >> ls), p.m_multi & 0x7FFFFFFFu);
-  const size_t base = (size_t)(p.leaf0 + p.o_lo) << ls;
-  const uint32_t slots = (o_hi - p.o_lo) << ls;
-  for (uint32_t x = threadIdx.x * 4; x < slots; x += RT * 4) {
-    *reinterpret_cast<uint4 *>(dest + base + x) = *reinterpret_cast<const uint4 *>(alt_dest + base + x);
-    *reinterpret_cast<uint4 *>(val + base + x) = *reinterpret_cast<const uint4 *>(alt_val + base + x);
-  }
-}
 
 // initial layout: src_n sentinels spread evenly (reference PCSR::PCSR, PCSR.cpp:796-837, in leaf-packed form)
 __global__ void k_init_sentinels(uint32_t *__restrict__ dest, uint32_t *__restrict__ val, uint32_t *__restrict__ beg,

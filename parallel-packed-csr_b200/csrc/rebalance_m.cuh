@@ -1,15 +1,10 @@
-// rebalance_m.cuh -- reb::k_rebalance_m: the rebalance kernel in its RANK-DENSE form (the default since round 2).
-// Same job, same plan (one chunk of <= CHUNK_SLOTS output slots per round trip) and same rank arithmetic as
-// k_rebalance_p (rebalance.cuh) -- replaces reference PCSR::redistribute + fix_sentinel + slide_right/slide_left +
-// double_list/half_list (src/pcsr/PCSR.cpp:222-249, 168-183, 326-390, 251-320) -- but the work is dealt by OUTPUT
-// RANK, not by source slot:
+// rebalance_m.cuh -- reb::k_rebalance_m: the rebalance of the windows that span more than SMALL_MAX_LEAVES leaves, and
+// of the whole array.  The rank arithmetic of rebalance.cuh, dealt by OUTPUT RANK: the windows are cut into chunks of
+// <= CHUNK_SLOTS output slots (k_plan_chunks_m), and a warp takes 32 CONSECUTIVE RANKS of the merged sequence per step
+// ("unit"), so every lane has an item.  (Dealing SOURCE slots instead leaves half the lanes idle at the 50-65 % density
+// of a PMA and costs every kept item a segmented scan, a marker look-up and a running maximum: ~760 instructions per
+// chunk and warp whatever the chunk holds, issue-bound at 0.76 slots per cycle on the 2^29-slot rebuild, ncu.)
 //
-//   k_rebalance_p gives every thread a quad of SOURCE slots: at the 50-65 % density of a PMA half of those lanes
-//   hold nothing, every kept item pays a segmented scan, a marker look-up and a running maximum, every insert a
-//   marker store, and a warp runs ~760 instructions per chunk whatever the chunk holds (ncu: 1.7 G warp
-//   instructions for the 2^29-slot rebuild, issue-bound at 0.76 slots per cycle).
-//
-//   Here a warp takes 32 CONSECUTIVE RANKS of the merged sequence per step ("unit"): every lane has an item.
 //   Two bit masks over the chunk's ranks say what a rank is:
 //     B   bit t set <=> rank t is one of the batch's inserts      (one shared-memory atomicOr per insert)
 //     HB  bit t set <=> a source leaf's merged run begins at t    (one atomicOr per non-empty source leaf)
@@ -27,9 +22,9 @@
 // insert-offset slices, the chunk's first 512 (1024 when the batch carries one value: no value list) inserts -- are
 // issued by the producer at the top of round r into the other half of a double buffer, a full round ahead.
 // Two block barriers per round (three for a chunk with tombstones AND inserts); the producer only arrives at the
-// second one.  Measured (B200): the 2^29-slot rebuild of C4 in 1.67 ms = 78 % of the HBM copy peak (k_rebalance_p:
-// 2.23 ms), DRAM-bound; the scale-20 rebuilds are bound by the shared-memory data pipe (68 % busy: left-packed rows put
-// every leaf's items on the low banks) at 60-67 %.
+// second one.  Measured (B200): the 2^29-slot rebuild of C4 in 1.67 ms = 78 % of the HBM copy peak, DRAM-bound; the
+// scale-20 rebuilds are bound by the shared-memory data pipe (68 % busy: left-packed rows put every leaf's items on the
+// low banks) at 60-67 %.
 #pragma once
 #include <type_traits>
 
@@ -100,7 +95,7 @@ __global__ void __launch_bounds__(RT) k_plan_chunks_m(const WindowDesc *__restri
     const uint32_t leaf = 1u << ls_src;
     // an insert ranks at R[leaf] + (its index in the leaf's run) + (kept items up to its predecessor, <= one leaf):
     // those of the first leaf before IO + (below - leaf) rank below a, those of the last from IO + (b - R) on at or
-    // above b (the clip k_plan_chunks makes, rebalance.cuh)
+    // above b -- a hub run spanning thousands of chunks is clipped to <= span + leaf inserts per chunk without a search
     p.i_lo = i_lo;
     p.nl = i_hi - i_lo + 1u;
     p.q_lo = min(IO[i_lo] + (below > leaf ? below - leaf : 0u), IO[i_lo + 1]);
@@ -116,9 +111,6 @@ __global__ void __launch_bounds__(RT) k_plan_chunks_m(const WindowDesc *__restri
 #ifndef PPCSR_M_CTAS
 #define PPCSR_M_CTAS 3
 #endif
-#ifndef PPCSR_M_AGG
-#define PPCSR_M_AGG 0
-#endif
 #ifndef PPCSR_M_PINS
 #define PPCSR_M_PINS 512
 #endif
@@ -126,7 +118,7 @@ constexpr int MT = 256;                        // consumer threads of a k_rebala
 constexpr int MTT = MT + 32;                   // + the producer warp
 constexpr int MCHUNK = CHUNK_SLOTS;            // output slots per chunk
 constexpr int MSEG = SEG_LEAVES_SLOTS;         // source slots per round
-constexpr int MSEG_MAX_LEAVES = PSEG_MAX_LEAVES;
+constexpr int MSEG_MAX_LEAVES = SEG_MAX_LEAVES;
 constexpr int MTBL = MSEG_MAX_LEAVES + 1;
 // staged inserts per chunk: what fits beside the other buffers at three CTAs per SM.  UNIV (every insert of the batch
 // carries the same value: no value array is read at all) leaves room for more of them
@@ -154,7 +146,7 @@ __device__ uint32_t g_m_trace[4][64][9][8];
 template <bool TOMB, bool UNIV>
 struct MSmem {
   static constexpr int MPINS = MCfg<TOMB, UNIV>::PINS;
-  uint32_t out_d[MCHUNK];  // the chunk's output slots in their final layout (128-byte aligned: first member)
+  uint32_t out_d[MCHUNK];  // the chunk's output slots in their final layout (first member: at the base, see k_rebalance_m)
   uint32_t out_v[MCHUNK];
   // one word-indexed region W: the source lines and staged inserts.  st_v - st_d == st_iv - st_id (== VOFF words), so
   // an item's value sits VOFF words behind its dest whichever it is (UNIV: no st_iv; the insert lanes read a word of
@@ -193,7 +185,11 @@ __device__ __forceinline__ void bar_mid_arrive() { asm volatile("bar.arrive 2, %
 template <bool TOMB, bool UNIV>
 __global__ void __launch_bounds__(MTT, PPCSR_M_CTAS) k_rebalance_m(Args A, const ChunkPlanM *__restrict__ gplan,
                                                                   uint32_t n_chunks) {
-  extern __shared__ __align__(128) uint8_t m_smem_raw[];
+  // The kernel has no static shared memory, so its dynamic shared memory starts at the base of the CTA's window,
+  // whatever alignment is declared here.  16, like every dynamic shared-memory declaration of the library: ptxas aligns
+  // the dynamic shared memory of ALL kernels of the module to one of these declarations (which one depends on the order
+  // the kernels are emitted in), and a larger one here would move it in the sort and routing kernels.
+  extern __shared__ __align__(16) uint8_t m_smem_raw[];
   using SM = MSmem<TOMB, UNIV>;
   constexpr int MPINS = SM::MPINS;
   SM &S = *reinterpret_cast<SM *>(m_smem_raw);
@@ -474,17 +470,9 @@ __global__ void __launch_bounds__(MTT, PPCSR_M_CTAS) k_rebalance_m(Args A, const
               below++;
             }
           }
-          // (PPCSR_M_AGG: the lanes that share a mask word OR their bits together and one of them updates the word --
-          // measured slower than the ~10-way same-word atomics it avoids: match.any costs more)
-#if PPCSR_M_AGG
-          const unsigned peers = __match_any_sync(0xFFFFFFFFu, word);
-          if (word != 0xFFFFFFFFu) {
-            const uint32_t bits = __reduce_or_sync(peers, bit);
-            if ((peers & lt) == 0u) atomicOr(&S.B[rpar][word], bits);
-          }
-#else
+          // (one atomic per lane: warp-aggregating the lanes that share a word through match.any measured slower than
+          // the ~10-way same-word atomics it avoids)
           if (word != 0xFFFFFFFFu) atomicOr(&S.B[rpar][word], bit);
-#endif
         }
         if (first_seg) {
           below = __reduce_add_sync(0xFFFFFFFFu, below);

@@ -70,9 +70,8 @@ __device__ __forceinline__ uint32_t sort_digit(uint64_t key, int lo_bits, int sh
   return (uint32_t)(sort_compact(key, lo_bits) >> shift) & mask;
 }
 
-// Where the FIRST pass of a sort (and the histogram kernel) takes its keys from: an array of key words, or the raw
-// update arrays themselves (batch.cuh: RawArrays / RawPacked / RawSegments build the key word on the fly, so the batch
-// is never materialised as an unsorted key array: one write and one read of the batch less).
+// Where a pass of the sort takes its keys (and payloads) from.  The kernels take it as a template parameter, so their
+// instance names (k_os_pass<false,prim::KeyArray,true>, which tests and profiles match) carry it.
 struct KeyArray {
   const uint64_t *keys;
   const uint32_t *pay;
@@ -207,33 +206,17 @@ __device__ __forceinline__ unsigned match_digit(uint32_t d) {
   return (m0 & m1 & m2) & (m3 & m4 & m5) & (m6 & m7);
 }
 
-// PPCSR_OS_MATCH_ATOMIC: the lanes holding the same digit find each other through ONE shared-memory atomicOr of their
-// lane bit into a per-warp, per-digit word (and one read back) instead of the eight ballots of match_digit: ~8
-// instead of ~36 instructions per key.  Keys-only passes (the extra 8 KB would cost a payload pass its fourth CTA).
-// Measured on B200 (C4, 100 M keys, six passes): 4.29 ms against 3.37 ms with the ballots -- three more shared-memory
-// operations per key cost more than the 28 ALU / vote instructions they replace.  Off.
-#ifndef PPCSR_OS_MATCH_ATOMIC
-#define PPCSR_OS_MATCH_ATOMIC 0
-#endif
-#ifndef PPCSR_OS_DPK  // keep the keys' digits in registers (four to a register) instead of extracting them three times
-#define PPCSR_OS_DPK 0
-#endif
-// PPCSR_OS_EARLY: the tile's digit histogram is taken by shared-memory atomics and published BEFORE the ranking phase
-// (the look-back of later tiles finds it sooner); 0: the counts fall out of the ranking and are published after it
-#ifndef PPCSR_OS_EARLY
-#define PPCSR_OS_EARLY 1
-#endif
 // dynamic shared memory of k_os_pass (bytes): keys[OS_TILE] u64 | pay[OS_TILE] u32 (HAS_PAY) |
-// cnt[OS_WARPS][OS_RADIX] u16 | goff[OS_RADIX] u32 | match[OS_WARPS][OS_RADIX] u32 (keys only)
+// cnt[OS_WARPS][OS_RADIX] u16 | goff[OS_RADIX] u32
 inline size_t os_pass_smem(bool has_pay) {
   return (size_t)OS_TILE * 8 + (has_pay ? (size_t)OS_TILE * 4 : 0) + (size_t)OS_WARPS * OS_RADIX * 2 +
-         (size_t)OS_RADIX * 4 + ((PPCSR_OS_MATCH_ATOMIC && !has_pay) ? (size_t)OS_WARPS * OS_RADIX * 4 : 0);
+         (size_t)OS_RADIX * 4;
 }
 
 // EARLY: the tile's digit counts are taken by shared-memory atomics and published before the ranking (see below);
 // !EARLY: they fall out of the ranking and are published after it -- measured faster for large batches (100 M keys:
 // 0.561 -> 0.545 ms per pass), slower for small ones (12.5 M: +3 %), so the host picks by batch size.
-template <bool HAS_PAY, class Src = KeyArray, bool EARLY = (PPCSR_OS_EARLY != 0)>
+template <bool HAS_PAY, class Src = KeyArray, bool EARLY = true>
 __global__ void __launch_bounds__(OS_THREADS, 4) k_os_pass(Src src, size_t n, DigitSel sel,
                                                            const uint32_t *__restrict__ gbase,
                                                            uint32_t *__restrict__ lookback, uint32_t *tile_counter,
@@ -244,14 +227,10 @@ __global__ void __launch_bounds__(OS_THREADS, 4) k_os_pass(Src src, size_t n, Di
   uint32_t *s_pay = reinterpret_cast<uint32_t *>(s_dyn + (size_t)OS_TILE * 8);
   uint16_t *s_cnt = reinterpret_cast<uint16_t *>(s_dyn + (size_t)OS_TILE * 8 + (HAS_PAY ? (size_t)OS_TILE * 4 : 0));
   uint32_t *s_goff = reinterpret_cast<uint32_t *>(s_cnt + OS_WARPS * OS_RADIX);
-  constexpr bool MATCH_ATOMIC = PPCSR_OS_MATCH_ATOMIC && !HAS_PAY;
-  uint32_t *s_match = s_goff + OS_RADIX;  // [OS_WARPS][OS_RADIX], MATCH_ATOMIC only
   __shared__ uint32_t s_warp[33];
   __shared__ uint32_t s_tile;
   if (threadIdx.x == 0) s_tile = atomicAdd(tile_counter, 1u);
   for (uint32_t d = threadIdx.x; d < OS_WARPS * OS_RADIX / 2; d += OS_THREADS) reinterpret_cast<uint32_t *>(s_cnt)[d] = 0;
-  if (MATCH_ATOMIC)
-    for (uint32_t d = threadIdx.x; d < OS_WARPS * OS_RADIX; d += OS_THREADS) s_match[d] = 0;
   s_goff[threadIdx.x] = 0;
   __syncthreads();
   const uint32_t tile = s_tile;
@@ -273,50 +252,22 @@ __global__ void __launch_bounds__(OS_THREADS, 4) k_os_pass(Src src, size_t n, Di
   // so that by the time this tile looks back most of its predecessors have already resolved their prefix
   static_assert(OS_THREADS == OS_RADIX, "one thread per digit");
   const uint32_t dg = threadIdx.x;
-#if PPCSR_OS_DPK
-  uint32_t dpk[OS_ITEMS / 4];  // the keys' digits, four to a register
-#endif
   uint32_t cnt = 0;
-  if (EARLY || PPCSR_OS_DPK) {
-#pragma unroll
-    for (int r = 0; r < OS_ITEMS; r++) {
-      const uint32_t d = sel_digit(k[r], sel);
-#if PPCSR_OS_DPK
-      if (r & 3) dpk[r >> 2] |= d << (8 * (r & 3));
-      else dpk[r >> 2] = d;
-#endif
-      if (EARLY) atomicAdd(&s_goff[d], 1u);
-    }
-  }
   if (EARLY) {
+#pragma unroll
+    for (int r = 0; r < OS_ITEMS; r++) atomicAdd(&s_goff[sel_digit(k[r], sel)], 1u);
     __syncthreads();
     // the padding keys of a partial last tile are counted in digit `mask`; nobody looks back through the last tile
     cnt = s_goff[dg];
     st_relaxed_gpu(lookback + (size_t)tile * OS_RADIX + dg, cnt | (tile == 0 ? OS_FLAG_INC : OS_FLAG_AGG));
   }
-  uint32_t *my_match = s_match + (size_t)w * OS_RADIX;
-  const uint32_t lbit = 1u << l;
 #pragma unroll
   for (int r = 0; r < OS_ITEMS; r++) {
-#if PPCSR_OS_DPK
-    const uint32_t d = (dpk[r >> 2] >> (8 * (r & 3))) & 0xFFu;
-#else
     const uint32_t d = sel_digit(k[r], sel);
-#endif
-    unsigned peers;
-    if (MATCH_ATOMIC) {
-      atomicOr(&my_match[d], lbit);
-      __syncwarp();
-      peers = *reinterpret_cast<volatile uint32_t *>(&my_match[d]);
-    } else {
-      peers = match_digit(d);
-    }
+    const unsigned peers = match_digit(d);
     const uint32_t base = my_cnt[d];
     __syncwarp();
-    if ((peers & lt) == 0) {
-      my_cnt[d] = (uint16_t)(base + __popc(peers));
-      if (MATCH_ATOMIC) my_match[d] = 0u;  // left clear for the next round
-    }
+    if ((peers & lt) == 0) my_cnt[d] = (uint16_t)(base + __popc(peers));
     __syncwarp();
     const uint32_t rk = base + __popc(peers & lt);
     if (r & 1) rank[r >> 1] |= rk << 16;
@@ -343,11 +294,7 @@ __global__ void __launch_bounds__(OS_THREADS, 4) k_os_pass(Src src, size_t n, Di
   // reorder the tile in shared memory: position = (digit base + warp offset) + rank inside the warp
 #pragma unroll
   for (int r = 0; r < OS_ITEMS; r++) {
-#if PPCSR_OS_DPK
-    const uint32_t d = (dpk[r >> 2] >> (8 * (r & 3))) & 0xFFu;
-#else
     const uint32_t d = sel_digit(k[r], sel);
-#endif
     const uint32_t rk = (r & 1) ? (rank[r >> 1] >> 16) : (rank[r >> 1] & 0xFFFFu);
     const uint32_t pos = my_cnt[d] + rk;
     s_keys[pos] = k[r];
@@ -522,16 +469,15 @@ inline int radix_sort_prepare(ppcsr_shard *s, size_t n, const SortPasses &P, uin
   return PPCSR_OK;
 }
 
-// Sorts n (key,payload) pairs by the key bits [0,lo_bits) and [32, 32+hi_bits).  The keys come from `src` (see
-// KeyArray); ka / kb (pa / pb) are the two buffer pairs the passes alternate between -- with a KeyArray source ka / pa
-// are its arrays, with a raw source ka / pa are scratch.  The sorted result ends up in *rk / *rp, which point at either
-// pair.  has_pay == false sorts keys only.
+// Sorts n (key,payload) pairs by the key bits [0,lo_bits) and [32, 32+hi_bits).  The keys (and payloads) are the
+// arrays ka / pa; ka / kb (pa / pb) are the two buffer pairs the passes alternate between.  The sorted result ends up in
+// *rk / *rp, which point at either pair.  pa == nullptr sorts keys only.
 // hist_done: the scratch was prepared (radix_sort_prepare, for at least n keys and this layout) and already holds the
 // digit histograms of this layout: no clearing, no k_os_hist.
-template <class Src>
-inline int radix_sort_from(ppcsr_shard *s, const Src &src, bool has_pay, uint64_t *ka, uint32_t *pa, uint64_t *kb,
-                           uint32_t *pb, size_t n, int lo_bits, int hi_bits, uint64_t **rk, uint32_t **rp,
-                           bool hist_done = false) {
+inline int radix_sort_pairs(ppcsr_shard *s, uint64_t *ka, uint32_t *pa, uint64_t *kb, uint32_t *pb, size_t n,
+                            int lo_bits, int hi_bits, uint64_t **rk, uint32_t **rp, bool hist_done = false) {
+  const bool has_pay = pa != nullptr;
+  const KeyArray src{ka, pa};
   *rk = ka;
   *rp = has_pay ? pa : nullptr;
   if (n == 0) return PPCSR_OK;
@@ -543,8 +489,8 @@ inline int radix_sort_from(ppcsr_shard *s, const Src &src, bool has_pay, uint64_
   if (n <= SS_MAX) {  // one CTA, one launch
     s->launches += 1;
     const uint32_t m = (uint32_t)n;
-    PPCSR_TRY(has_pay ? (sort_small_dispatch<true, Src>(s, src, m, P, kb, pb))
-                      : (sort_small_dispatch<false, Src>(s, src, m, P, kb, pb)));
+    PPCSR_TRY(has_pay ? (sort_small_dispatch<true, KeyArray>(s, src, m, P, kb, pb))
+                      : (sort_small_dispatch<false, KeyArray>(s, src, m, P, kb, pb)));
     CUDA_TRY(cudaGetLastError());
     *rk = kb;
     *rp = has_pay ? pb : nullptr;
@@ -559,16 +505,12 @@ inline int radix_sort_from(ppcsr_shard *s, const Src &src, bool has_pay, uint64_
   uint32_t *ghist = s->hist.p;
   uint32_t *counters = ghist + OS_MAX_PASSES * OS_RADIX;
   uint32_t *lookback = counters + 64;
-  {  // > 48 KB of dynamic shared memory needs an explicit opt-in: per device and source type, once, thread-safe
+  {  // > 48 KB of dynamic shared memory needs an explicit opt-in: per device, once, thread-safe
     static std::once_flag once[64];
     static cudaError_t once_err[64];
     const int dv = s->device & 63;
     std::call_once(once[dv], [&] {
-      once_err[dv] = cudaFuncSetAttribute(k_os_pass<true, Src>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)os_pass_smem(true));
-      if (once_err[dv] == cudaSuccess)
-        once_err[dv] = cudaFuncSetAttribute(k_os_pass<false, Src>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)os_pass_smem(false));
-      if (once_err[dv] == cudaSuccess)
-        once_err[dv] = cudaFuncSetAttribute(k_os_pass<true, KeyArray>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)os_pass_smem(true));
+      once_err[dv] = cudaFuncSetAttribute(k_os_pass<true, KeyArray>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)os_pass_smem(true));
       if (once_err[dv] == cudaSuccess)
         once_err[dv] = cudaFuncSetAttribute(k_os_pass<false, KeyArray>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)os_pass_smem(false));
       if (once_err[dv] == cudaSuccess)
@@ -580,25 +522,20 @@ inline int radix_sort_from(ppcsr_shard *s, const Src &src, bool has_pay, uint64_
   if (!hist_done) {
     const unsigned hblocks = (unsigned)std::min<size_t>((n + (size_t)OSH_THREADS * OSH_ITEMS - 1) / ((size_t)OSH_THREADS * OSH_ITEMS), 148 * 4);
     s->launches += 1;
-    k_os_hist<Src><<<hblocks, OSH_THREADS, 0, s->stream>>>(src, n, P, ghist);
+    k_os_hist<KeyArray><<<hblocks, OSH_THREADS, 0, s->stream>>>(src, n, P, ghist);
   }
   k_os_scan<<<P.n_pass, OS_RADIX, 0, s->stream>>>(ghist, lookback, rows);
   const bool late_counts = n >= OS_LATE_MIN_KEYS;  // keys-only passes of a large batch publish their counts after the ranking
-  // pass 0 reads the source and writes (kb, pb); the later passes alternate between the two buffer pairs
+  // the passes alternate between the two buffer pairs; pass 0 publishes its counts early whatever the batch size
   uint64_t *src_k = ka, *dst_k = kb;
   uint32_t *src_p = pa, *dst_p = pb;
   for (int p = 0; p < P.n_pass; p++) {
     const DigitSel sel = make_digit_sel(lo_bits, P.shift[p], P.mask[p]);
     uint32_t *gb = ghist + p * OS_RADIX, *lb = lookback + ((size_t)p * rows + OS_LB_DEPTH) * OS_RADIX;
-    if (p == 0) {
-      if (has_pay) k_os_pass<true, Src><<<(unsigned)ntiles, OS_THREADS, os_pass_smem(true), s->stream>>>(src, n, sel, gb, lb, counters + p, dst_k, dst_p);
-      else k_os_pass<false, Src><<<(unsigned)ntiles, OS_THREADS, os_pass_smem(false), s->stream>>>(src, n, sel, gb, lb, counters + p, dst_k, nullptr);
-    } else {
-      const KeyArray a{src_k, src_p};
-      if (has_pay) k_os_pass<true, KeyArray><<<(unsigned)ntiles, OS_THREADS, os_pass_smem(true), s->stream>>>(a, n, sel, gb, lb, counters + p, dst_k, dst_p);
-      else if (late_counts) k_os_pass<false, KeyArray, false><<<(unsigned)ntiles, OS_THREADS, os_pass_smem(false), s->stream>>>(a, n, sel, gb, lb, counters + p, dst_k, nullptr);
-      else k_os_pass<false, KeyArray><<<(unsigned)ntiles, OS_THREADS, os_pass_smem(false), s->stream>>>(a, n, sel, gb, lb, counters + p, dst_k, nullptr);
-    }
+    const KeyArray a{src_k, src_p};
+    if (has_pay) k_os_pass<true, KeyArray><<<(unsigned)ntiles, OS_THREADS, os_pass_smem(true), s->stream>>>(a, n, sel, gb, lb, counters + p, dst_k, dst_p);
+    else if (late_counts && p > 0) k_os_pass<false, KeyArray, false><<<(unsigned)ntiles, OS_THREADS, os_pass_smem(false), s->stream>>>(a, n, sel, gb, lb, counters + p, dst_k, nullptr);
+    else k_os_pass<false, KeyArray><<<(unsigned)ntiles, OS_THREADS, os_pass_smem(false), s->stream>>>(a, n, sel, gb, lb, counters + p, dst_k, nullptr);
     std::swap(src_k, dst_k);
     std::swap(src_p, dst_p);
   }
@@ -606,12 +543,6 @@ inline int radix_sort_from(ppcsr_shard *s, const Src &src, bool has_pay, uint64_
   *rk = src_k;
   *rp = has_pay ? src_p : nullptr;
   return PPCSR_OK;
-}
-
-// the keys (and payloads) are the arrays ka / pa themselves; pa == nullptr sorts keys only
-inline int radix_sort_pairs(ppcsr_shard *s, uint64_t *ka, uint32_t *pa, uint64_t *kb, uint32_t *pb, size_t n,
-                            int lo_bits, int hi_bits, uint64_t **rk, uint32_t **rp, bool hist_done = false) {
-  return radix_sort_from(s, KeyArray{ka, pa}, pa != nullptr, ka, pa, kb, pb, n, lo_bits, hi_bits, rk, rp, hist_done);
 }
 
 }  // namespace prim

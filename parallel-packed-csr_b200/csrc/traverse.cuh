@@ -14,7 +14,7 @@
 // than n_p entries.  Regions of n_p entries therefore cannot overflow, nothing is reset between levels, and no
 // atomic ever targets another GPU's memory.
 //
-// PageRank: every shard pushes into its own full-length fp64 accumulator (global dst ids, qry::k_pagerank_push*),
+// PageRank: every shard pushes into its own full-length fp64 accumulator (global dst ids, qry::k_pagerank_push_leaves),
 // then every owner sums its slice of all accumulators in the fixed shard order (k_group_pagerank_reduce): the
 // reduce-scatter is the only traffic between GPUs.
 #pragma once
