@@ -162,6 +162,21 @@ int ppcsr_remove_edge(ppcsr_shard *h, uint32_t src, uint32_t dst, int *found);
 int ppcsr_set_whole_array_policy(ppcsr_shard *h, int mode);
 /* reference PCSR::add_node (src/pcsr/PCSR.cpp:681-703): appends `count` vertices after the last one. */
 int ppcsr_add_nodes(ppcsr_shard *h, uint32_t count);
+/* Every edge out of or into the listed vertices removed (host ids < n); the vertices stay, without edges.  The result
+ * is that of ONE remove batch holding exactly the live edges (u, w) with u or w in the set (reference
+ * PCSR::remove_edge per edge, src/pcsr/PCSR.cpp:709-773): num_neighbors[u] drops by one per removed edge out of u (an
+ * isolated vertex keeps its old value minus its degree), edges to ids >= n are removed only with their source, n and
+ * the sentinels do not change.  For a shard holding the whole graph (as ppcsr_bfs): ids are that shard's vertex ids.
+ * Found on the device in one pass over the packed array (no edge reaches the host), then window selection and
+ * rebalance as after a batch.  Duplicate ids are allowed; count == 0 is a no-op with zeroed stats.  An id >= n returns
+ * PPCSR_ERR_ARG and a poisoned handle PPCSR_ERR_CAPACITY, both with nothing changed; everything the call needs (n / 8 B
+ * of bitmap and the id list, freed at the end, plus what a batch of removes needs) is allocated before the shard is
+ * modified, so PPCSR_ERR_CAPACITY also means "nothing removed".  A failure in the rebalance poisons the handle, as a
+ * batch does.  Stats (nullable; ppcsr_last_stats returns the same) as for a batch: batch_size = ids passed, n_unique =
+ * distinct ids, n_deleted = edges removed, the window / resize / rebalance fields as usual; ms_sort times the copy of
+ * the ids and the bitmap build, ms_locate the filter pass over the array.  A snapshot stays valid: ppcsr_restore
+ * brings back the graph before the isolation. */
+int ppcsr_isolate_vertices(ppcsr_shard *h, const uint32_t *ids, uint64_t count, ppcsr_batch_stats *stats);
 int ppcsr_last_stats(ppcsr_shard *h, ppcsr_batch_stats *stats);
 
 /* ---- multi-GPU routing helper (reference PPPCSR::get_partiton, src/pppcsr/PPPCSR.cpp:58-66) ---- */
@@ -230,7 +245,8 @@ int ppcsr_group_apply(ppcsr_group *g, const uint32_t *src, const uint32_t *dst, 
  * region_cap or a failed allocation returns PPCSR_ERR_CAPACITY with nothing in flight: everything the routing needs
  * is allocated in submit.  A failing wait reports the first failing shard, as ppcsr_group_apply does; the other batch
  * in flight stays valid and is applied by its own wait.  While a batch is in flight, ppcsr_group_apply,
- * ppcsr_group_bfs, ppcsr_group_pagerank and ppcsr_group_repartition return PPCSR_ERR_ARG and change nothing, and the
+ * ppcsr_group_bfs, ppcsr_group_pagerank, ppcsr_group_repartition and ppcsr_group_isolate_vertices return PPCSR_ERR_ARG
+ * and change nothing, and the
  * group's shards must not be modified through shard-level calls; ppcsr_group_destroy synchronises and frees the
  * batches in flight without applying them.  Ordering: a streamed batch is ordered after the group's last apply,
  * traversal or repartition and before the next, also when the shards run on external streams (ppcsr_set_stream).
@@ -285,6 +301,16 @@ typedef struct {
  * are freed (their sizes depend on the ranges).  Ordered after the group's last apply or traversal, before the next;
  * stats nullable. */
 int ppcsr_group_repartition(ppcsr_group *g, const uint64_t *new_starts, ppcsr_repartition_stats *stats);
+/* ppcsr_isolate_vertices over all shards of the group: GLOBAL ids < n (n counted as the traversals count it; a shard
+ * other than the last that no longer holds exactly its range gives PPCSR_ERR_ARG).  Every shard filters its own array
+ * with a bitmap of the n global ids on its device (n / 8 B each, freed at the end; only the id list is copied to each
+ * device, no edge crosses shards): the out-edges of a vertex are removed at its owner, its in-edges wherever they are.
+ * Checks and allocations for every shard come first, so PPCSR_ERR_ARG (bad id, a submitted batch in flight) and
+ * PPCSR_ERR_CAPACITY (a poisoned shard, no memory) leave the whole group unchanged.  Each shard then runs on its own
+ * host thread, ordered after the group's last apply, traversal or repartition, and before the next routed batch, also
+ * on external streams.  A failing shard is reported as ppcsr_group_apply reports one.  stats (nullable): one entry per
+ * shard, its n_deleted the edges removed from that shard. */
+int ppcsr_group_isolate_vertices(ppcsr_group *g, const uint32_t *ids, uint64_t count, ppcsr_batch_stats *stats);
 
 /* ---- reads ---- */
 int ppcsr_geometry_of(ppcsr_shard *h, ppcsr_geometry *out);

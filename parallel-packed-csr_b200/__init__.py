@@ -92,9 +92,11 @@ SYMBOLS = {
     "ppcsr_group_bfs": (_i, [_vp, _u32, _vp]),
     "ppcsr_group_pagerank": (_i, [_vp, _u32, C.c_double, _vp]),
     "ppcsr_group_repartition": (_i, [_vp, _vp, C.POINTER(RepartitionStats)]),
+    "ppcsr_group_isolate_vertices": (_i, [_vp, _vp, _u64, C.POINTER(BatchStats)]),
     "ppcsr_add_edge": (_i, [_vp, _u32, _u32, _u32]),
     "ppcsr_remove_edge": (_i, [_vp, _u32, _u32, C.POINTER(_i)]),
     "ppcsr_add_nodes": (_i, [_vp, _u32]),
+    "ppcsr_isolate_vertices": (_i, [_vp, _vp, _u64, C.POINTER(BatchStats)]),
     "ppcsr_last_stats": (_i, [_vp, C.POINTER(BatchStats)]),
     "ppcsr_bin_by_owner": (_i, [_i, _vp, _vp, _u32, _vp, _vp, _vp, _u64, _vp, _vp, _vp, _vp]),
     "ppcsr_bin_by_owner_packed": (_i, [_i, _vp, _vp, _u32, _vp, _vp, _vp, _u64, _vp, _vp, _vp]),
@@ -262,6 +264,14 @@ class Shard:
 
     def add_nodes(self, k=1):
         _check(self.L.ppcsr_add_nodes(self.h, k))
+
+    def isolate_vertices(self, ids) -> dict:
+        """Removes every edge out of or into the listed vertices (ppcsr_isolate_vertices); the vertices stay.  Ids
+        below n, duplicates allowed.  Returns the stats (n_deleted = edges removed)."""
+        ids = _u32_array(ids).reshape(-1)
+        st = BatchStats()
+        _check(self.L.ppcsr_isolate_vertices(self.h, _np_ptr(ids), ids.shape[0], C.byref(st)))
+        return st.as_dict()
 
     def reserve(self, max_slots=0, max_batch=0):
         _check(self.L.ppcsr_reserve(self.h, max_slots, max_batch))
@@ -521,6 +531,14 @@ class Group:
         _check(self.L.ppcsr_group_repartition(self.g, _np_ptr(new_starts), C.byref(st)))
         self.starts = new_starts.copy()
         return st.as_dict()
+
+    def isolate_vertices(self, ids) -> list[dict]:
+        """Removes every edge out of or into the listed GLOBAL vertices on every shard (ppcsr_group_isolate_vertices);
+        ids below self.n.  One stats dict per shard."""
+        ids = _u32_array(ids).reshape(-1)
+        st = (BatchStats * len(self.shards))()
+        _check(self.L.ppcsr_group_isolate_vertices(self.g, _np_ptr(ids), ids.shape[0], st))
+        return [x.as_dict() for x in st]
 
     def close(self):
         if getattr(self, "g", None):

@@ -10,6 +10,7 @@
 
 #include "batch.cuh"
 #include "common.cuh"
+#include "isolate.cuh"
 #include "migrate.cuh"
 #include "parse.cuh"
 #include "primitives.cuh"
@@ -405,7 +406,8 @@ int finish_batch_impl(ppcsr_shard *s, size_t list_cap, ppcsr_batch_stats *st) {
     return PPCSR_OK;
   }
   if (h.n_inserted == 0 && h.n_deleted == 0) {  // overwrites / misses only: nothing moves
-    for (int e = 3; e <= 6; e++) CUDA_TRY(cudaEventRecord(s->ev[e], s->stream));
+    // ev[4] last: finalize_stats waits for it alone and then reads every other event's time
+    for (int e : {3, 5, 6, 4}) CUDA_TRY(cudaEventRecord(s->ev[e], s->stream));
     st->n_windows = 0;
     return PPCSR_OK;
   }
@@ -733,6 +735,87 @@ int layout_stats(ppcsr_shard *s, ppcsr_batch_stats *st) {
 }
 
 bool submit_pending(const ppcsr_shard *s) { return s->pending[0].busy || s->pending[1].busy; }
+
+// ---- vertex isolation (isolate.cuh) ------------------------------------------------------------------------------
+// PPCSR_ERR_ARG unless every id is below n
+int isolate_check_ids(const uint32_t *ids, uint64_t count, uint64_t n, const char *who) {
+  for (uint64_t i = 0; i < count; i++) {
+    if (ids[i] >= n) {
+      g_ppcsr_error = std::string(who) + ": vertex id " + std::to_string(ids[i]) + " is not below n = " +
+                      std::to_string(n);
+      return PPCSR_ERR_ARG;
+    }
+  }
+  return PPCSR_OK;
+}
+
+struct IsolateBufs {
+  DevBuf<uint32_t> ids, bits;  // the id list on the shard's device, the bitmap of the n_bits vertex ids
+};
+void isolate_free(int device, IsolateBufs &b) {
+  cudaSetDevice(device);
+  dev_free(b.ids);
+  dev_free(b.bits);
+}
+
+// Everything an isolation of `count` ids over n_bits vertex ids needs, allocated before the shard is modified: the id
+// list and the bitmap, what a batch of removes can need (reserve_worst_case), and the window list at its largest (every
+// leaf touched), the list_cap isolate_run hands to finish_batch.  The insert list stays empty but must exist: the
+// rebalance kernels take its pointers.
+int isolate_reserve(ppcsr_shard *s, uint64_t count, uint64_t n_bits, IsolateBufs *b) {
+  PPCSR_TRY(set_device(s));
+  PPCSR_TRY(dev_reserve(b->ids, count, s->stream));
+  PPCSR_TRY(dev_reserve(b->bits, (size_t)((n_bits + 31) / 32), s->stream));
+  PPCSR_TRY(reserve_worst_case(s, 0));
+  PPCSR_TRY(reserve_window_arrays(s, s->geo.n_leaves));
+  PPCSR_TRY(dev_reserve(s->ins_dst, 1, s->stream));
+  PPCSR_TRY(dev_reserve(s->ins_val, 1, s->stream));
+  PPCSR_TRY(dev_reserve(s->ins_pred, 1, s->stream));
+  return PPCSR_OK;
+}
+
+// Removes every edge of the shard whose source (vertex_offset + local id) or destination (if < n_bits) is one of the
+// ids (host array, every id < n_bits), then runs the back half of a batch.  isolate_reserve first.  Stats as for a
+// batch: ms_sort = copy of the ids + bitmap, ms_locate = the filter pass.
+int isolate_run(ppcsr_shard *s, const uint32_t *ids, uint64_t count, uint64_t vertex_offset, uint64_t n_bits,
+                IsolateBufs &b, ppcsr_batch_stats *stats) {
+  PPCSR_TRY(set_device(s));
+  const Geometry g = s->geo;
+  ppcsr_batch_stats st{};
+  st.batch_size = count;
+  st.slots_before = st.slots_after = g.N;
+  BatchScalars *sc = s->d_scalars;
+  CUDA_TRY(cudaMemsetAsync(sc, 0, sizeof(BatchScalars), s->stream));
+  s->all_touched = 0;
+  CUDA_TRY(cudaEventRecord(s->ev[0], s->stream));
+  s->launches = 2;  // bitmap, filter
+  CUDA_TRY(cudaMemcpyAsync(b.ids.p, ids, count * sizeof(uint32_t), cudaMemcpyHostToDevice, s->stream));
+  CUDA_TRY(cudaMemsetAsync(b.bits.p, 0, (size_t)((n_bits + 31) / 32) * sizeof(uint32_t), s->stream));
+  iso::k_isolate_bitmap<<<std::min<unsigned>(div_up(count, iso::IT), 148 * 8), iso::IT, 0, s->stream>>>(
+      b.ids.p, count, b.bits.p, sc);
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaEventRecord(s->ev[1], s->stream));
+  if (!s->cnt_clean) {
+    CUDA_TRY(cudaMemsetAsync(s->ins_cnt.p, 0, (size_t)g.n_leaves * sizeof(uint32_t), s->stream));
+    CUDA_TRY(cudaMemsetAsync(s->del_cnt.p, 0, (size_t)g.n_leaves * sizeof(uint32_t), s->stream));
+  }
+  s->cnt_clean = false;
+  s->last_sparse = false;
+  s->ins_uniform_val = 0;
+  if (s->n) {
+    const unsigned blocks = std::min<unsigned>(div_up(g.N, (uint64_t)iso::IT * iso::FL_BATCH), 148 * 16);
+    iso::k_isolate_filter<<<blocks, iso::IT, 0, s->stream>>>(s->dest.p, s->val.p, s->leaf_cnt.p, s->beg.p, s->nn.p,
+                                                            s->del_cnt.p, g.leaf_shift, s->n, g.N, b.bits.p,
+                                                            (uint32_t)n_bits, (uint32_t)vertex_offset, sc);
+  }
+  CUDA_TRY(cudaGetLastError());
+  CUDA_TRY(cudaEventRecord(s->ev[2], s->stream));
+  // no more than one window per leaf: isolate_reserve sized the window list for that
+  PPCSR_TRY(finish_batch(s, g.n_leaves, &st));
+  PPCSR_TRY(finalize_stats(s, &st));
+  if (stats) *stats = st;
+  return PPCSR_OK;
+}
 
 }  // namespace
 
@@ -1391,6 +1474,25 @@ int ppcsr_add_nodes(ppcsr_shard *s, uint32_t count) {
   reb::k_set_u32<<<1, 1, 0, s->stream>>>(s->beg.p + s->n, (uint32_t)s->geo.N);
   PPCSR_TRY(finalize_stats(s, &st));
   return PPCSR_OK;
+}
+
+int ppcsr_isolate_vertices(ppcsr_shard *s, const uint32_t *ids, uint64_t count, ppcsr_batch_stats *stats) {
+  if (!s || (count && !ids)) return PPCSR_ERR_ARG;
+  PPCSR_TRY(set_device(s));
+  PPCSR_TRY(isolate_check_ids(ids, count, s->n, "ppcsr_isolate_vertices"));
+  if (count == 0) {
+    ppcsr_batch_stats st{};
+    st.slots_before = st.slots_after = s->geo.N;
+    s->last = st;
+    if (stats) *stats = st;
+    return PPCSR_OK;
+  }
+  if (s->poisoned) return poisoned_error();
+  IsolateBufs b;
+  int rc = isolate_reserve(s, count, s->n, &b);
+  if (rc == PPCSR_OK) rc = isolate_run(s, ids, count, 0, s->n, b, stats);
+  isolate_free(s->device, b);
+  return rc;
 }
 
 int ppcsr_set_whole_array_policy(ppcsr_shard *s, int mode) {
