@@ -179,6 +179,42 @@ int ppcsr_add_nodes(ppcsr_shard *h, uint32_t count);
 int ppcsr_isolate_vertices(ppcsr_shard *h, const uint32_t *ids, uint64_t count, ppcsr_batch_stats *stats);
 int ppcsr_last_stats(ppcsr_shard *h, ppcsr_batch_stats *stats);
 
+/* ---- change capture: what each batch changed, left on the device ----
+ * Off by default, per shard; while it is off a batch runs exactly as without this feature (same kernels, no extra
+ * allocation, launch or host synchronisation).  While it is on, every batch -- ppcsr_apply_batch[_device|_pairs|
+ * _packed_device|_segments_device], ppcsr_wait, ppcsr_group_apply / ppcsr_group_wait on each shard, ppcsr_add_edge /
+ * ppcsr_remove_edge (batches of one) -- leaves two lists in the shard's device memory, valid until the next call that
+ * modifies the shard:
+ *   changes    one entry per key whose state the batch changed, ascending (src, dst); src is shard-local.  old_val = 0:
+ *              absent before the batch (inserted); new_val = 0: absent after it (deleted); both non-zero: overwritten,
+ *              also with the same value.  A key absent before and after (e.g. insert then remove of a new edge) is not
+ *              listed.  n_changes = n_inserted + n_overwritten + n_deleted of the batch's stats, per kind as well.
+ *   not found  one (src, dst) per remove CALL that missed under the sequential rule of n_not_found (a remove of an
+ *              absent edge, or right after a remove of the same key), ascending, a key repeated once per miss:
+ *              n_not_found entries, as a multiset the `not found s d` lines the reference prints at -threads=1
+ *              (reference PCSR.cpp:751).
+ * Ignored updates (src >= n, dst == 0xFFFFFFFF) appear in neither list.  Both lists are empty after a failed call
+ * (any status), an empty batch, and every modifying call that is not a batch: ppcsr_isolate_vertices /
+ * ppcsr_group_isolate_vertices, ppcsr_load_csr, ppcsr_add_nodes, ppcsr_restore, ppcsr_group_repartition.
+ * Applying (src, dst, val = old_val) of the changes as one batch restores the edges and values before the batch (not
+ * num_neighbors, which keeps its call-count meaning).
+ * Memory while on: about 29 B per update of the largest batch (a kind byte and an old value per update, 16 B per
+ * change entry and 8 B per not-found entry, each list bounded by the batch), reserved with the batch's other worst-case
+ * buffers before the shard is modified, so PPCSR_ERR_CAPACITY still means "nothing applied".  Turning capture off
+ * frees it. */
+int ppcsr_set_change_capture(ppcsr_shard *h, int on);
+typedef struct {
+  const uint32_t *src, *dst, *old_val, *new_val; /* DEVICE pointers on `device`, n_changes entries each (NULL if 0) */
+  uint64_t n_changes;
+  const uint32_t *nf_src, *nf_dst;               /* DEVICE pointers, n_not_found entries each (NULL if 0)           */
+  uint64_t n_not_found;
+  int device;
+} ppcsr_changes;
+/* The lists of the last batch (PPCSR_ERR_ARG while capture is off).  The pointers belong to the shard: read them with
+ * ppcsr_copy_to_host or on the device, and copy them before passing them back into the same shard -- the next batch
+ * may reallocate or overwrite them. */
+int ppcsr_last_changes(ppcsr_shard *h, ppcsr_changes *out);
+
 /* ---- multi-GPU routing helper (reference PPPCSR::get_partiton, src/pppcsr/PPPCSR.cpp:58-66) ---- */
 /* Bins `count` device-resident updates by owning shard: shard p owns sources [starts[p], starts[p+1]).
  * Writes the updates grouped by owner (stable) with src made shard-local (src - starts[owner],

@@ -45,6 +45,12 @@ class RepartitionStats(C.Structure):
         return {n: getattr(self, n) for n, _ in self._fields_}
 
 
+class Changes(C.Structure):
+    _fields_ = [("src", C.c_void_p), ("dst", C.c_void_p), ("old_val", C.c_void_p), ("new_val", C.c_void_p),
+                ("n_changes", C.c_uint64), ("nf_src", C.c_void_p), ("nf_dst", C.c_void_p), ("n_not_found", C.c_uint64),
+                ("device", C.c_int)]
+
+
 class Geometry(C.Structure):
     _fields_ = [("N", C.c_uint64), ("logN", C.c_uint32), ("H", C.c_uint32), ("n", C.c_uint64), ("items", C.c_uint64)]
 
@@ -98,6 +104,8 @@ SYMBOLS = {
     "ppcsr_add_nodes": (_i, [_vp, _u32]),
     "ppcsr_isolate_vertices": (_i, [_vp, _vp, _u64, C.POINTER(BatchStats)]),
     "ppcsr_last_stats": (_i, [_vp, C.POINTER(BatchStats)]),
+    "ppcsr_set_change_capture": (_i, [_vp, _i]),
+    "ppcsr_last_changes": (_i, [_vp, C.POINTER(Changes)]),
     "ppcsr_bin_by_owner": (_i, [_i, _vp, _vp, _u32, _vp, _vp, _vp, _u64, _vp, _vp, _vp, _vp]),
     "ppcsr_bin_by_owner_packed": (_i, [_i, _vp, _vp, _u32, _vp, _vp, _vp, _u64, _vp, _vp, _vp]),
     "ppcsr_apply_batch_packed_device": (_i, [_vp, _vp, _vp, _u64, _u32, C.POINTER(BatchStats)]),
@@ -272,6 +280,32 @@ class Shard:
         st = BatchStats()
         _check(self.L.ppcsr_isolate_vertices(self.h, _np_ptr(ids), ids.shape[0], C.byref(st)))
         return st.as_dict()
+
+    def set_change_capture(self, on: bool = True):
+        """Turns change capture on or off (ppcsr_set_change_capture): with it on, every batch leaves the lists that
+        last_changes() returns."""
+        _check(self.L.ppcsr_set_change_capture(self.h, 1 if on else 0))
+
+    def last_changes_device(self) -> Changes:
+        """The raw ppcsr_changes of the last batch: device pointers on self.device, valid until the next call that
+        modifies the shard."""
+        c = Changes()
+        _check(self.L.ppcsr_last_changes(self.h, C.byref(c)))
+        return c
+
+    def last_changes(self) -> dict:
+        """What the last batch changed (ppcsr_last_changes), copied to the host: src, dst, old_val, new_val (one entry
+        per changed key, ascending; old_val 0 = inserted, new_val 0 = deleted) and nf_src, nf_dst (one entry per
+        remove that missed, ascending), all uint32 numpy arrays; src and nf_src are shard-local."""
+        c = self.last_changes_device()
+        out = {}
+        for name, n in (("src", c.n_changes), ("dst", c.n_changes), ("old_val", c.n_changes), ("new_val", c.n_changes),
+                        ("nf_src", c.n_not_found), ("nf_dst", c.n_not_found)):
+            a = np.zeros(n, dtype=np.uint32)
+            if n:
+                _check(self.L.ppcsr_copy_to_host(c.device, _np_ptr(a), getattr(c, name), n * 4))
+            out[name] = a
+        return out
 
     def reserve(self, max_slots=0, max_batch=0):
         _check(self.L.ppcsr_reserve(self.h, max_slots, max_batch))
@@ -531,6 +565,20 @@ class Group:
         _check(self.L.ppcsr_group_repartition(self.g, _np_ptr(new_starts), C.byref(st)))
         self.starts = new_starts.copy()
         return st.as_dict()
+
+    def set_change_capture(self, on: bool = True):
+        """Change capture on every shard (Shard.set_change_capture)."""
+        for s in self.shards:
+            s.set_change_capture(on)
+
+    def last_changes(self) -> dict:
+        """What the last routed batch changed, over all shards: each shard's lists (Shard.last_changes) with src and
+        nf_src made global by adding the shard's first vertex, concatenated in shard order -- still ascending."""
+        parts = [s.last_changes() for s in self.shards]
+        for r, p in enumerate(parts):
+            for k in ("src", "nf_src"):
+                p[k] = (p[k].astype(np.uint64) + np.uint64(self.starts[r])).astype(np.uint32)
+        return {k: np.concatenate([p[k] for p in parts]) for k in parts[0]}
 
     def isolate_vertices(self, ids) -> list[dict]:
         """Removes every edge out of or into the listed GLOBAL vertices on every shard (ppcsr_group_isolate_vertices);

@@ -454,17 +454,24 @@ __device__ __forceinline__ bool find_fast(const LocSmem &S, const uint32_t *__re
 // of its instructions on an insert batch.
 // DELONLY: the mirror image -- no values, no op bit, value 0: every update is a remove (no insert counts, no insert
 // list; a remove misses iff the edge is absent or the previous update of the batch removed the same key).
-template <bool SPARSE, bool INSONLY = false, bool DELONLY = false>
-__global__ void __launch_bounds__(LT, 8) k_locate(const uint64_t *__restrict__ keys, const uint32_t *__restrict__ pay,
-                                               uint32_t default_val, size_t count, uint64_t invalid_key,
-                                               const uint32_t *__restrict__ dest, uint32_t *__restrict__ val,
-                                               const uint32_t *__restrict__ leaf_cnt, const uint32_t *__restrict__ beg,
-                                               uint32_t ls, uint32_t n_slots, uint32_t *__restrict__ nn,
-                                               uint32_t *__restrict__ tile_dst, uint32_t *__restrict__ tile_val,
-                                               uint32_t *__restrict__ tile_pred, uint32_t *__restrict__ tile_cnt,
-                                               uint32_t *__restrict__ ins_cnt, uint32_t *__restrict__ del_cnt,
-                                               uint32_t op_bit, BatchScalars *sc, uint32_t *touched,
-                                               uint32_t *touch_stamp, uint32_t touch_epoch, uint32_t dst_mask) {
+// CAPTURE (k_locate_capture, ppcsr_set_change_capture): every sorted update also leaves its outcome for the change
+// lists -- cap_kind[i] = CAP_* class of a winner (0: not a winner, a miss or ignored) | misses of this update << 2, and
+// cap_old[i] = the value the winner's overwrite or tombstone replaced.  Misses follow the sequential rule counted in
+// n_not_found: a remove right after a remove of the same key (miss_dup, on that update) and a run whose first op is a
+// remove of an absent key (miss_first, on the winner), so an update carries 0, 1 or 2 of them.
+enum : uint8_t { CAP_INSERT = 1, CAP_OVERWRITE = 2, CAP_DELETE = 3 };
+template <bool SPARSE, bool INSONLY, bool DELONLY, bool CAPTURE>
+__device__ __forceinline__ void locate_tile(const uint64_t *__restrict__ keys, const uint32_t *__restrict__ pay,
+                                            uint32_t default_val, size_t count, uint64_t invalid_key,
+                                            const uint32_t *__restrict__ dest, uint32_t *__restrict__ val,
+                                            const uint32_t *__restrict__ leaf_cnt, const uint32_t *__restrict__ beg,
+                                            uint32_t ls, uint32_t n_slots, uint32_t *__restrict__ nn,
+                                            uint32_t *__restrict__ tile_dst, uint32_t *__restrict__ tile_val,
+                                            uint32_t *__restrict__ tile_pred, uint32_t *__restrict__ tile_cnt,
+                                            uint32_t *__restrict__ ins_cnt, uint32_t *__restrict__ del_cnt,
+                                            uint32_t op_bit, BatchScalars *sc, uint32_t *touched,
+                                            uint32_t *touch_stamp, uint32_t touch_epoch, uint32_t dst_mask,
+                                            uint8_t *__restrict__ cap_kind, uint32_t *__restrict__ cap_old) {
   // Small-batch path (SPARSE, sparse.cuh): the batch was sorted on a SPECULATED dst width (no host round
   // trip after the key builder); a dst beyond it means the order is wrong -- leave before anything is modified, the
   // host runs the batch again the general way.  The first update to reach a leaf appends it to the touched list.
@@ -595,6 +602,7 @@ __global__ void __launch_bounds__(LT, 8) k_locate(const uint64_t *__restrict__ k
             hit = mode == 3u ? find_tab(S.tab.first, S.tab.cnt8, wa >> ls, dest, vb[r], ve[r], ls, d, &slot)
                              : find_in(D, doff, C, coff, vb[r], ve[r], true, ls, d, &slot);
           }
+          if (CAPTURE && hit) cap_old[i] = val[slot];
           if (INSONLY || (!DELONLY && v != 0)) {
             cls = hit ? CLS_OVERWRITE : CLS_INSERT;
             if (hit) val[slot] = v;  // duplicate insert overwrites the value (reference PCSR.cpp:529-532)
@@ -612,6 +620,8 @@ __global__ void __launch_bounds__(LT, 8) k_locate(const uint64_t *__restrict__ k
           }
         }
       }
+      if (CAPTURE)
+        cap_kind[i] = (uint8_t)((cls < CLS_MISS ? cls + 1u : 0u) | ((uint32_t)miss_dup + (uint32_t)miss_first) << 2);
     }
     // call counts: one atomic per run of equal sources inside the warp
     {
@@ -705,6 +715,76 @@ __global__ void __launch_bounds__(LT, 8) k_locate(const uint64_t *__restrict__ k
     tile_pred[base + x] = S.o_pred[x];
   }
 }
+
+#define PPCSR_LOCATE_PARAMS                                                                                            \
+  const uint64_t *__restrict__ keys, const uint32_t *__restrict__ pay, uint32_t default_val, size_t count,             \
+      uint64_t invalid_key, const uint32_t *__restrict__ dest, uint32_t *__restrict__ val,                             \
+      const uint32_t *__restrict__ leaf_cnt, const uint32_t *__restrict__ beg, uint32_t ls, uint32_t n_slots,          \
+      uint32_t *__restrict__ nn, uint32_t *__restrict__ tile_dst, uint32_t *__restrict__ tile_val,                     \
+      uint32_t *__restrict__ tile_pred, uint32_t *__restrict__ tile_cnt, uint32_t *__restrict__ ins_cnt,               \
+      uint32_t *__restrict__ del_cnt, uint32_t op_bit, BatchScalars *sc, uint32_t *touched, uint32_t *touch_stamp,     \
+      uint32_t touch_epoch, uint32_t dst_mask
+#define PPCSR_LOCATE_ARGS                                                                                              \
+  keys, pay, default_val, count, invalid_key, dest, val, leaf_cnt, beg, ls, n_slots, nn, tile_dst, tile_val,           \
+      tile_pred, tile_cnt, ins_cnt, del_cnt, op_bit, sc, touched, touch_stamp, touch_epoch, dst_mask
+template <bool SPARSE, bool INSONLY = false, bool DELONLY = false>
+__global__ void __launch_bounds__(LT, 8) k_locate(PPCSR_LOCATE_PARAMS) {
+  locate_tile<SPARSE, INSONLY, DELONLY, false>(PPCSR_LOCATE_ARGS, nullptr, nullptr);
+}
+// the same with change capture: a kernel of its own, so that the instantiations above stay what they were
+template <bool SPARSE, bool INSONLY = false, bool DELONLY = false>
+__global__ void __launch_bounds__(LT, 8) k_locate_capture(PPCSR_LOCATE_PARAMS, uint8_t *__restrict__ cap_kind,
+                                                          uint32_t *__restrict__ cap_old) {
+  locate_tile<SPARSE, INSONLY, DELONLY, true>(PPCSR_LOCATE_ARGS, cap_kind, cap_old);
+}
+#undef PPCSR_LOCATE_PARAMS
+#undef PPCSR_LOCATE_ARGS
+
+// ---- the change lists of a batch (ppcsr_last_changes), compacted from k_locate_capture's kind bytes in key order by
+// two device scans: one for the changes, one for the misses (an update can carry two misses, and each scan sums one
+// 32-bit count per element).  `skip`: the small-batch path's abort flag -- k_locate left before writing a kind byte,
+// and the batch runs again the general way.
+struct InCapChange {
+  const uint8_t *kind;
+  const unsigned int *skip;
+  __device__ uint32_t operator()(size_t i) const { return *skip ? 0u : (kind[i] & 3u) != 0u; }
+};
+struct InCapMiss {
+  const uint8_t *kind;
+  const unsigned int *skip;
+  __device__ uint32_t operator()(size_t i) const { return *skip ? 0u : (uint32_t)kind[i] >> 2; }
+};
+struct OutCapChange {
+  const uint64_t *keys;
+  const uint32_t *pay;  // nullptr: every insert of the batch carries default_val
+  const uint8_t *kind;
+  const uint32_t *old;
+  uint64_t km;          // strips the op bit
+  uint32_t default_val;
+  uint32_t *src, *dst, *old_val, *new_val;
+  __device__ void operator()(size_t i, uint32_t at, uint32_t own) const {
+    if (!own) return;
+    const uint64_t k = keys[i] & km;
+    const uint32_t c = kind[i] & 3u;
+    src[at] = (uint32_t)(k >> 32);
+    dst[at] = (uint32_t)k;
+    old_val[at] = c == CAP_INSERT ? 0u : old[i];
+    new_val[at] = c == CAP_DELETE ? 0u : pay ? pay[i] : default_val;
+  }
+};
+struct OutCapMiss {
+  const uint64_t *keys;
+  uint64_t km;
+  uint32_t *src, *dst;
+  __device__ void operator()(size_t i, uint32_t at, uint32_t own) const {
+    if (!own) return;
+    const uint64_t k = keys[i] & km;
+    for (uint32_t j = 0; j < own; j++) {
+      src[at + j] = (uint32_t)(k >> 32);
+      dst[at + j] = (uint32_t)k;
+    }
+  }
+};
 
 // the tiles' insert runs, moved to their place in the global key-ordered insert list (tile_off = exclusive scan of the
 // tile counts)

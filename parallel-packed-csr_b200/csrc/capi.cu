@@ -238,6 +238,34 @@ int reserve_worst_case(ppcsr_shard *s, uint64_t count) {
   const size_t scan_tiles = (size_t)div_up(std::max<uint64_t>(std::max<uint64_t>(g2.n_leaves, count), 1), prim::SCAN_TILE) + 2;
   PPCSR_TRY(dev_reserve(s->block_tmp, scan_tiles, s->stream));
   PPCSR_TRY(prim::reserve_scan_state(s, std::max<size_t>(scan_tiles, (size_t)div_up(count, batch::LTILE) + 2)));
+  if (s->capture) {  // the kind bytes, old values and both lists: each is bounded by the batch (29 B per update)
+    PPCSR_TRY(dev_reserve(s->cap_kind, count, s->stream));
+    PPCSR_TRY(dev_reserve(s->cap_old, count, s->stream));
+    for (DevBuf<uint32_t> *b : {&s->chg_src, &s->chg_dst, &s->chg_old, &s->chg_new, &s->nf_src, &s->nf_dst})
+      PPCSR_TRY(dev_reserve(*b, count, s->stream));
+  }
+  return PPCSR_OK;
+}
+
+// Every call that modifies the shard starts here: the change lists describe the last successful batch only.
+void changes_clear(ppcsr_shard *s) { s->n_changes = s->n_nf = 0; }
+void changes_set(ppcsr_shard *s, const ppcsr_batch_stats &st) {
+  s->n_changes = st.n_inserted + st.n_overwritten + st.n_deleted;
+  s->n_nf = st.n_not_found;
+}
+
+// The change lists of the batch k_locate_capture just classified (keys / pay: the sorted batch, still in place).
+// Nothing is read back: their lengths are the class counts the batch reads anyway.
+int capture_compact(ppcsr_shard *s, const uint64_t *keys, const uint32_t *pay, uint32_t op_bit, uint32_t default_val,
+                    uint64_t count) {
+  const uint64_t km = op_bit ? ~batch::KEY_OP_BIT : ~0ull;
+  const unsigned int *skip = &s->d_scalars->sparse_abort;
+  PPCSR_TRY(prim::device_scan(s, batch::InCapChange{s->cap_kind.p, skip},
+                              batch::OutCapChange{keys, pay, s->cap_kind.p, s->cap_old.p, km, default_val, s->chg_src.p,
+                                                  s->chg_dst.p, s->chg_old.p, s->chg_new.p},
+                              count, nullptr, nullptr));
+  PPCSR_TRY(prim::device_scan(s, batch::InCapMiss{s->cap_kind.p, skip},
+                              batch::OutCapMiss{keys, km, s->nf_src.p, s->nf_dst.p}, count, nullptr, nullptr));
   return PPCSR_OK;
 }
 int poisoned_error() {
@@ -889,6 +917,8 @@ void ppcsr_destroy(ppcsr_shard *s) {
   dev_free(s->block_tmp); dev_free(s->hist); dev_free(s->pr_acc); dev_free(s->misc);
   dev_free(s->scan_state); dev_free(s->scan_ticket); dev_free(s->tile_cnt);
   dev_free(s->touch_stamp); dev_free(s->touched_flags);
+  dev_free(s->cap_kind); dev_free(s->cap_old); dev_free(s->chg_src); dev_free(s->chg_dst); dev_free(s->chg_old);
+  dev_free(s->chg_new); dev_free(s->nf_src); dev_free(s->nf_dst);
   dev_free(s->snap.dest); dev_free(s->snap.val); dev_free(s->snap.leaf_cnt); dev_free(s->snap.tree);
   dev_free(s->snap.beg); dev_free(s->snap.nn);
   for (auto &P : s->pending) {
@@ -975,6 +1005,7 @@ static int apply_device_common(ppcsr_shard *s, const uint32_t *d_src, const uint
                                const batch::SegmentTable *segments = nullptr, bool pairs = false,
                                bool no_sparse = false) {
   PPCSR_TRY(set_device(s));
+  changes_clear(s);
   ppcsr_batch_stats st{};
   st.batch_size = count;
   st.slots_before = st.slots_after = s->geo.N;
@@ -1140,7 +1171,23 @@ static int apply_device_common(ppcsr_shard *s, const uint32_t *d_src, const uint
         (uint32_t)g.N, s->nn.p, t_dst, t_val, t_pred, s->tile_cnt.p, s->ins_cnt.p, s->del_cnt.p, op_bit, sc, touched,
         stamp, epoch, dst_mask);
   };
-  if (sparse) {
+  // with change capture: the same kernel plus the per-update outcome (batch::k_locate_capture)
+  auto locate_cap = [&](auto kernel, uint32_t *touched, uint32_t *stamp, uint32_t epoch) {
+    kernel<<<lblocks, batch::LT, sizeof(batch::LocSmem), s->stream>>>(
+        keys, pay, default_val, count, invalid_key, s->dest.p, s->val.p, s->leaf_cnt.p, s->beg.p, g.leaf_shift,
+        (uint32_t)g.N, s->nn.p, t_dst, t_val, t_pred, s->tile_cnt.p, s->ins_cnt.p, s->del_cnt.p, op_bit, sc, touched,
+        stamp, epoch, dst_mask, s->cap_kind.p, s->cap_old.p);
+  };
+  if (s->capture) {
+    if (sparse) {
+      if (ins_only) locate_cap(batch::k_locate_capture<true, true>, s->touched.p, s->touch_stamp.p, s->touch_epoch);
+      else locate_cap(batch::k_locate_capture<true, false>, s->touched.p, s->touch_stamp.p, s->touch_epoch);
+    } else {
+      if (ins_only) locate_cap(batch::k_locate_capture<false, true>, nullptr, nullptr, 0u);
+      else if (del_only) locate_cap(batch::k_locate_capture<false, false, true>, nullptr, nullptr, 0u);
+      else locate_cap(batch::k_locate_capture<false, false>, nullptr, nullptr, 0u);
+    }
+  } else if (sparse) {
     if (ins_only) locate(batch::k_locate<true, true>, s->touched.p, s->touch_stamp.p, s->touch_epoch);
     else locate(batch::k_locate<true, false>, s->touched.p, s->touch_stamp.p, s->touch_epoch);
   } else {
@@ -1155,6 +1202,8 @@ static int apply_device_common(ppcsr_shard *s, const uint32_t *d_src, const uint
     batch::k_gather_inserts<<<div_up(lblocks, batch::GATHER_TILES), batch::LT, 0, s->stream>>>(
         tile_dst, tile_val, s->uloc.p, s->tile_cnt.p, s->ins_dst.p, s->ins_val.p, s->ins_pred.p, sc, lblocks);
   }
+  // the change lists, while the sorted batch is still in place (counted in ms_locate)
+  if (s->capture) PPCSR_TRY(capture_compact(s, keys, pay, op_bit, default_val, count));
   if (stage_ev) CUDA_TRY(cudaEventRecord(s->ev[2], s->stream));
   if (sparse) {
     // 5s. tree, windows and rebalance of the small-batch path, then the ONE host synchronisation of the batch
@@ -1211,6 +1260,7 @@ static int apply_device_common(ppcsr_shard *s, const uint32_t *d_src, const uint
       s->last_sparse = true;
       s->last_touched = (uint32_t)h.n_touched;
       PPCSR_TRY(finalize_stats(s, &st, stage_ev));
+      if (s->capture) changes_set(s, st);
       if (stats) *stats = st;
       return PPCSR_OK;
     }
@@ -1228,18 +1278,21 @@ static int apply_device_common(ppcsr_shard *s, const uint32_t *d_src, const uint
   // 5. windows + rebalance
   PPCSR_TRY(finish_batch(s, count, &st));
   PPCSR_TRY(finalize_stats(s, &st));
+  if (s->capture) changes_set(s, st);
   if (stats) *stats = st;
   return PPCSR_OK;
 }
 
 int ppcsr_apply_batch_device(ppcsr_shard *s, const uint32_t *d_src, const uint32_t *d_dst, const uint32_t *d_val,
                              uint64_t count, uint32_t default_val, ppcsr_batch_stats *stats) {
+  if (s) changes_clear(s);
   if (!s || (count && (!d_src || !d_dst))) return PPCSR_ERR_ARG;
   return apply_device_common(s, d_src, d_dst, nullptr, d_val, count, default_val, stats);
 }
 
 int ppcsr_apply_batch_packed_device(ppcsr_shard *s, const uint64_t *d_packed, const uint32_t *d_val, uint64_t count,
                                     uint32_t default_val, ppcsr_batch_stats *stats) {
+  if (s) changes_clear(s);
   if (!s || (count && !d_packed)) return PPCSR_ERR_ARG;
   return apply_device_common(s, nullptr, nullptr, d_packed, d_val, count, default_val, stats);
 }
@@ -1247,6 +1300,7 @@ int ppcsr_apply_batch_packed_device(ppcsr_shard *s, const uint64_t *d_packed, co
 int ppcsr_apply_batch_segments_device(ppcsr_shard *s, const uint64_t *d_packed, const uint32_t *d_val,
                                       uint64_t region_cap, const uint64_t *d_counts, uint32_t n_segments,
                                       uint64_t max_total, uint32_t default_val, ppcsr_batch_stats *stats) {
+  if (s) changes_clear(s);
   if (!s || !d_counts || !d_packed || n_segments == 0 || n_segments > batch::BIN_MAX_PARTS) return PPCSR_ERR_ARG;
   batch::SegmentTable T{};
   T.n_seg = n_segments;
@@ -1261,6 +1315,7 @@ int ppcsr_apply_batch_segments_device(ppcsr_shard *s, const uint64_t *d_packed, 
 
 int ppcsr_apply_batch(ppcsr_shard *s, const uint32_t *src, const uint32_t *dst, const uint32_t *val, uint64_t count,
                       uint32_t default_val, ppcsr_batch_stats *stats) {
+  if (s) changes_clear(s);
   if (!s || (count && (!src || !dst))) return PPCSR_ERR_ARG;
   PPCSR_TRY(set_device(s));
   if (count == 0) return ppcsr_apply_batch_device(s, nullptr, nullptr, nullptr, 0, default_val, stats);
@@ -1307,6 +1362,7 @@ int ppcsr_submit_batch(ppcsr_shard *s, const uint32_t *src, const uint32_t *dst,
 
 int ppcsr_wait(ppcsr_shard *s, uint64_t ticket, ppcsr_batch_stats *stats) {
   if (!s) return PPCSR_ERR_ARG;
+  changes_clear(s);
   PPCSR_TRY(set_device(s));
   ppcsr_shard::Pending &P = s->pending[ticket & 1u];
   if (!P.busy || P.ticket != ticket) {
@@ -1329,6 +1385,7 @@ int ppcsr_wait(ppcsr_shard *s, uint64_t ticket, ppcsr_batch_stats *stats) {
 // ---- binary input path: interleaved (src, dst) pairs, e.g. an mmap'd edge file -----------------------------------
 int ppcsr_apply_batch_pairs(ppcsr_shard *s, const uint32_t *pairs, uint64_t count, uint32_t default_val,
                             ppcsr_batch_stats *stats) {
+  if (s) changes_clear(s);
   if (!s || (count && !pairs)) return PPCSR_ERR_ARG;
   PPCSR_TRY(set_device(s));
   if (count == 0) return ppcsr_apply_batch_device(s, nullptr, nullptr, nullptr, 0, default_val, stats);
@@ -1412,6 +1469,7 @@ int ppcsr_copy_to_host(int device, void *host, const void *dev, uint64_t bytes) 
 }
 
 int ppcsr_add_edge(ppcsr_shard *s, uint32_t src, uint32_t dst, uint32_t value) {
+  if (s) changes_clear(s);
   if (value == 0) return PPCSR_OK;  // reference PCSR.cpp:1375: a zero value is silently ignored
   return ppcsr_apply_batch(s, &src, &dst, &value, 1, 1, nullptr);
 }
@@ -1426,6 +1484,7 @@ int ppcsr_remove_edge(ppcsr_shard *s, uint32_t src, uint32_t dst, int *found) {
 
 int ppcsr_add_nodes(ppcsr_shard *s, uint32_t count) {
   if (!s) return PPCSR_ERR_ARG;
+  changes_clear(s);
   if (count == 0) return PPCSR_OK;
   PPCSR_TRY(set_device(s));
   if (s->poisoned) return poisoned_error();
@@ -1478,6 +1537,7 @@ int ppcsr_add_nodes(ppcsr_shard *s, uint32_t count) {
 
 int ppcsr_isolate_vertices(ppcsr_shard *s, const uint32_t *ids, uint64_t count, ppcsr_batch_stats *stats) {
   if (!s || (count && !ids)) return PPCSR_ERR_ARG;
+  if (s) changes_clear(s);
   PPCSR_TRY(set_device(s));
   PPCSR_TRY(isolate_check_ids(ids, count, s->n, "ppcsr_isolate_vertices"));
   if (count == 0) {
@@ -1504,6 +1564,38 @@ int ppcsr_set_whole_array_policy(ppcsr_shard *s, int mode) {
 int ppcsr_last_stats(ppcsr_shard *s, ppcsr_batch_stats *stats) {
   if (!s || !stats) return PPCSR_ERR_ARG;
   *stats = s->last;
+  return PPCSR_OK;
+}
+
+int ppcsr_set_change_capture(ppcsr_shard *s, int on) {
+  if (!s) return PPCSR_ERR_ARG;
+  PPCSR_TRY(set_device(s));
+  changes_clear(s);
+  if (!on && s->capture) {  // give the memory back: nothing of it is used while capture is off
+    CUDA_TRY(cudaStreamSynchronize(s->stream));
+    dev_free(s->cap_kind); dev_free(s->cap_old); dev_free(s->chg_src); dev_free(s->chg_dst); dev_free(s->chg_old);
+    dev_free(s->chg_new); dev_free(s->nf_src); dev_free(s->nf_dst);
+  }
+  s->capture = on != 0;
+  return PPCSR_OK;
+}
+
+int ppcsr_last_changes(ppcsr_shard *s, ppcsr_changes *out) {
+  if (!s || !out) return PPCSR_ERR_ARG;
+  if (!s->capture) {
+    g_ppcsr_error = "ppcsr_last_changes: change capture is off (ppcsr_set_change_capture)";
+    return PPCSR_ERR_ARG;
+  }
+  const bool c = s->n_changes != 0, m = s->n_nf != 0;
+  out->src = c ? s->chg_src.p : nullptr;
+  out->dst = c ? s->chg_dst.p : nullptr;
+  out->old_val = c ? s->chg_old.p : nullptr;
+  out->new_val = c ? s->chg_new.p : nullptr;
+  out->n_changes = s->n_changes;
+  out->nf_src = m ? s->nf_src.p : nullptr;
+  out->nf_dst = m ? s->nf_dst.p : nullptr;
+  out->n_not_found = s->n_nf;
+  out->device = s->device;
   return PPCSR_OK;
 }
 
@@ -1819,6 +1911,7 @@ int ppcsr_export_csr(ppcsr_shard *s, uint64_t *rowptr, uint32_t *col, uint32_t *
 int ppcsr_load_csr(ppcsr_shard *s, uint32_t n, const uint64_t *rowptr, const uint32_t *col, const uint32_t *val,
                    const uint32_t *nn) {
   if (!s || !rowptr) return PPCSR_ERR_ARG;
+  changes_clear(s);
   PPCSR_TRY(set_device(s));
   if (s->poisoned) {
     g_ppcsr_error = "ppcsr_load_csr: the shard is poisoned by a failed batch; ppcsr_restore it first";
@@ -2036,6 +2129,7 @@ int ppcsr_snapshot(ppcsr_shard *s) {
 }
 
 int ppcsr_restore(ppcsr_shard *s) {
+  if (s) changes_clear(s);
   if (!s || !s->snap.valid) return PPCSR_ERR_ARG;
   PPCSR_TRY(set_device(s));
   Snapshot &k = s->snap;

@@ -236,6 +236,13 @@ struct ppcsr_shard {
   DevBuf<uint32_t> hist;               // radix histograms
   DevBuf<double> pr_acc;               // pagerank fp64 accumulator
   DevBuf<uint32_t> misc;               // misc query scratch
+  // change capture (ppcsr_set_change_capture): allocated only while it is on
+  bool capture = false;
+  DevBuf<uint8_t> cap_kind;            // [batch] per sorted update: class of a winner | misses << 2 (batch::k_locate_capture)
+  DevBuf<uint32_t> cap_old;            // [batch] per sorted update: value an overwrite or delete replaced
+  DevBuf<uint32_t> chg_src, chg_dst, chg_old, chg_new;  // [batch] the last batch's changes, key order
+  DevBuf<uint32_t> nf_src, nf_dst;     // [batch] the last batch's removes that missed, key order
+  uint64_t n_changes = 0, n_nf = 0;    // their lengths; 0 after anything but a successful batch
 
   BatchScalars *d_scalars = nullptr;   // device
   BatchScalars *h_scalars = nullptr;   // pinned host

@@ -158,6 +158,31 @@ float PCSR::apply_batch_pairs(const uint32_t *pairs, size_t count, uint32_t defa
   return st.ms_total;
 }
 
+void PCSR::set_change_capture(bool on) {
+  if (ppcsr_set_change_capture(shard_, on ? 1 : 0) != PPCSR_OK) fail("ppcsr_set_change_capture");
+}
+
+PCSR::Changes PCSR::last_changes(uint64_t vertex_offset) const {
+  ppcsr_changes c{};
+  if (ppcsr_last_changes(shard_, &c) != PPCSR_OK) fail("ppcsr_last_changes");
+  Changes out;
+  const struct {
+    std::vector<uint32_t> *host;
+    const uint32_t *dev;
+    uint64_t n;
+  } lists[] = {{&out.src, c.src, c.n_changes},     {&out.dst, c.dst, c.n_changes},
+               {&out.old_val, c.old_val, c.n_changes}, {&out.new_val, c.new_val, c.n_changes},
+               {&out.nf_src, c.nf_src, c.n_not_found}, {&out.nf_dst, c.nf_dst, c.n_not_found}};
+  for (const auto &l : lists) {
+    l.host->resize(l.n);
+    if (l.n && ppcsr_copy_to_host(c.device, l.host->data(), l.dev, l.n * sizeof(uint32_t)) != PPCSR_OK)
+      fail("ppcsr_copy_to_host");
+  }
+  for (uint32_t &s : out.src) s += (uint32_t)vertex_offset;
+  for (uint32_t &s : out.nf_src) s += (uint32_t)vertex_offset;
+  return out;
+}
+
 // after a batch went through the C-ABI behind this object's back (PPPCSR's group route) or through apply_batch
 void PCSR::batch_applied() {
   nodes_dirty_ = true;

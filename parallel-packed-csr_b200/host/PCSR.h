@@ -83,6 +83,15 @@ class PCSR {
   int device() const { return device_; }
   bool print_not_found = true;  // the reference prints "not found s d" per miss (PCSR.cpp:751)
 
+  // What each batch changed (C-ABI ppcsr_set_change_capture / ppcsr_last_changes), copied to the host: one entry per
+  // changed key (old_val 0 = inserted, new_val 0 = deleted) and one (nf_src, nf_dst) per remove that missed, both in
+  // ascending (src, dst) order.  Sources are shard-local plus `vertex_offset`.
+  struct Changes {
+    std::vector<uint32_t> src, dst, old_val, new_val, nf_src, nf_dst;
+  };
+  void set_change_capture(bool on);
+  Changes last_changes(uint64_t vertex_offset = 0) const;
+
  private:
   void refresh_geometry();
   void refresh_nodes() const;

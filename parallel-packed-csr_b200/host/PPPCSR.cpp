@@ -100,6 +100,27 @@ void PPPCSR::wait_batch(uint64_t ticket, std::vector<ppcsr_batch_stats> *stats) 
   if (stats) *stats = st;
 }
 
+void PPPCSR::set_change_capture(bool on) {
+  for (auto &part : partitions) part.set_change_capture(on);
+}
+
+PCSR::Changes PPPCSR::last_changes() const {
+  PCSR::Changes all;
+  for (std::size_t p = 0; p < partitions.size(); p++) {
+    const PCSR::Changes c = partitions[p].last_changes(distribution[p]);
+    auto append = [](std::vector<uint32_t> &to, const std::vector<uint32_t> &from) {
+      to.insert(to.end(), from.begin(), from.end());
+    };
+    append(all.src, c.src);
+    append(all.dst, c.dst);
+    append(all.old_val, c.old_val);
+    append(all.new_val, c.new_val);
+    append(all.nf_src, c.nf_src);
+    append(all.nf_dst, c.nf_dst);
+  }
+  return all;
+}
+
 std::size_t PPPCSR::get_partiton(size_t vertex_id) const {
   // first partition whose successor starts beyond the vertex; ids past the end go to the last one
   // (reference PPPCSR.cpp:58-66)

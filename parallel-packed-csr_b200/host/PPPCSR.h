@@ -66,6 +66,10 @@ class PPPCSR {
   // boundaries[p] (boundaries[0] == 0, strictly ascending, one entry per partition; the last partition ends at
   // get_n()).  The logical graph is unchanged.
   ppcsr_repartition_stats repartition(const std::vector<size_t> &boundaries);
+  // Change capture on every partition (PCSR::set_change_capture); last_changes() concatenates the partitions' lists of
+  // the last batch in partition order with GLOBAL sources, so both lists stay in ascending (src, dst) order.
+  void set_change_capture(bool on);
+  PCSR::Changes last_changes() const;
 
  private:
   void build(uint32_t init_n, bool lock_search, bool use_numa);

@@ -22,6 +22,10 @@
 // them two ahead (-ppcsr: ppcsr_submit_batch / ppcsr_wait; partitioned modes: PPPCSR::submit_batch / wait_batch), so the
 // copy (and, partitioned, the routing) of the next batch runs while the current one is applied; the second "Elapsed
 // wall clock time" line covers the whole stream, "not found" sums over its batches.  Default 1: one batch.
+// -not_found_lines turns change capture on for the update phase and prints one "not found <src> <dst>" line (global
+// ids) per remove that missed, as the reference prints them (reference PCSR.cpp:751), in place of the
+// "not found <N> edges" count: the same multiset of lines as the reference at -threads=1, batch by batch in ascending
+// (src, dst) order rather than in call order.
 // Traversals after the updates, on the devices (-ppcsr: one shard; partitioned modes: across all partitions):
 //   -bfs=<start>         prints "BFS from <start>: reached <k> levels <L> hash <016x>": k reached vertices, L = 1 + the
 //                        largest hop count (0 if nothing is reached), hash = sum mod 2^64 of
@@ -192,10 +196,11 @@ static void run_phase(const EdgeArrays &e, Pool *pool, int threads, size_t count
 }
 
 template <typename Pool>
-static void execute(int threads, int size, int batches, const EdgeArrays &core, const EdgeArrays &updates,
-                    std::unique_ptr<Pool> &pool) {
+static void execute(int threads, int size, int batches, bool not_found_lines, const EdgeArrays &core,
+                    const EdgeArrays &updates, std::unique_ptr<Pool> &pool) {
   run_phase(core, pool.get(), threads, core.size());
   pool->set_batches(batches);
+  if (not_found_lines) pool->set_not_found_lines(true);
   run_phase(updates, pool.get(), threads, (size_t)size);
 }
 
@@ -284,7 +289,7 @@ static void run_traversals(G &graph, long bfs_start, long pr_iterations) {
 int main(int argc, char *argv[]) {
   int threads = 8, size = 1000000, num_nodes = 0, partitions_per_domain = 1, batches = 1;
   bool lock_search = true, insert = true, check = false, host_parse = false, balanced = false, checksum = false,
-       repartition = false;
+       repartition = false, not_found_lines = false;
   long bfs_start = -1, pr_iterations = -1;  // -bfs= / -pagerank= (negative: not requested)
   Version v = Version::PPPCSRNUMA;
   EdgeArrays core_graph, updates;
@@ -328,6 +333,8 @@ int main(int argc, char *argv[]) {
       check = true;
     } else if (starts_with(s, "-host_parse")) {
       host_parse = true;
+    } else if (starts_with(s, "-not_found_lines")) {
+      not_found_lines = true;
     } else if (starts_with(s, "-repartition")) {
       repartition = true;
     } else if (starts_with(s, "-balanced")) {
@@ -356,7 +363,7 @@ int main(int argc, char *argv[]) {
   uint64_t sum[3] = {0, 0, 0};  // -checksum: edges, edge hash, num_neighbors hash of the logical graph
   if (v == Version::PPCSR) {
     auto pool = std::make_unique<ThreadPool>(threads, lock_search, num_nodes + 1, partitions_per_domain);
-    execute(threads, size, batches, core_graph, updates, pool);
+    execute(threads, size, batches, not_found_lines, core_graph, updates, pool);
     const ppcsr_batch_stats &st = pool->last_stats();
     std::cout << "{\"updates\": " << st.batch_size << ", \"device_ms\": " << st.ms_total
               << ", \"rebalance_bytes_per_update\": " << (st.batch_size ? (double)st.rebalance_bytes / st.batch_size : 0)
@@ -378,7 +385,7 @@ int main(int argc, char *argv[]) {
       pool = std::make_unique<ThreadPoolPPPCSR>(threads, lock_search, num_nodes + 1, partitions_per_domain,
                                                 v == Version::PPPCSRNUMA);
     }
-    execute(threads, size, batches, core_graph, updates, pool);
+    execute(threads, size, batches, not_found_lines, core_graph, updates, pool);
     const auto &sts = pool->last_stats();
     uint64_t upd = 0, bytes = 0, windows = 0;
     float device_ms = 0;

@@ -15,6 +15,18 @@ ThreadPool::ThreadPool(const int NUM_OF_THREADS, bool lock_search, uint32_t init
 
 ThreadPool::~ThreadPool() { delete pcsr; }
 
+void ThreadPool::set_not_found_lines(bool on) {
+  nf_lines_ = on;
+  pcsr->set_change_capture(on);
+}
+
+void ThreadPool::collect_not_found() {
+  if (!nf_lines_) return;
+  const PCSR::Changes c = pcsr->last_changes();
+  nf_src_.insert(nf_src_.end(), c.nf_src.begin(), c.nf_src.end());
+  nf_dst_.insert(nf_dst_.end(), c.nf_dst.begin(), c.nf_dst.end());
+}
+
 // thread_id is irrelevant on the device (ThreadPoolPPPCSR ignores it in the reference too,
 // src/thread_pool_pppcsr/thread_pool_pppcsr.cpp:97); submission order is kept: last op wins per edge.
 void ThreadPool::submit_add(int thread_id, int src, int dest) {
@@ -47,6 +59,8 @@ void ThreadPool::start(int threads) {
   (void)threads;
   t0_ = std::chrono::steady_clock::now();
   finished_ = false;
+  nf_src_.clear();
+  nf_dst_.clear();
   std::cout << "Thread 0 has " << src_.size() + reads_.size() << " tasks" << std::endl;
   pcsr->edges.global_lock->registerThread();
   if (batches_ > 1 && !src_.empty()) {
@@ -69,10 +83,12 @@ void ThreadPool::start(int threads) {
             std::exit(EXIT_FAILURE);
           }
           add_batch_stats(stats_, st);
+          collect_not_found();
         });
     pcsr->batch_applied();
   } else if (!src_.empty()) {
     pcsr->apply_batch(src_, dst_, val_, &stats_);
+    collect_not_found();
   }
   for (int v : reads_) pcsr->read_neighbourhood(v);
   pcsr->edges.global_lock->unregisterThread();
@@ -86,7 +102,12 @@ void ThreadPool::stop() {
   }
   std::cout << "Done" << std::endl;
   t1_ = std::chrono::steady_clock::now();
-  if (stats_.n_not_found) std::cout << "not found " << stats_.n_not_found << " edges" << std::endl;
+  if (nf_lines_) {
+    for (size_t i = 0; i < nf_src_.size(); i++) std::cout << "not found " << nf_src_[i] << " " << nf_dst_[i] << "\n";
+    std::cout << std::flush;
+  } else if (stats_.n_not_found) {
+    std::cout << "not found " << stats_.n_not_found << " edges" << std::endl;
+  }
   std::cout << "Elapsed wall clock time: "
             << std::chrono::duration_cast<std::chrono::milliseconds>(t1_ - t0_).count() << std::endl;
   src_.clear();

@@ -29,6 +29,9 @@ class ThreadPool {
   // start() applies the staged updates as `k` consecutive batches of ceil(count / k), streamed two ahead through
   // ppcsr_submit_batch / ppcsr_wait (k = 1: one batch); last_stats() then sums the counters over the batches
   void set_batches(int k) { batches_ = k; }
+  // on: the batches capture what they change, and stop() prints one "not found <src> <dst>" line (global ids) per
+  // remove that missed, as the reference does (PCSR.cpp:751), in place of the "not found <N> edges" count
+  void set_not_found_lines(bool on);
 
   const ppcsr_batch_stats &last_stats() const { return stats_; }
 
@@ -40,4 +43,7 @@ class ThreadPool {
   ppcsr_batch_stats stats_{};
   int threads_;
   int batches_ = 1;
+  bool nf_lines_ = false;
+  std::vector<uint32_t> nf_src_, nf_dst_;  // the misses of the phase, batch by batch (set_not_found_lines)
+  void collect_not_found();
 };

@@ -54,6 +54,18 @@ void ThreadPoolPPPCSR::init_tables(int NUM_OF_THREADS) {
 
 ThreadPoolPPPCSR::~ThreadPoolPPPCSR() { delete pcsr; }
 
+void ThreadPoolPPPCSR::set_not_found_lines(bool on) {
+  nf_lines_ = on;
+  pcsr->set_change_capture(on);
+}
+
+void ThreadPoolPPPCSR::collect_not_found() {
+  if (!nf_lines_) return;
+  const PCSR::Changes c = pcsr->last_changes();
+  nf_src_.insert(nf_src_.end(), c.nf_src.begin(), c.nf_src.end());
+  nf_dst_.insert(nf_dst_.end(), c.nf_dst.begin(), c.nf_dst.end());
+}
+
 // Global ids, submission order: the owner of every op is found ON THE DEVICE when the batch starts (the reference
 // looks it up here, per op: thread_pool_pppcsr.cpp:98).
 void ThreadPoolPPPCSR::stage(int src, int dest, uint32_t value) {
@@ -86,6 +98,8 @@ void ThreadPoolPPPCSR::start(int threads) {
   t0_ = std::chrono::steady_clock::now();
   finished_ = false;
   not_found_ = 0;
+  nf_src_.clear();
+  nf_dst_.clear();
   std::cout << "Thread 0 has " << src_.size() << " tasks for " << pcsr->partition_count()
             << " partitions, routed on the device" << std::endl;
   for (std::size_t p = 0; p < pcsr->partition_count(); p++) pcsr->registerThread((int)p);
@@ -98,9 +112,11 @@ void ThreadPoolPPPCSR::start(int threads) {
         [&](uint64_t ticket) {
           pcsr->wait_batch(ticket, &st);
           for (std::size_t p = 0; p < st.size(); p++) add_batch_stats(stats_[p], st[p]);
+          collect_not_found();
         });
   } else if (!src_.empty()) {
     pcsr->apply_batch(src_.data(), dst_.data(), val_.data(), src_.size(), &stats_);
+    collect_not_found();
   }
   for (std::size_t p = 0; p < pcsr->partition_count(); p++) pcsr->unregisterThread((int)p);
   for (auto &st : stats_) not_found_ += st.n_not_found;
@@ -117,7 +133,12 @@ void ThreadPoolPPPCSR::stop() {
     std::cout << "Done" << std::endl;
   }
   t1_ = std::chrono::steady_clock::now();
-  if (not_found_) std::cout << "not found " << not_found_ << " edges" << std::endl;
+  if (nf_lines_) {
+    for (size_t i = 0; i < nf_src_.size(); i++) std::cout << "not found " << nf_src_[i] << " " << nf_dst_[i] << "\n";
+    std::cout << std::flush;
+  } else if (not_found_) {
+    std::cout << "not found " << not_found_ << " edges" << std::endl;
+  }
   std::cout << "Elapsed wall clock time: "
             << std::chrono::duration_cast<std::chrono::milliseconds>(t1_ - t0_).count() << std::endl;
   src_.clear();

@@ -33,6 +33,9 @@ class ThreadPoolPPPCSR {
   // start() applies the staged updates as `k` consecutive batches of ceil(count / k), streamed two ahead through
   // PPPCSR::submit_batch / wait_batch (k = 1: one batch); last_stats() then sums the counters over the batches
   void set_batches(int k) { batches_ = k; }
+  // on: the batches capture what they change, and stop() prints one "not found <src> <dst>" line (global ids) per
+  // remove that missed, as the reference does (PCSR.cpp:751), in place of the "not found <N> edges" count
+  void set_not_found_lines(bool on);
 
   // thread -> domain table of the reference (thread_pool_pppcsr.cpp:32-47), kept for the CPU-side reads
   const std::vector<int> &thread_to_domain() const { return threadToDomain; }
@@ -51,6 +54,9 @@ class ThreadPoolPPPCSR {
   uint64_t not_found_ = 0;
   std::vector<ppcsr_batch_stats> stats_;
   int batches_ = 1;
+  bool nf_lines_ = false;
+  std::vector<uint32_t> nf_src_, nf_dst_;  // the misses of the phase, batch by batch (set_not_found_lines)
+  void collect_not_found();
 
   const int available_nodes;  // GPUs used as "domains"
   int partitions_per_domain = 1;
